@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 sensitivity hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (config 2 of BASELINE.json): a batch of 4096 dense random QPs, n=64, m_eq=16,
 m_ineq=64 (KKT order N=144).  One *solve* = KKT assembly + one LU factorisation + one forward
@@ -24,6 +24,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (the tree may be read-only)
 
 N_VAR, M_INEQ, P_EQ = 64, 64, 16
 KKT_N = N_VAR + M_INEQ + P_EQ
@@ -247,7 +248,7 @@ def run_reference(args, rank, world):
         cpu_reference_rate(d, min(sample, 16 * procs), procs)
     dt = 0.0
     done = 0
-    steps = min(args.steps, 20)   # each step is the full 4096-instance batch (~0.2 s on 32 cores)
+    steps = args.steps   # each step is the full 4096-instance batch (~0.2 s on 32 cores)
     for _ in range(steps):
         dt += sample / cpu_reference_rate(d, sample, procs)   # times the worker map only, not pool start-up
         done += sample
@@ -288,6 +289,32 @@ def bind_to_gpu_numa_node(local_rank):
         return {"numa_node": node, "bound": True, "cpus": len(cpus)}
     except Exception as e:  # pragma: no cover
         return {"bound": False, "why": str(e)[:80]}
+
+
+DUMP_LIMIT_BYTES = 60_000_000   # array data; the files stay under 64 MB with their .npy headers
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """Writes what the timed call returned in its last step, every rank's shard in instance order, as
+    out_dir/<name>.npy in float64: the inputs are seeded, so two builds can be compared output for output.  Above
+    DUMP_LIMIT_BYTES in all, a fixed seeded sample of instances is kept and their indices go to instance.npy."""
+    import torch.distributed as dist
+    host = {k: v.cpu().numpy().astype(np.float64) for k, v in arrays.items()}
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, host)
+        host = {k: np.concatenate([p[k] for p in parts]) for k in host}
+    if rank != 0:
+        return
+    B = len(host["fwd"])
+    row_bytes = sum(v[0].nbytes for v in host.values())
+    if B * row_bytes > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT_BYTES // (row_bytes + 8), replace=False))
+        host = {k: v[keep] for k, v in host.items()}
+        host["instance"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def run_b200(args, rank, world, local_rank):
@@ -391,6 +418,8 @@ def run_b200(args, rank, world, local_rank):
     t1 = time.perf_counter()
     launches = ctx.launch_count - l0
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"fwd": fwd, "rev": rev, "info": info}, rank, world)
     kernel_ms = ms / args.steps   # device time per launch: the timed region holds nothing but the K launches
     # the blocking form of the same call (what the reference-facing API does): a few calls, for the record
     step_device_blocking()
@@ -823,7 +852,13 @@ def main():
     ap.add_argument("--batch", type=int, default=4096)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-aux", action="store_true", help="skip the active-set sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the forward / reverse sensitivities and info codes of the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the CPU arm only times the reference's work)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
