@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("DIFFOPT_B200_LIB") or os.path.join(HERE, "lib", "libd
 
 HOST, DEVICE = 0, 1
 QP_SHARED_MATRICES, QP_SHARED_DIRECTION, QP_PACKED_Q, QP_ASYNC, QP_ALLREDUCE = 1, 2, 4, 8, 16
-CONE_ZERO, CONE_NONNEG, CONE_SOC, CONE_PSD = 0, 1, 2, 3
+CONE_ZERO, CONE_NONNEG, CONE_SOC, CONE_PSD, CONE_EXP, CONE_DUAL_EXP = 0, 1, 2, 3, 4, 5
 
 _lib = None
 

@@ -9,7 +9,7 @@ import time
 
 import numpy as np
 
-from ._capi import CONE_NONNEG, CONE_PSD, CONE_SOC, CONE_ZERO, HOST, Context, ptr  # noqa: F401
+from ._capi import CONE_DUAL_EXP, CONE_EXP, CONE_NONNEG, CONE_PSD, CONE_SOC, CONE_ZERO, HOST, Context, ptr  # noqa: F401
 from .lsqr import DEFAULTS, julia_csc
 
 

@@ -67,10 +67,14 @@ struct ConicState {
     CsrDev A;
     DevBuf b, c, x, s, y, v, vp;
     // per-row cone metadata and per-cone data
-    DevBuf row_kind;     // int8 per row: 0 identity (zero cone -> free dual), 1 nonneg, 2 soc, 3 psd
+    DevBuf row_kind;     // int8 per row: 0 zero / nonneg (diagonal), 2 soc, 3 psd, 4 + j row j of a 3 x 3 block cone
     DevBuf nn_scale;     // double per row: (sign(v)+1)/2 for nonneg rows, 1 for zero rows
     DevBuf soc_off, soc_dim, soc_case, soc_nx;  // per SOC cone
     int64_t nsoc = 0;
+    // cones with a symmetric 3 x 3 Dpi block (exponential, dual exponential): first row, v negated (DIFFOPT_CONE_EXP:
+    // pi onto K* = -(pi onto K°)(-v)); blk3: 3 coefficients per row of such a cone (row i: blk3[3 i .. 3 i + 2])
+    DevBuf exp_off, exp_neg, blk3;
+    int64_t nexp = 0;
     // PSD cones
     DevBuf psd_off, psd_d, psd_uoff;  // per PSD cone: row offset, side d, offset into U/B storage
     DevBuf psd_U, psd_Bm, psd_ident;  // eigenvectors (col-major d x d), B matrix, identity flag

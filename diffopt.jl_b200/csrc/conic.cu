@@ -4,6 +4,7 @@
 #include <cmath>
 #include <vector>
 
+#include "exp_cone.cuh"
 #include "lsqr.cuh"
 
 ConicOpView conic_view(diffopt_b200_ctx* ctx, bool stream_blocks);
@@ -293,7 +294,8 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     const int64_t* cd = (const int64_t*)hcd;
     // cone bookkeeping (host): row kinds and per-cone index lists
     std::vector<signed char> kind((size_t)m, 0), rowtype((size_t)m, 0);
-    std::vector<int> soc_off, soc_dim, psd_off, psd_d;
+    std::vector<int> soc_off, soc_dim, psd_off, psd_d, exp_off;
+    std::vector<signed char> exp_neg;
     std::vector<long long> psd_uoff;
     int64_t row = 0, sumd2 = 0, maxd = 0;
     for (int64_t k = 0; k < ncones; ++k) {
@@ -321,6 +323,13 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
                 sumd2 += d * d;
                 maxd = d > maxd ? d : maxd;
             } break;
+            case DIFFOPT_CONE_EXP:
+            case DIFFOPT_CONE_DUAL_EXP:
+                if (dim != 3) BAD_ARG(ctx, "conic_setup: exponential cone dimension must be 3");
+                for (int64_t i = 0; i < 3; ++i) kind[(size_t)(row + i)] = (signed char)(4 + i);
+                exp_off.push_back((int)row);
+                exp_neg.push_back(ct[k] == DIFFOPT_CONE_EXP ? 1 : 0);
+                break;
             default:
                 BAD_ARG(ctx, "conic_setup: unknown cone type");
         }
@@ -330,6 +339,7 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     S.n = n; S.m = m; S.ncones = ncones;
     S.nsoc = (int64_t)soc_off.size();
     S.npsd = (int64_t)psd_off.size();
+    S.nexp = (int64_t)exp_off.size();
     S.psd_sumd2 = sumd2;
     S.psd_maxd = maxd;
     if (int32_t rc = csr_from_csc_host(ctx, m, n, (const int64_t*)hc, (const int64_t*)hr, (const double*)hv, S.A))
@@ -353,6 +363,9 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     DO_CUDA(ctx, keep(S.psd_off, psd_off.data(), sizeof(int) * psd_off.size(), cudaMemcpyHostToDevice));
     DO_CUDA(ctx, keep(S.psd_d, psd_d.data(), sizeof(int) * psd_d.size(), cudaMemcpyHostToDevice));
     DO_CUDA(ctx, keep(S.psd_uoff, psd_uoff.data(), sizeof(long long) * psd_uoff.size(), cudaMemcpyHostToDevice));
+    DO_CUDA(ctx, keep(S.exp_off, exp_off.data(), sizeof(int) * exp_off.size(), cudaMemcpyHostToDevice));
+    DO_CUDA(ctx, keep(S.exp_neg, exp_neg.data(), exp_neg.size(), cudaMemcpyHostToDevice));
+    DO_CUDA(ctx, S.blk3.reserve(exp_off.empty() ? 8 : d8 * 3 * (size_t)m));
     {   // flattened list of 32 x 32 output tiles of the PSD apply
         std::vector<int> toff(psd_d.size() + 1, 0);
         for (size_t k = 0; k < psd_d.size(); ++k) {
@@ -389,6 +402,13 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
         cone_soc_kernel<<<blocks, 256, 0, ctx->stream>>>((int)S.nsoc, S.soc_off.as<int>(), S.soc_dim.as<int>(),
                                                           S.v.as<double>(), S.soc_case.as<int>(), S.soc_nx.as<double>(),
                                                           S.vp.as<double>());
+        ctx->launches++;
+    }
+    if (S.nexp > 0) {
+        int blocks = (int)((S.nexp + 127) / 128);
+        if (blocks > ctx->sm_count * 16) blocks = ctx->sm_count * 16;
+        cone_exp_kernel<<<blocks, 128, 0, ctx->stream>>>((int)S.nexp, S.exp_off.as<int>(), S.exp_neg.as<signed char>(),
+                                                          S.v.as<double>(), S.vp.as<double>(), S.blk3.as<double>(), nullptr);
         ctx->launches++;
     }
     if (S.npsd > 0)

@@ -445,8 +445,16 @@ __device__ void psd_apply_all(Dev& d, const ConicOpView& op, const double* __res
 // problems with PSD cones; their kernels stay small).
 template <bool PSD>
 __device__ void dpi_apply(Dev& d, const ConicOpView& op, const double* __restrict__ y, double* out, bool transpose) {
-    for (int i = d.gtid; i < op.m; i += d.gthreads)
-        if (op.kind[i] == 0) out[i] = op.diag[i] * __ldcg(y + i);
+    for (int i = d.gtid; i < op.m; i += d.gthreads) {
+        const int k = op.kind[i];
+        if (k == 0) {
+            out[i] = op.diag[i] * __ldcg(y + i);
+        } else if (k >= 4) {  // row k - 4 of a symmetric 3 x 3 block (exp cones): the same for Dpi and Dpi'
+            const double* br = op.blk3 + 3 * (long long)i;
+            const double* yc = y + (i - (k - 4));
+            out[i] = br[0] * __ldcg(yc) + br[1] * __ldcg(yc + 1) + br[2] * __ldcg(yc + 2);
+        }
+    }
     {
         const int T = 8;
         const int lig = d.lane & (T - 1);
@@ -1287,6 +1295,7 @@ ConicOpView conic_view(diffopt_b200_ctx* ctx, bool stream_blocks = false) {
     o.c = s.c.as<double>();
     o.diag = s.nn_scale.as<double>();
     o.kind = s.row_kind.as<signed char>();
+    o.blk3 = s.blk3.as<double>();
     o.nsoc = (int)s.nsoc;
     o.soc_off = s.soc_off.as<int>();
     o.soc_dim = s.soc_dim.as<int>();
@@ -1476,6 +1485,7 @@ static int32_t lsqr_stream_conic(diffopt_b200_ctx* ctx, const double* rhs_dev, L
         if (b < 1) b = 1;
         return (unsigned)b;
     };
+    // Dpi: one thread per row (diagonal and 3 x 3 block rows), 8 lanes per SOC cone
     const unsigned g_vec = blocks_for(N), g_dpi = blocks_for(std::max<int64_t>(m, (int64_t)cs.nsoc * 8));
     // SpMV kernels: persistent over the row blocks, every resident CTA slot filled exactly once (8 CTAs per SM)
     auto blocks_spmv = [&](int64_t nblk) {

@@ -27,7 +27,8 @@ struct ConicOpView {
     CsrView At;  // n x m
     const double *b, *c;
     const double* diag;       // per row: 1 (zero cone -> dual is free), (sign(v)+1)/2 (nonneg); unused on SOC/PSD rows
-    const signed char* kind;  // per row: 0 diag row, 2 SOC row, 3 PSD row
+    const signed char* kind;  // per row: 0 diag row, 2 SOC row, 3 PSD row, 4 + j row j of a 3 x 3 block cone
+    const double* blk3;       // rows of 3 x 3 block cones: out[i] = blk3[3i .. 3i+2] . y[first row .. first row + 2]
     int nsoc;
     const int* soc_off;   // first row of each SOC cone
     const int* soc_dim;

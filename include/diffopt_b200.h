@@ -43,6 +43,14 @@ typedef struct diffopt_b200_ctx diffopt_b200_ctx;
 #define DIFFOPT_CONE_NONNEG 1 /* MOI.Nonnegatives    */
 #define DIFFOPT_CONE_SOC 2    /* MOI.SecondOrderCone */
 #define DIFFOPT_CONE_PSD 3    /* MOI.PositiveSemidefiniteConeTriangle (unscaled, column-wise upper) */
+/* MOI.ExponentialCone K = cl{(x, y, z) : y > 0, y e^(x/y) <= z}, dimension 3; pi onto K* (Moreau:
+ * Pi_K*(v) = v + Pi_K(-v), DPi_K*(v) = I - DPi_K(-v)) */
+#define DIFFOPT_CONE_EXP 4
+/* MOI.DualExponentialCone K* = cl{(u, v, w) : u < 0, -u e^(v/u) <= e w}, dimension 3; pi onto K.
+ * Pi_K(v), v = (r, s, t), cases in this order (the order decides ties): v in K -> v, I;
+ * v in -K* -> 0, 0; r <= 0 and s <= 0 -> (r, 0, max(t, 0)), diag(1, 0, [t > 0]);
+ * else the curved boundary (root of Friberg's univariate h), symmetric 3 x 3 Jacobian. */
+#define DIFFOPT_CONE_DUAL_EXP 5
 
 /* ---- lifetime ------------------------------------------------------------------- */
 int32_t diffopt_b200_version(void);

@@ -317,6 +317,8 @@ _cone_code(::Type{MOI.Zeros}) = Int32(0)
 _cone_code(::Type{MOI.Nonnegatives}) = Int32(1)
 _cone_code(::Type{MOI.SecondOrderCone}) = Int32(2)
 _cone_code(::Type{MOI.PositiveSemidefiniteConeTriangle}) = Int32(3)
+_cone_code(::Type{MOI.ExponentialCone}) = Int32(4)
+_cone_code(::Type{MOI.DualExponentialCone}) = Int32(5)
 _cone_code(::Type{S}) where {S} = error("DiffOptB200.ConicModel: unsupported set $S")
 
 "cone list in row order (cone_type, cone_dim) from the ProductOfSets -- what `Dπ` / `π` iterate over (diff_opt.jl:491-519)"
