@@ -202,10 +202,10 @@ __global__ void conic_rev_rhs_batch_kernel(int n, int m, const double* __restric
 // g_p (the problem's x region), getters dc_p = g[1:n] - g[N] x, db_p = g[n+I] - g[N] vp (:396-428) and the LSQR
 // statistics, gathered into the caller's instance-major arrays.
 __global__ void conic_rev_out_batch_kernel(int n, int m, const ConicBatchPtrs* __restrict__ pp, const double* __restrict__ work,
-                                           size_t stride, size_t stats_off, double* g_out, double* dc, double* db, double* stats) {
+                                           LsqrBatchLayout L, double* g_out, double* dc, double* db, double* stats) {
     const int p = blockIdx.y;
     const int N = n + m + 1;
-    const double* g = work + (size_t)p * stride + (size_t)(N + 1);
+    const double* g = work + (size_t)p * L.stride + L.x;
     const double gN = g[n + m];
     const double* x = pp[p].x;
     const double* vp = pp[p].vp;
@@ -219,7 +219,7 @@ __global__ void conic_rev_out_batch_kernel(int n, int m, const ConicBatchPtrs* _
         }
     }
     if (stats && blockIdx.x == 0 && threadIdx.x < 4)
-        stats[(size_t)p * 4 + threadIdx.x] = work[(size_t)p * stride + stats_off + threadIdx.x];
+        stats[(size_t)p * 4 + threadIdx.x] = work[(size_t)p * L.stride + L.stats + threadIdx.x];
 }
 
 int32_t to_host_copy(diffopt_b200_ctx* ctx, const void* src, size_t bytes, int memspace, std::vector<char>& tmp,
@@ -656,10 +656,8 @@ int32_t diffopt_b200_conic_batch_reverse(diffopt_b200_ctx* ctx, const double* dx
     const int n = (int)bt->n, m = (int)bt->m, N = n + m + 1, C = bt->C;
     const int64_t B = bt->B;
     const size_t d8 = sizeof(double);
-    // per problem: rhs (N + 1) | x, u, v, w (N each) | partial sums | statistics
-    const size_t stats_off = (size_t)(N + 1) + 4 * (size_t)N + (size_t)LSQR_NSLOTS * C;
-    const size_t stride = (stats_off + 8 + 1) & ~(size_t)1;
-    DO_CUDA(ctx, bt->work.reserve(d8 * stride * (size_t)B));
+    const LsqrBatchLayout L(N, C);
+    DO_CUDA(ctx, bt->work.reserve(d8 * L.stride * (size_t)B));
     if (!bt->ptrs.ptr) {
         std::vector<ConicBatchPtrs> hp((size_t)B);
         for (int64_t p = 0; p < B; ++p) hp[(size_t)p] = ConicBatchPtrs{bt->states[(size_t)p].x.as<double>(), bt->states[(size_t)p].vp.as<double>()};
@@ -669,12 +667,12 @@ int32_t diffopt_b200_conic_batch_reverse(diffopt_b200_ctx* ctx, const double* dx
     const void* dseed;
     DO_CUDA(ctx, stage_in(ctx, ctx->in[0], dx_seeds, d8 * (size_t)n * (size_t)B, memspace, &dseed));
     conic_rev_rhs_batch_kernel<<<(unsigned)B, 512, 0, ctx->stream>>>(n, m, (const double*)dseed, bt->ptrs.as<ConicBatchPtrs>(),
-                                                                    bt->work.as<double>(), stride);
+                                                                    bt->work.as<double>(), L.stride);
     ctx->launches++;
     LsqrParams prm{atol, btol, conlim, maxiter > 0 ? maxiter : (int64_t)N};
     const char* env = getenv("DIFFOPT_B200_CONIC_BATCH_STAGE");
     const bool stage = !(env && env[0] == '0');
-    if (int32_t rc = lsqr_run_conic_batch(ctx, bt->states, C, stage, bt->work.as<double>(), stride, prm, 1e-4 /* :369 */,
+    if (int32_t rc = lsqr_run_conic_batch(ctx, bt->states, C, stage, bt->work.as<double>(), L, prm, 1e-4 /* :369 */,
                                           bt->ops, bt->vecs, bt->rhs))
         return rc;
     void *dg, *ddc, *ddb, *dst;
@@ -683,8 +681,7 @@ int32_t diffopt_b200_conic_batch_reverse(diffopt_b200_ctx* ctx, const double* dx
     DO_CUDA(ctx, stage_out_prepare(ctx->out[2], db_out, d8 * (size_t)m * (size_t)B, memspace, &ddb));
     DO_CUDA(ctx, stage_out_prepare(ctx->out[3], out_stats, d8 * 4 * (size_t)B, memspace, &dst));
     conic_rev_out_batch_kernel<<<dim3((unsigned)((N + 255) / 256), (unsigned)B), 256, 0, ctx->stream>>>(
-        n, m, bt->ptrs.as<ConicBatchPtrs>(), bt->work.as<double>(), stride, stats_off, (double*)dg, (double*)ddc, (double*)ddb,
-        (double*)dst);
+        n, m, bt->ptrs.as<ConicBatchPtrs>(), bt->work.as<double>(), L, (double*)dg, (double*)ddc, (double*)ddb, (double*)dst);
     ctx->launches++;
     DO_CUDA(ctx, cudaGetLastError());
     DO_CUDA(ctx, stage_out_finish(ctx, dg, g_out, d8 * (size_t)N * (size_t)B, memspace));

@@ -15,7 +15,6 @@ namespace cg = cooperative_groups;
 namespace {
 
 constexpr int LSQR_THREADS = 256;
-constexpr int NSLOTS = 8;
 
 #ifdef LSQR_PROF
 __device__ long long g_prof[8192];
@@ -29,7 +28,7 @@ __device__ __forceinline__ long long gtimer() {
 
 struct Dev {
     cg::grid_group grid;
-    double* partials;  // [NSLOTS][nblk]
+    double* partials;  // [LSQR_NSLOTS][nblk]
     double* red;       // shared scratch (>= 2 * warps doubles)
     int tid, lane, warp, nwarp, nblk, gtid, gthreads;
     bool cluster = false;  // the whole grid is ONE thread-block cluster: hardware barrier instead of grid.sync()
@@ -58,6 +57,12 @@ struct Dev {
             grid.sync();
     }
 };
+
+// Dev of a problem solved by the whole grid, its partial sums in columns of `nblk`
+__device__ __forceinline__ Dev make_dev(double* partials, double* red, int nblk) {
+    return Dev{cg::this_grid(), partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
+               (int)(blockDim.x >> 5), nblk, (int)(blockIdx.x * blockDim.x + threadIdx.x), (int)(gridDim.x * blockDim.x)};
+}
 
 __device__ __forceinline__ double warp_sum_all(double v) {
 #pragma unroll
@@ -501,6 +506,86 @@ __device__ void csr_apply(Dev& d, const CsrView& A, const double* __restrict__ s
     block_partial(d, slot, acc);
 }
 
+// ---- Row-block phases of the conic operator, shared by conic_apply<CL = true> and the streaming kernels.  The CTAs
+// that share the row blocks number `ncta`, this one is `cta`; prod / red: shared scratch of spmv_stream.  xw / xs: the
+// vectors the products gather from (wc and src or src + n, or their copies staged in shared memory for XM = 2).
+// Partial sums accumulate into acc (||dst||^2) and dot.  dst is read with ld.global.cg where other CTAs of the same
+// launch wrote it (XM != 0), with plain loads in the one-kernel-per-phase streaming driver.
+template <int XM>
+__device__ __forceinline__ double ld_dst(const double* p) { return XM == 0 ? *p : __ldcg(p); }
+
+// M src: rows 0..n-1 (A' wc)_j + c_j t3, rows n..n+m-1 -(A t1)_i + t2_i - wc_i + b_i t3; dst = s_src * row + s_dst * dst,
+// dot += c't1 + b'wc
+template <int THREADS, int NPT, int XM>
+__device__ __forceinline__ void conic_M_rows(const ConicOpView& op, int cta, int ncta, double* prod, double* red,
+                                             const double* __restrict__ src, const double* xw, const double* xs, double t3,
+                                             double s_src, double* dst, double s_dst, double& acc, double& dot) {
+    const int n = op.n, nbt = op.At.nblk;
+    spmv_stream<THREADS, NPT, XM>(
+        cta, ncta, nbt + op.A.nblk, prod, red,
+        [&](int b, const CsrView*& A, const double*& x, int& lb) {
+            if (b < nbt) { A = &op.At; x = xw; lb = b; }
+            else { A = &op.A; x = xs; lb = b - nbt; }
+        },
+        [&](int b, int row) {
+            return b < nbt ? make_double4(op.c[row], ld_dst<XM>(dst + row), __ldcg(src + row), 0.0)
+                           : make_double4(__ldcg(op.wc + row), __ldcg(src + n + row), op.b[row], ld_dst<XM>(dst + n + row));
+        },
+        [&](int b, int row, double t, const double4& o) {
+            if (b < nbt) {
+                t = (t + o.x * t3) * s_src + s_dst * o.y;
+                dst[row] = t;
+                acc += t * t;
+                dot += o.x * o.z;
+            } else {
+                t = (-t + o.y - o.x + o.z * t3) * s_src + s_dst * o.w;
+                dst[n + row] = t;
+                acc += t * t;
+                dot += o.z * o.x;
+            }
+        });
+}
+
+// M' src, phase 1: wc = A u1 - u2 - b u3, dot += b'u2
+template <int THREADS, int NPT, int XM>
+__device__ __forceinline__ void conic_Mt_A(const ConicOpView& op, int cta, int ncta, double* prod, double* red,
+                                           const double* __restrict__ src, const double* xs, double u3, double& dot) {
+    const int n = op.n;
+    spmv_stream<THREADS, NPT, XM>(
+        cta, ncta, op.A.nblk, prod, red,
+        [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.A; x = xs; lb = b; },
+        [&](int, int row) { return make_double4(__ldcg(src + n + row), op.b[row], 0.0, 0.0); },
+        [&](int, int row, double t, const double4& o) {
+            op.wc[row] = t - o.x - o.y * u3;
+            dot += o.y * o.x;
+        });
+}
+
+// M' src, phase 3 (after r2 = Dpi' wc, stored behind wc): rows 0..n-1 -(A' u2)_j - c_j u3, rows n..n+m-1 r2_i + u2_i;
+// dst = s_src * row + s_dst * dst, dot += c'u1
+template <int THREADS, int NPT, int XM>
+__device__ __forceinline__ void conic_Mt_rows(const ConicOpView& op, int cta, int ncta, double* prod, double* red,
+                                              const double* __restrict__ src, const double* xs, double u3, double s_src,
+                                              double* dst, double s_dst, double& acc, double& dot) {
+    const int n = op.n, m = op.m;
+    spmv_stream<THREADS, NPT, XM>(
+        cta, ncta, op.At.nblk, prod, red,
+        [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.At; x = xs; lb = b; },
+        [&](int, int row) { return make_double4(op.c[row], ld_dst<XM>(dst + row), __ldcg(src + row), 0.0); },
+        [&](int, int row, double t, const double4& o) {
+            t = (-t - o.x * u3) * s_src + s_dst * o.y;
+            dst[row] = t;
+            acc += t * t;
+            dot += o.x * o.z;
+        });
+    const double* r2 = op.wc + m;
+    for (int i = cta * THREADS + (int)threadIdx.x; i < m; i += ncta * THREADS) {
+        const double t = (__ldcg(r2 + i) + __ldcg(src + n + i)) * s_src + s_dst * ld_dst<XM>(dst + n + i);
+        dst[n + i] = t;
+        acc += t * t;
+    }
+}
+
 // dst = s_src * (M src) + s_dst * dst ; slots: slot (norm), slot+1 (last-row dot)
 // `src_last` / `dst_last` are every thread's private copies of src[N-1] / dst[N-1] (all threads compute the last row
 // identically): nobody reads those entries from memory, so thread 0 may store the new one right after the barrier
@@ -514,7 +599,6 @@ __device__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const
     const int n = op.n, m = op.m, N = n + m + 1;
     double dotacc = 0.0;
     if constexpr (CL) {
-        double* prod = cl_prod;
         double* xs_m = cl_prod + CL_CHUNK;  // staged gather vectors (SM): m entries, then n entries
         double* xs_n = xs_m + m;
         constexpr int XM = SM ? 2 : 1;
@@ -535,32 +619,8 @@ __device__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const
                 stage(xs_n, src, n);
                 __syncthreads();
             }
-            const double t3 = src_last;
-            const int nbt = op.At.nblk;
-            spmv_stream<CL_THREADS, CL_NPT, XM>(
-                d.rank(), d.nblk, nbt + op.A.nblk, prod, d.red,
-                [&](int b, const CsrView*& A, const double*& x, int& lb) {
-                    if (b < nbt) { A = &op.At; x = SM ? xs_m : op.wc; lb = b; }
-                    else { A = &op.A; x = SM ? xs_n : src; lb = b - nbt; }
-                },
-                [&](int b, int row) {
-                    return b < nbt ? make_double4(op.c[row], __ldcg(dst + row), __ldcg(src + row), 0.0)
-                                   : make_double4(__ldcg(op.wc + row), __ldcg(src + n + row), op.b[row],
-                                                  __ldcg(dst + n + row));
-                },
-                [&](int b, int row, double t, const double4& o) {
-                    if (b < nbt) {  // rows 0..n-1:  (A' wc)_j + c_j t3
-                        t = (t + o.x * t3) * s_src + s_dst * o.y;
-                        dst[row] = t;
-                        acc += t * t;
-                        dotacc += o.x * o.z;
-                    } else {        // rows n..n+m-1:  -(A t1)_i + t2_i - wc_i + b_i t3
-                        t = (-t + o.y - o.x + o.z * t3) * s_src + s_dst * o.w;
-                        dst[n + row] = t;
-                        acc += t * t;
-                        dotacc += o.z * o.x;
-                    }
-                });
+            conic_M_rows<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : op.wc, SM ? xs_n : src,
+                                                 src_last, s_src, dst, s_dst, acc, dotacc);
             block_partial(d, slot, acc);
             block_partial(d, slot + 1, dotacc);
             d.sync();
@@ -574,34 +634,13 @@ __device__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const
                 stage(xs_n, src, n);
                 __syncthreads();
             }
-            spmv_stream<CL_THREADS, CL_NPT, XM>(  // wc = A u1 - u2 - b u3
-                d.rank(), d.nblk, op.A.nblk, prod, d.red,
-                [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.A; x = SM ? xs_n : src; lb = b; },
-                [&](int, int row) { return make_double4(__ldcg(src + n + row), op.b[row], 0.0, 0.0); },
-                [&](int, int row, double t, const double4& o) {
-                    op.wc[row] = t - o.x - o.y * u3;
-                    dotacc += o.y * o.x;
-                });
+            conic_Mt_A<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_n : src, u3, dotacc);
             d.sync();
-            double* r2 = op.wc + m;
-            dpi_apply<PSD>(d, op, op.wc, r2, true);
+            dpi_apply<PSD>(d, op, op.wc, op.wc + m, true);
             if constexpr (SM) stage(xs_m, src + n, m);   // (src is not touched by dpi_apply: no barrier needed before)
             d.sync();
-            spmv_stream<CL_THREADS, CL_NPT, XM>(  // rows 0..n-1: -(A' u2)_j - c_j u3
-                d.rank(), d.nblk, op.At.nblk, prod, d.red,
-                [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.At; x = SM ? xs_m : src + n; lb = b; },
-                [&](int, int row) { return make_double4(op.c[row], __ldcg(dst + row), __ldcg(src + row), 0.0); },
-                [&](int, int row, double t, const double4& o) {
-                    t = (-t - o.x * u3) * s_src + s_dst * o.y;
-                    dst[row] = t;
-                    acc += t * t;
-                    dotacc += o.x * o.z;
-                });
-            for (int i = d.gtid; i < m; i += d.gthreads) {
-                const double t = (__ldcg(r2 + i) + __ldcg(src + n + i)) * s_src + s_dst * __ldcg(dst + n + i);
-                dst[n + i] = t;
-                acc += t * t;
-            }
+            conic_Mt_rows<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : src + n, u3, s_src,
+                                                  dst, s_dst, acc, dotacc);
             block_partial(d, slot, acc);
             block_partial(d, slot + 1, dotacc);
             d.sync();
@@ -650,10 +689,6 @@ __device__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const
             dotacc += op.b[row] * u2;
         });
         d.sync();
-        // out2 = Dpi' r + u2 : first Dpi' r into a second scratch = reuse psd-free path by writing to dst later.
-        // We need dst's old value (s_dst * dst), so stage Dpi' r in op.wc's partner buffer: the x-part of dst is
-        // disjoint, so compute into `tmp = psd_w-independent` region: use op.wc in place is unsafe (SOC reads all
-        // entries of its cone) -> stage through dst? no.  Use the dedicated second scratch stored after wc.
         double* r2 = op.wc + m;  // second half of the 2m scratch
         dpi_apply<PSD>(d, op, op.wc, r2, true);
         d.sync();
@@ -703,6 +738,161 @@ __device__ double op_apply(Dev& d, const OpArgs& o, bool adjoint, const double* 
     return norm2;
 }
 
+// Scalars of LSQR (Paige-Saunders, damp = 0): the Golub-Kahan bidiagonalisation with true vectors u = su * u_mem and
+// v = sv * v_mem, the plane rotations, the norm and condition estimates and the stop code.  Every driver advances them
+// with these methods in the same order: start, first_alpha, then per iteration the stop tests of the previous one,
+// next_beta, next_alpha (when beta > 0) and rotate.
+struct LsqrScalars {
+    double alpha, beta, su, sv, rhobar, phibar, rho, t1, t2, tau;
+    double anorm, acond, ddnorm, res2, xnorm, xxnorm, z, sn2, cs2, rnorm, arnorm, bnorm;
+    long long itn;
+    int istop;
+
+    // beta = ||b|| from ||b||^2; right-hand sides of norm <= zero_below count as zero.  True when v = A'u is to be formed.
+    __device__ __forceinline__ bool start(double b2, double zero_below) {
+        *this = LsqrScalars{};
+        beta = sqrt(b2);
+        if (beta <= zero_below) beta = 0.0;
+        su = sv = rho = 1.0;
+        cs2 = -1.0;
+        rnorm = beta;
+        if (beta > 0) su = 1.0 / beta;
+        return beta > 0;
+    }
+    // alpha = ||A'u|| from its square (0 when beta = 0) and the start-up values of the recurrences
+    __device__ __forceinline__ void first_alpha(double a2) {
+        alpha = sqrt(a2);
+        if (alpha > 0) sv = 1.0 / alpha;
+        arnorm = alpha * beta;
+        bnorm = beta;
+        rhobar = alpha;
+        phibar = beta;
+    }
+    // stop tests of the iteration rotated last; dd: its share of ddnorm (sum of ||w / rho||^2)
+    __device__ __forceinline__ void stop_tests(double dd, const LsqrParams& prm) {
+        ddnorm += dd;
+        acond = anorm * sqrt(ddnorm);
+        const double test1 = rnorm / bnorm;
+        const double test2 = arnorm / (anorm * rnorm);
+        const double test3 = 1.0 / acond;
+        const double t1_ = test1 / (1.0 + anorm * xnorm / bnorm);
+        const double rtol = prm.btol + prm.atol * anorm * xnorm / bnorm;
+        const double ctol = prm.conlim > 0 ? 1.0 / prm.conlim : 0.0;
+        if (itn >= prm.maxiter) istop = 7;
+        if (1.0 + test3 <= 1.0) istop = 6;
+        if (1.0 + test2 <= 1.0) istop = 5;
+        if (1.0 + t1_ <= 1.0) istop = 4;
+        if (test3 <= ctol) istop = 3;
+        if (test2 <= prm.atol) istop = 2;
+        if (test1 <= rtol) istop = 1;
+    }
+    // next iteration: beta = ||A v - alpha u|| from its square.  True when the next alpha is to be formed.
+    __device__ __forceinline__ bool next_beta(double u2) {
+        itn += 1;
+        beta = sqrt(u2);
+        if (beta > 0) {
+            su = 1.0 / beta;
+            anorm = sqrt(anorm * anorm + alpha * alpha + beta * beta);
+        } else {
+            su = 1.0;  // u_mem is exactly zero
+        }
+        return beta > 0;
+    }
+    // alpha = ||A'u - beta v|| from its square
+    __device__ __forceinline__ void next_alpha(double v2) {
+        alpha = sqrt(v2);
+        sv = alpha > 0 ? 1.0 / alpha : 1.0;
+    }
+    __device__ __forceinline__ void rotate() {
+        const double rhobar1 = rhobar;
+        rho = hypot(rhobar1, beta);
+        const double cs = rhobar1 / rho, sn = beta / rho;
+        const double theta = sn * alpha;
+        rhobar = -cs * alpha;
+        const double phi = cs * phibar;
+        phibar = sn * phibar;
+        tau = sn * phi;
+        t1 = phi / rho;
+        t2 = -theta / rho;
+        const double delta = sn2 * rho, gambar = -cs2 * rho, rhs_ = phi - delta * z;
+        const double zbar = rhs_ / gambar;
+        xnorm = sqrt(xxnorm + zbar * zbar);
+        const double gamma = hypot(gambar, theta);
+        cs2 = gambar / gamma;
+        sn2 = theta / gamma;
+        z = rhs_ / gamma;
+        xxnorm += z * z;
+        rnorm = sqrt(phibar * phibar + res2);
+        arnorm = alpha * fabs(tau);
+    }
+    __device__ __forceinline__ void write_stats(double* stats) const {
+        stats[0] = (double)istop;
+        stats[1] = (double)itn;
+        stats[2] = rnorm;
+        stats[3] = arnorm;
+        stats[4] = anorm;
+        stats[5] = acond;
+        stats[6] = xnorm;
+    }
+};
+
+// u = b, x = v = w = 0; ||b||^2 into slot 0
+__device__ __forceinline__ void lsqr_init(Dev& d, int nr, int nc, const double* __restrict__ rhs, const LsqrVectors& vec) {
+    double acc = 0.0;
+    for (int i = d.gtid; i < nr; i += d.gthreads) {
+        const double t = rhs[i];
+        vec.u[i] = t;
+        acc += t * t;
+    }
+    for (int i = d.gtid; i < nc; i += d.gthreads) {
+        vec.x[i] = 0.0;
+        vec.v[i] = 0.0;
+        vec.w[i] = 0.0;
+    }
+    block_partial(d, 0, acc);
+}
+
+// LSQR's deferred vector update: w = sv v on the first call, later x += t1 w and w = sv v + t2 w; ||w / rho||^2 into
+// slot 4.  ilast >= 0: v[ilast] is read from the register copy v_last (see conic_apply).
+__device__ __forceinline__ void lsqr_update(Dev& d, const LsqrScalars& s, bool first, int nc, const LsqrVectors& vec, int ilast,
+                                            double v_last) {
+    double *v = vec.v, *w = vec.w, *x = vec.x;
+    const double sv = s.sv, t1 = s.t1, t2 = s.t2;
+    double dd = 0.0;
+    if (first) {
+        for (int i = d.gtid; i < nc; i += d.gthreads) w[i] = sv * (i == ilast ? v_last : v[i]);
+    } else {
+        const double irho = 1.0 / s.rho;
+        int i = d.gtid;
+        for (; i + 3 * d.gthreads < nc; i += 4 * d.gthreads) {   // four independent elements in flight per thread
+            double wi[4], vi[4], xi[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int k = i + q * d.gthreads;
+                wi[q] = w[k];
+                vi[q] = k == ilast ? v_last : v[k];
+                xi[q] = x[k];
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int k = i + q * d.gthreads;
+                const double dk = wi[q] * irho;
+                dd += dk * dk;
+                x[k] = xi[q] + t1 * wi[q];
+                w[k] = sv * vi[q] + t2 * wi[q];
+            }
+        }
+        for (; i < nc; i += d.gthreads) {
+            double wi = w[i];
+            double dk = wi * irho;
+            dd += dk * dk;
+            x[i] += t1 * wi;
+            w[i] = sv * (i == ilast ? v_last : v[i]) + t2 * wi;
+        }
+    }
+    block_partial(d, 4, dd);
+}
+
 // The whole LSQR iteration (Paige-Saunders) for one operator; called by every thread of the CTAs that share the problem
 // (the whole grid, one cluster, or -- batched launches -- one cluster / CTA per problem).  zero_below: right-hand sides of
 // norm <= zero_below give x = 0 without iterating (ConicProgram.jl:369 tests 1e-4 on the reverse seed; -1 disables).
@@ -710,140 +900,36 @@ template <bool STREAM, bool PSD, bool SM>
 __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rhs, const LsqrParams prm, const LsqrVectors vec,
                           const double zero_below) {
     const int nr = o.nrows, nc = o.ncols;
-    double *u = vec.u, *v = vec.v, *w = vec.w, *x = vec.x;
+    double *u = vec.u, *v = vec.v;
 
     // private copies of the last entries of u and v (see conic_apply)
     double u_last = nr > 0 ? rhs[nr - 1] : 0.0, v_last = 0.0;
-    // u = b, beta = ||b||
-    {
-        double acc = 0.0;
-        for (int i = d.gtid; i < nr; i += d.gthreads) {
-            double t = rhs[i];
-            u[i] = t;
-            acc += t * t;
-        }
-        for (int i = d.gtid; i < nc; i += d.gthreads) {
-            x[i] = 0.0;
-            v[i] = 0.0;
-            w[i] = 0.0;
-        }
-        block_partial(d, 0, acc);
-    }
+    lsqr_init(d, nr, nc, rhs, vec);
     d.sync();
-    double beta = sqrt(total_of(d, 0));
-    if (beta <= zero_below) beta = 0.0;
-    double alpha = 0.0;
-    double su = 1.0, sv = 1.0;  // true u = su * u_mem, true v = sv * v_mem
-    int istop = 0;
-    long long itn = 0;
-    double anorm = 0, acond = 0, ddnorm = 0, res2 = 0, xnorm = 0, xxnorm = 0, z = 0, sn2 = 0, cs2 = -1.0;
-    double rnorm = beta, arnorm = 0.0;
-    if (beta > 0) {
-        su = 1.0 / beta;
-        alpha = sqrt(op_apply<STREAM, PSD, SM>(d, o, true, u, su, v, 0.0, 2, u_last, v_last));   // v_mem = A' u_true
-    }
-    if (alpha > 0) sv = 1.0 / alpha;
-    arnorm = alpha * beta;
-    const double bnorm = beta;
-    double rhobar = alpha, phibar = beta;
-    const double ctol = prm.conlim > 0 ? 1.0 / prm.conlim : 0.0;
-    double t1 = 0, t2 = 0, rho = 1.0, tau = 0;
+    LsqrScalars s;
+    const bool op1 = s.start(total_of(d, 0), zero_below);
+    s.first_alpha(op1 ? op_apply<STREAM, PSD, SM>(d, o, true, u, s.su, v, 0.0, 2, u_last, v_last) : 0.0);  // v_mem = A' u_true
     bool first = true;
     bool pending = false;  // an iteration whose x/w update and stop tests are still to be applied
 
-    if (arnorm != 0.0) {
+    if (s.arnorm != 0.0) {
         while (true) {
-            // ---- deferred vector update of the previous iteration (or w = v at start), fused with the next
-            //      bidiagonalisation product
-            double dd = 0.0;
-            // (conic operator: the last entry of v is read from its register copy, see conic_apply)
-            const int ilast = o.kind == 1 ? nc - 1 : -1;
-            if (first) {
-                for (int i = d.gtid; i < nc; i += d.gthreads) w[i] = sv * (i == ilast ? v_last : v[i]);
-            } else {
-                const double irho = 1.0 / rho;
-                int i = d.gtid;
-                for (; i + 3 * d.gthreads < nc; i += 4 * d.gthreads) {   // four independent elements in flight per thread
-                    double wi[4], vi[4], xi[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int k = i + q * d.gthreads;
-                        wi[q] = w[k];
-                        vi[q] = k == ilast ? v_last : v[k];
-                        xi[q] = x[k];
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int k = i + q * d.gthreads;
-                        const double dk = wi[q] * irho;
-                        dd += dk * dk;
-                        x[k] = xi[q] + t1 * wi[q];
-                        w[k] = sv * vi[q] + t2 * wi[q];
-                    }
-                }
-                for (; i < nc; i += d.gthreads) {
-                    double wi = w[i];
-                    double dk = wi * irho;
-                    dd += dk * dk;
-                    x[i] += t1 * wi;
-                    w[i] = sv * (i == ilast ? v_last : v[i]) + t2 * wi;
-                }
-            }
-            block_partial(d, 4, dd);
-            const bool more = itn < prm.maxiter;
+            // deferred vector update of the previous iteration (or w = v at start), fused with the next
+            // bidiagonalisation product (conic operator: the last entry of v is read from its register copy, see conic_apply)
+            lsqr_update(d, s, first, nc, vec, o.kind == 1 ? nc - 1 : -1, v_last);
+            const bool more = s.itn < prm.maxiter;
             double unorm2 = 0.0;
-            if (more) unorm2 = op_apply<STREAM, PSD, SM>(d, o, false, v, sv, u, -alpha * su, 0, v_last, u_last);  // u_mem = A v_true - alpha u_true
+            if (more) unorm2 = op_apply<STREAM, PSD, SM>(d, o, false, v, s.sv, u, -s.alpha * s.su, 0, v_last, u_last);  // u_mem = A v_true - alpha u_true
             else d.sync();  // the partial sums of the update above
             if (pending) {
-                ddnorm += total_of(d, 4);
-                acond = anorm * sqrt(ddnorm);
-                const double test1 = rnorm / bnorm;
-                const double test2 = arnorm / (anorm * rnorm);
-                const double test3 = 1.0 / acond;
-                const double t1_ = test1 / (1.0 + anorm * xnorm / bnorm);
-                const double rtol = prm.btol + prm.atol * anorm * xnorm / bnorm;
-                if (itn >= prm.maxiter) istop = 7;
-                if (1.0 + test3 <= 1.0) istop = 6;
-                if (1.0 + test2 <= 1.0) istop = 5;
-                if (1.0 + t1_ <= 1.0) istop = 4;
-                if (test3 <= ctol) istop = 3;
-                if (test2 <= prm.atol) istop = 2;
-                if (test1 <= rtol) istop = 1;
+                s.stop_tests(total_of(d, 4), prm);
                 pending = false;
             }
             first = false;
-            if (istop > 0 || !more) break;
-            itn += 1;
-            beta = sqrt(unorm2);
-            if (beta > 0) {
-                su = 1.0 / beta;
-                anorm = sqrt(anorm * anorm + alpha * alpha + beta * beta);
-                alpha = sqrt(op_apply<STREAM, PSD, SM>(d, o, true, u, su, v, -beta * sv, 2, u_last, v_last));  // v_mem = A' u_true - beta v_true
-                sv = alpha > 0 ? 1.0 / alpha : 1.0;
-            } else {
-                su = 1.0;  // u_mem is exactly zero
-            }
-            // plane rotations (damp = 0)
-            const double rhobar1 = rhobar;
-            rho = hypot(rhobar1, beta);
-            const double cs = rhobar1 / rho, sn = beta / rho;
-            const double theta = sn * alpha;
-            rhobar = -cs * alpha;
-            const double phi = cs * phibar;
-            phibar = sn * phibar;
-            tau = sn * phi;
-            t1 = phi / rho;
-            t2 = -theta / rho;
-            const double delta = sn2 * rho, gambar = -cs2 * rho, rhs_ = phi - delta * z;
-            const double zbar = rhs_ / gambar;
-            xnorm = sqrt(xxnorm + zbar * zbar);
-            const double gamma = hypot(gambar, theta);
-            cs2 = gambar / gamma;
-            sn2 = theta / gamma;
-            z = rhs_ / gamma;
-            xxnorm += z * z;
-            rnorm = sqrt(phibar * phibar + res2);
-            arnorm = alpha * fabs(tau);
+            if (s.istop > 0 || !more) break;
+            if (s.next_beta(unorm2))
+                s.next_alpha(op_apply<STREAM, PSD, SM>(d, o, true, u, s.su, v, -s.beta * s.sv, 2, u_last, v_last));  // v_mem = A' u_true - beta v_true
+            s.rotate();
             pending = true;
         }
     }
@@ -855,21 +941,14 @@ __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rh
         g_prof_n = 0;
     }
 #endif
-    if (d.gtid == 0) {
-        vec.stats[0] = (double)istop;
-        vec.stats[1] = (double)itn;
-        vec.stats[2] = rnorm;
-        vec.stats[3] = arnorm;
-        vec.stats[4] = anorm;
-        vec.stats[5] = acond;
-        vec.stats[6] = xnorm;
-    }
+    if (d.gtid == 0) s.write_stats(vec.stats);
 }
 
 template <int THREADS, int MINB, bool CLUSTER, bool STREAM, bool PSD>
 __global__ void __launch_bounds__(THREADS, MINB) lsqr_kernel_t(OpArgs o, const double* __restrict__ rhs, LsqrParams prm,
                                                                LsqrVectors vec) {
     __shared__ double red[64];
+    // (Dev built in place in the persistent kernels: from make_dev, ptxas allocates their registers worse and spills more)
     Dev d{cg::this_grid(), vec.partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
           (int)(blockDim.x >> 5), (int)gridDim.x, (int)(blockIdx.x * blockDim.x + threadIdx.x),
           (int)(gridDim.x * blockDim.x), CLUSTER};
@@ -901,9 +980,7 @@ __global__ void __launch_bounds__(CL_THREADS, 1) lsqr_batch_kernel(const OpArgs*
 __global__ void __launch_bounds__(LSQR_THREADS) conic_M_kernel(ConicOpView op, int transpose, const double* t, double* out,
                                                               double* partials) {
     __shared__ double red[64];
-    Dev d{cg::this_grid(), partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
-          (int)(blockDim.x >> 5), (int)gridDim.x, (int)(blockIdx.x * blockDim.x + threadIdx.x),
-          (int)(gridDim.x * blockDim.x)};
+    Dev d = make_dev(partials, red, (int)gridDim.x);
     double last = 0.0, norm2 = 0.0;
     conic_apply<false, true>(d, op, transpose != 0, t, 1.0, out, 0.0, 0, __ldcg(t + op.n + op.m), last, norm2);
 }
@@ -911,34 +988,26 @@ __global__ void __launch_bounds__(LSQR_THREADS) conic_M_kernel(ConicOpView op, i
 __global__ void __launch_bounds__(LSQR_THREADS) conic_dpi_kernel(ConicOpView op, int transpose, const double* t, double* out,
                                                                 double* partials) {
     __shared__ double red[64];
-    Dev d{cg::this_grid(), partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
-          (int)(blockDim.x >> 5), (int)gridDim.x, (int)(blockIdx.x * blockDim.x + threadIdx.x),
-          (int)(gridDim.x * blockDim.x)};
+    Dev d = make_dev(partials, red, (int)gridDim.x);
     dpi_apply<true>(d, op, t, out, transpose != 0);
 }
 
 
 // ================================================================================================================
-// Streaming LSQR for LARGE conic operators (working set beyond L2): the same iteration as lsqr_kernel, but every
+// Streaming LSQR for LARGE conic operators (working set beyond L2): the same iteration as lsqr_body, but every
 // phase is its own kernel at full occupancy (the persistent kernel is capped at a few hundred CTAs by grid.sync and
-// its register footprint, far too few loads in flight to cover HBM latency).  All Golub-Kahan scalars, the stop
-// tests and the `done` flag live in a device struct: the host only enqueues iterations in batches and looks at the
-// flag between batches; kernels of an iteration after convergence return at once.  Same arithmetic and the same
-// deterministic reductions (per-CTA partials, fixed-order sums) as the persistent kernel.  No PSD cones here.
+// its register footprint, far too few loads in flight to cover HBM latency).  The LsqrScalars and the `done` flag
+// live in a device struct: the host only enqueues iterations in batches and looks at the flag between batches;
+// kernels of an iteration after convergence return at once.  The phases call the persistent kernel's own code
+// (LsqrScalars, lsqr_init, lsqr_update, the conic row-block phases) with the same deterministic reductions (per-CTA
+// partials, fixed-order sums).  No PSD cones here.
 struct LsqrState {
-    double alpha, beta, su, sv, rhobar, phibar, rho, t1, t2, tau;
-    double anorm, acond, ddnorm, res2, xnorm, xxnorm, z, sn2, cs2, rnorm, arnorm, bnorm;
+    LsqrScalars sc;
     double op_src, op_dst;  // scalars of the operator application in flight: dst = op_src * OP(src) + op_dst * dst
-    long long itn;
-    int istop, first, pending, done, more, do_op1;
+    int first, pending, done, more, do_op1;
 };
 
 constexpr int ST_THREADS = 256;
-#define ST_DEV(partials)                                                                                          \
-    __shared__ double red[64];                                                                                    \
-    Dev d{cg::this_grid(), partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),     \
-          (int)(blockDim.x >> 5), ST_STRIDE, (int)(blockIdx.x * blockDim.x + threadIdx.x),                        \
-          (int)(gridDim.x * blockDim.x)}
 
 __device__ double st_total(const double* partials, int slot, int stride, int count, double* red) {
     // fixed-order sum of `count` CTA partials by one 256-thread block
@@ -986,20 +1055,10 @@ __device__ void st_total3(const double* partials, int stride, int s0, int c0, in
     }
 }
 
-__global__ void __launch_bounds__(ST_THREADS) st_init_kernel(int nr, int nc, const double* __restrict__ rhs, LsqrVectors vec, LsqrState* S) {
-    ST_DEV(vec.partials);
-    double acc = 0.0;
-    for (int i = d.gtid; i < nr; i += d.gthreads) {
-        const double t = rhs[i];
-        vec.u[i] = t;
-        acc += t * t;
-    }
-    for (int i = d.gtid; i < nc; i += d.gthreads) {
-        vec.x[i] = 0.0;
-        vec.v[i] = 0.0;
-        vec.w[i] = 0.0;
-    }
-    block_partial(d, 0, acc);
+__global__ void __launch_bounds__(ST_THREADS) st_init_kernel(int nr, int nc, const double* __restrict__ rhs, LsqrVectors vec) {
+    __shared__ double red[64];
+    Dev d = make_dev(vec.partials, red, ST_STRIDE);
+    lsqr_init(d, nr, nc, rhs, vec);
 }
 
 // after st_init_kernel: beta, su; sets up v = A' u (op1 with s_dst = 0)
@@ -1008,15 +1067,8 @@ __global__ void __launch_bounds__(ST_THREADS) st_init_fin_kernel(LsqrVectors vec
     const double t0 = st_total(vec.partials, 0, stride, cnt0, red);
     if (threadIdx.x == 0) {
         LsqrState s{};
-        s.beta = sqrt(t0);
-        s.su = 1.0;
-        s.sv = 1.0;
-        s.cs2 = -1.0;
-        s.rho = 1.0;
-        s.rnorm = s.beta;
-        s.do_op1 = s.beta > 0 ? 1 : 0;
-        if (s.beta > 0) s.su = 1.0 / s.beta;
-        s.op_src = s.su;
+        s.do_op1 = s.sc.start(t0, -1.0);
+        s.op_src = s.sc.su;
         s.op_dst = 0.0;
         s.first = 1;
         *S = s;
@@ -1026,29 +1078,18 @@ __global__ void __launch_bounds__(ST_THREADS) st_init_fin_kernel(LsqrVectors vec
 // x, w update of the previous iteration (LSQR's deferred vector update), ||w / rho||^2 into slot 4
 __global__ void __launch_bounds__(ST_THREADS) st_update_kernel(int nc, LsqrVectors vec, LsqrState* S) {
     if (S->done) return;
-    ST_DEV(vec.partials);
-    const double sv = S->sv, t1 = S->t1, t2 = S->t2;
-    double dd = 0.0;
-    if (S->first) {
-        for (int i = d.gtid; i < nc; i += d.gthreads) vec.w[i] = sv * vec.v[i];
-    } else {
-        const double irho = 1.0 / S->rho;
-        for (int i = d.gtid; i < nc; i += d.gthreads) {
-            const double wi = vec.w[i];
-            const double dk = wi * irho;
-            dd += dk * dk;
-            vec.x[i] += t1 * wi;
-            vec.w[i] = sv * vec.v[i] + t2 * wi;
-        }
-    }
-    block_partial(d, 4, dd);
+    __shared__ double red[64];
+    Dev d = make_dev(vec.partials, red, ST_STRIDE);
+    const LsqrScalars s = S->sc;
+    lsqr_update(d, s, S->first, nc, vec, -1, 0.0);
 }
 
 // ---- M src (non-transposed), phase 1: wc = Dpi src2
 __global__ void __launch_bounds__(ST_THREADS) st_dpi_kernel(ConicOpView op, const double* __restrict__ y, double* out, int transpose,
                                                             const LsqrState* S, int which) {
     if (S->done || (which == 0 ? !S->more : !S->do_op1)) return;
-    ST_DEV(nullptr);
+    __shared__ double red[64];
+    Dev d = make_dev(nullptr, red, ST_STRIDE);
     dpi_apply<false>(d, op, y, out, transpose != 0);
 }
 
@@ -1056,37 +1097,11 @@ __global__ void __launch_bounds__(ST_THREADS) st_dpi_kernel(ConicOpView op, cons
 __global__ void __launch_bounds__(SP_THREADS, 8) st_M_rows_kernel(ConicOpView op, const double* __restrict__ src, double* dst, double* partials,
                                                                const LsqrState* S) {
     if (S->done || !S->more) return;
-    ST_DEV(partials);
-    const int n = op.n, m = op.m;
-    const double s_src = S->op_src, s_dst = S->op_dst;
-    const double t3 = __ldcg(src + n + m);
+    __shared__ double red[64], prod[ST_CHUNK];
+    Dev d = make_dev(partials, red, ST_STRIDE);
     double acc = 0.0, dotacc = 0.0;
-    const int nbt = op.At.nblk;
-    __shared__ double prod[ST_CHUNK];
-    spmv_stream<SP_THREADS, ST_NPT, 0>(
-        (int)blockIdx.x, (int)gridDim.x,
-        nbt + op.A.nblk, prod, red,
-        [&](int b, const CsrView*& A, const double*& x, int& lb) {
-            if (b < nbt) { A = &op.At; x = op.wc; lb = b; }
-            else { A = &op.A; x = src; lb = b - nbt; }
-        },
-        [&](int b, int row) {
-            return b < nbt ? make_double4(op.c[row], dst[row], __ldcg(src + row), 0.0)
-                           : make_double4(__ldcg(op.wc + row), __ldcg(src + n + row), op.b[row], dst[n + row]);
-        },
-        [&](int b, int row, double t, const double4& o) {
-            if (b < nbt) {  // rows 0..n-1:  (A' wc)_j + c_j t3
-                t = (t + o.x * t3) * s_src + s_dst * o.y;
-                dst[row] = t;
-                acc += t * t;
-                dotacc += o.x * o.z;
-            } else {        // rows n..n+m-1:  -(A t1)_i + t2_i - wc_i + b_i t3
-                t = (-t + o.y - o.x + o.z * t3) * s_src + s_dst * o.w;
-                dst[n + row] = t;
-                acc += t * t;
-                dotacc += o.z * o.x;
-            }
-        });
+    conic_M_rows<SP_THREADS, ST_NPT, 0>(op, (int)blockIdx.x, (int)gridDim.x, prod, red, src, op.wc, src, __ldcg(src + op.n + op.m),
+                                        S->op_src, dst, S->op_dst, acc, dotacc);
     block_partial(d, 0, acc);
     block_partial(d, 1, dotacc);
 }
@@ -1107,40 +1122,19 @@ __global__ void __launch_bounds__(ST_THREADS) st_mid_kernel(int N, LsqrVectors v
         unorm2 += last * last;
     }
     if (s.pending) {
-        s.ddnorm += tot4;
-        s.acond = s.anorm * sqrt(s.ddnorm);
-        const double test1 = s.rnorm / s.bnorm;
-        const double test2 = s.arnorm / (s.anorm * s.rnorm);
-        const double test3 = 1.0 / s.acond;
-        const double t1_ = test1 / (1.0 + s.anorm * s.xnorm / s.bnorm);
-        const double rtol = prm.btol + prm.atol * s.anorm * s.xnorm / s.bnorm;
-        const double ctol = prm.conlim > 0 ? 1.0 / prm.conlim : 0.0;
-        if (s.itn >= prm.maxiter) s.istop = 7;
-        if (1.0 + test3 <= 1.0) s.istop = 6;
-        if (1.0 + test2 <= 1.0) s.istop = 5;
-        if (1.0 + t1_ <= 1.0) s.istop = 4;
-        if (test3 <= ctol) s.istop = 3;
-        if (test2 <= prm.atol) s.istop = 2;
-        if (test1 <= rtol) s.istop = 1;
+        s.sc.stop_tests(tot4, prm);
         s.pending = 0;
     }
     s.first = 0;
-    if (s.istop > 0 || !s.more) {
+    if (s.sc.istop > 0 || !s.more) {
         s.done = 1;
         *S = s;
         return;
     }
-    s.itn += 1;
-    s.beta = sqrt(unorm2);
-    if (s.beta > 0) {
-        s.su = 1.0 / s.beta;
-        s.anorm = sqrt(s.anorm * s.anorm + s.alpha * s.alpha + s.beta * s.beta);
-        s.op_src = s.su;
-        s.op_dst = -s.beta * s.sv;
-        s.do_op1 = 1;
-    } else {
-        s.su = 1.0;
-        s.do_op1 = 0;
+    s.do_op1 = s.sc.next_beta(unorm2);
+    if (s.do_op1) {
+        s.op_src = s.sc.su;
+        s.op_dst = -s.sc.beta * s.sc.sv;
     }
     *S = s;
 }
@@ -1149,20 +1143,10 @@ __global__ void __launch_bounds__(ST_THREADS) st_mid_kernel(int N, LsqrVectors v
 __global__ void __launch_bounds__(SP_THREADS, 8) st_Mt_A_kernel(ConicOpView op, const double* __restrict__ src, double* partials,
                                                              const LsqrState* S) {
     if (S->done || !S->do_op1) return;
-    ST_DEV(partials);
-    const int n = op.n, m = op.m;
-    const double u3 = __ldcg(src + n + m);
+    __shared__ double red[64], prod[ST_CHUNK];
+    Dev d = make_dev(partials, red, ST_STRIDE);
     double dotacc = 0.0;
-    __shared__ double prod[ST_CHUNK];
-    spmv_stream<SP_THREADS, ST_NPT, 0>(
-        (int)blockIdx.x, (int)gridDim.x,
-        op.A.nblk, prod, red,
-        [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.A; x = src; lb = b; },
-        [&](int, int row) { return make_double4(__ldcg(src + n + row), op.b[row], 0.0, 0.0); },
-        [&](int, int row, double t, const double4& o) {
-            op.wc[row] = t - o.x - o.y * u3;
-            dotacc += o.y * o.x;
-        });
+    conic_Mt_A<SP_THREADS, ST_NPT, 0>(op, (int)blockIdx.x, (int)gridDim.x, prod, red, src, src, __ldcg(src + op.n + op.m), dotacc);
     block_partial(d, 3, dotacc);
 }
 
@@ -1170,29 +1154,11 @@ __global__ void __launch_bounds__(SP_THREADS, 8) st_Mt_A_kernel(ConicOpView op, 
 __global__ void __launch_bounds__(SP_THREADS, 8) st_Mt_rows_kernel(ConicOpView op, const double* __restrict__ src, double* dst, double* partials,
                                                                 const LsqrState* S) {
     if (S->done || !S->do_op1) return;
-    ST_DEV(partials);
-    const int n = op.n, m = op.m;
-    const double s_src = S->op_src, s_dst = S->op_dst;
-    const double u3 = __ldcg(src + n + m);
-    const double* r2 = op.wc + m;
+    __shared__ double red[64], prod[ST_CHUNK];
+    Dev d = make_dev(partials, red, ST_STRIDE);
     double acc = 0.0, dotacc = 0.0;
-    __shared__ double prod[ST_CHUNK];
-    spmv_stream<SP_THREADS, ST_NPT, 0>(
-        (int)blockIdx.x, (int)gridDim.x,
-        op.At.nblk, prod, red,
-        [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.At; x = src + n; lb = b; },
-        [&](int, int row) { return make_double4(op.c[row], dst[row], __ldcg(src + row), 0.0); },
-        [&](int, int row, double t, const double4& o) {
-            t = (-t - o.x * u3) * s_src + s_dst * o.y;
-            dst[row] = t;
-            acc += t * t;
-            dotacc += o.x * o.z;
-        });
-    for (int i = d.gtid; i < m; i += d.gthreads) {
-        const double t = (__ldcg(r2 + i) + __ldcg(src + n + i)) * s_src + s_dst * dst[n + i];
-        dst[n + i] = t;
-        acc += t * t;
-    }
+    conic_Mt_rows<SP_THREADS, ST_NPT, 0>(op, (int)blockIdx.x, (int)gridDim.x, prod, red, src, src + op.n, __ldcg(src + op.n + op.m),
+                                         S->op_src, dst, S->op_dst, acc, dotacc);
     block_partial(d, 2, acc);
     block_partial(d, 5, dotacc);
 }
@@ -1206,64 +1172,27 @@ __global__ void __launch_bounds__(ST_THREADS) st_end_kernel(int N, LsqrVectors v
     st_total3(vec.partials, stride, 2, cnt_rows, 3, cnt_a, 5, cnt_rows, red, tot2, tot3, tot5);
     if (threadIdx.x != 0) return;
     LsqrState s = *S;
+    double alpha2 = 0.0;
     if (s.do_op1) {
         const double last = (tot3 + tot5) * s.op_src + s.op_dst * vec.v[N - 1];
         vec.v[N - 1] = last;
-        s.alpha = sqrt(tot2 + last * last);
-        if (startup) {
-            if (s.alpha > 0) s.sv = 1.0 / s.alpha;
-        } else {
-            s.sv = s.alpha > 0 ? 1.0 / s.alpha : 1.0;
-        }
+        alpha2 = tot2 + last * last;
     }
     if (startup) {
-        s.arnorm = s.alpha * s.beta;
-        s.bnorm = s.beta;
-        s.rhobar = s.alpha;
-        s.phibar = s.beta;
-        s.more = s.itn < prm.maxiter ? 1 : 0;
-        s.op_src = s.sv;
-        s.op_dst = -s.alpha * s.su;
-        if (s.arnorm == 0.0) s.done = 1;
-        *S = s;
-        return;
+        s.sc.first_alpha(alpha2);
+        if (s.sc.arnorm == 0.0) s.done = 1;
+    } else {
+        if (s.do_op1) s.sc.next_alpha(alpha2);
+        s.sc.rotate();
+        s.pending = 1;
     }
-    const double rhobar1 = s.rhobar;
-    s.rho = hypot(rhobar1, s.beta);
-    const double cs = rhobar1 / s.rho, sn = s.beta / s.rho;
-    const double theta = sn * s.alpha;
-    s.rhobar = -cs * s.alpha;
-    const double phi = cs * s.phibar;
-    s.phibar = sn * s.phibar;
-    s.tau = sn * phi;
-    s.t1 = phi / s.rho;
-    s.t2 = -theta / s.rho;
-    const double delta = s.sn2 * s.rho, gambar = -s.cs2 * s.rho, rhs_ = phi - delta * s.z;
-    const double zbar = rhs_ / gambar;
-    s.xnorm = sqrt(s.xxnorm + zbar * zbar);
-    const double gamma = hypot(gambar, theta);
-    s.cs2 = gambar / gamma;
-    s.sn2 = theta / gamma;
-    s.z = rhs_ / gamma;
-    s.xxnorm += s.z * s.z;
-    s.rnorm = sqrt(s.phibar * s.phibar + s.res2);
-    s.arnorm = s.alpha * fabs(s.tau);
-    s.pending = 1;
-    s.more = s.itn < prm.maxiter ? 1 : 0;
-    s.op_src = s.sv;
-    s.op_dst = -s.alpha * s.su;
+    s.more = s.sc.itn < prm.maxiter ? 1 : 0;
+    s.op_src = s.sc.sv;
+    s.op_dst = -s.sc.alpha * s.sc.su;
     *S = s;
 }
 
-__global__ void st_stats_kernel(const LsqrState* S, double* stats) {
-    stats[0] = (double)S->istop;
-    stats[1] = (double)S->itn;
-    stats[2] = S->rnorm;
-    stats[3] = S->arnorm;
-    stats[4] = S->anorm;
-    stats[5] = S->acond;
-    stats[6] = S->xnorm;
-}
+__global__ void st_stats_kernel(const LsqrState* S, double* stats) { S->sc.write_stats(stats); }
 
 CsrView view_of(const DevBuf& rp, const DevBuf& ci, const DevBuf& v, int64_t nrows, int64_t ncols,
                 const DevBuf* blk = nullptr, int64_t nblk = 0, const DevBuf* sval = nullptr, const DevBuf* scol = nullptr,
@@ -1335,6 +1264,23 @@ static int coop_grid(diffopt_b200_ctx* ctx, const void* kernel, int64_t work) {
 constexpr int64_t CL_MAX_WORK = (int64_t)1 << 20;
 constexpr int64_t CL_CLUSTER_WORK = (int64_t)512 << 10;
 
+// launch of `grid` CL_THREADS-thread CTAs in thread-block clusters of `cs`; `at` stores the cluster attribute
+static cudaLaunchConfig_t cluster_config(unsigned grid, unsigned cs, size_t dyn, cudaStream_t stream, cudaLaunchAttribute& at) {
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(CL_THREADS);
+    cfg.dynamicSmemBytes = dyn;
+    cfg.stream = stream;
+    at = cudaLaunchAttribute{};
+    at.id = cudaLaunchAttributeClusterDimension;
+    at.val.clusterDim.x = cs;
+    at.val.clusterDim.y = 1;
+    at.val.clusterDim.z = 1;
+    cfg.attrs = &at;
+    cfg.numAttrs = 1;
+    return cfg;
+}
+
 static int cluster_size_for(diffopt_b200_ctx* ctx, const void* kernel) {
     static int cached = -1;  // per process; every B200 in a box is the same part
     if (cached >= 0) return cached;
@@ -1343,17 +1289,8 @@ static int cluster_size_for(diffopt_b200_ctx* ctx, const void* kernel) {
         cudaGetLastError();
     }
     for (int cs : {16, 8}) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)cs);
-        cfg.blockDim = dim3(CL_THREADS);
-        cfg.dynamicSmemBytes = CL_CHUNK * sizeof(double);
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = (unsigned)cs;
-        at[0].val.clusterDim.y = 1;
-        at[0].val.clusterDim.z = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
+        cudaLaunchAttribute at;
+        const cudaLaunchConfig_t cfg = cluster_config((unsigned)cs, (unsigned)cs, CL_CHUNK * sizeof(double), nullptr, at);
         int n = 0;
         if (cudaOccupancyMaxActiveClusters(&n, kernel, &cfg) == cudaSuccess && n >= 1) {
             cached = cs;
@@ -1414,26 +1351,16 @@ static int32_t lsqr_launch(diffopt_b200_ctx* ctx, OpArgs& o, int64_t work, const
             pick(o.adj, ctx->lsqr_mat, !fwd_is_t);
         }
     }
-    DO_CUDA(ctx, wk.tmp.reserve(d * (size_t)NSLOTS * (size_t)grid));
+    DO_CUDA(ctx, wk.tmp.reserve(d * (size_t)LSQR_NSLOTS * (size_t)grid));
     DO_CUDA(ctx, wk.scal.reserve(d * 8));
-    DO_CUDA(ctx, cudaMemsetAsync(wk.tmp.ptr, 0, d * (size_t)NSLOTS * (size_t)grid, ctx->stream));
+    DO_CUDA(ctx, cudaMemsetAsync(wk.tmp.ptr, 0, d * (size_t)LSQR_NSLOTS * (size_t)grid, ctx->stream));
     LsqrVectors vec{wk.u.as<double>(), wk.v.as<double>(), wk.w.as<double>(), x_dev, wk.tmp.as<double>(),
                     wk.scal.as<double>()};
     void* args[] = {&o, (void*)&rhs_dev, &prm, &vec};
     DO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     if (variant == 1) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)cs);
-        cfg.blockDim = dim3(CL_THREADS);
-        cfg.dynamicSmemBytes = dyn;
-        cfg.stream = ctx->stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = (unsigned)cs;
-        at[0].val.clusterDim.y = 1;
-        at[0].val.clusterDim.z = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
+        cudaLaunchAttribute at;
+        const cudaLaunchConfig_t cfg = cluster_config((unsigned)cs, (unsigned)cs, dyn, ctx->stream, at);
         DO_CUDA(ctx, cudaLaunchKernelExC(&cfg, k_cluster, args));
     } else if (variant == 2) {
         DO_CUDA(ctx, cudaLaunchCooperativeKernel(k_gstream, dim3(grid), dim3(CL_THREADS), args, dyn, ctx->stream));
@@ -1474,7 +1401,7 @@ static int32_t lsqr_stream_conic(diffopt_b200_ctx* ctx, const double* rhs_dev, L
     DO_CUDA(ctx, wk.v.reserve(dsz * (size_t)N));
     DO_CUDA(ctx, wk.w.reserve(dsz * (size_t)N));
     const int stride = ST_STRIDE;
-    DO_CUDA(ctx, wk.tmp.reserve(dsz * (size_t)NSLOTS * (size_t)stride));
+    DO_CUDA(ctx, wk.tmp.reserve(dsz * (size_t)LSQR_NSLOTS * (size_t)stride));
     DO_CUDA(ctx, wk.scal.reserve(dsz * 8 + sizeof(LsqrState) + 64));
     double* stats = wk.scal.as<double>();
     LsqrState* S = reinterpret_cast<LsqrState*>(stats + 8);
@@ -1498,7 +1425,7 @@ static int32_t lsqr_stream_conic(diffopt_b200_ctx* ctx, const double* rhs_dev, L
     const unsigned g_trows = blocks_spmv(std::max<int64_t>(cs.A.t_nblk, ((int64_t)m + SP_THREADS * 8 - 1) / (SP_THREADS * 8)));
     cudaStream_t st = ctx->stream;
     DO_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
-    st_init_kernel<<<g_vec, ST_THREADS, 0, st>>>(N, N, rhs_dev, vec, S);
+    st_init_kernel<<<g_vec, ST_THREADS, 0, st>>>(N, N, rhs_dev, vec);
     st_init_fin_kernel<<<1, ST_THREADS, 0, st>>>(vec, stride, (int)g_vec, S);
     auto apply_Mt = [&](int startup) {  // v = su M' u + op_dst v
         st_Mt_A_kernel<<<g_a, SP_THREADS, 0, st>>>(op, vec.u, vec.partials, S);
@@ -1560,7 +1487,7 @@ static int32_t conic_small_launch(diffopt_b200_ctx* ctx, const void* kernel, con
     ConicOpView op = conic_view(ctx);
     int64_t work = s.A.nnz * 2 + s.n + 2 * s.m + s.psd_sumd2 * 8;
     int grid = coop_grid(ctx, kernel, work);
-    DO_CUDA(ctx, ctx->lsqr.tmp.reserve(sizeof(double) * (size_t)NSLOTS * (size_t)grid));
+    DO_CUDA(ctx, ctx->lsqr.tmp.reserve(sizeof(double) * (size_t)LSQR_NSLOTS * (size_t)grid));
     double* partials = ctx->lsqr.tmp.as<double>();
     int tr = transpose ? 1 : 0;
     void* args[] = {&op, &tr, (void*)&t_dev, &out_dev, &partials};
@@ -1577,10 +1504,11 @@ int32_t conic_apply_dpi(diffopt_b200_ctx* ctx, const double* t_dev, bool transpo
 }
 
 // Lock-step batch of conic problems (diffopt_b200_conic_batch_reverse): one persistent kernel, problem p on the C CTAs of
-// cluster p.  `work` holds one region of `stride` doubles per problem: [rhs (N+1) | x (N) | u (N) | v (N) | w (N) |
-// partials (NSLOTS * C) | stats (8)].  With C == 1 and `stage` the gather vectors are staged in shared memory.
-int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& states, int C, bool stage, double* work, size_t stride,
-                             LsqrParams prm, double zero_below, DevBuf& ops_buf, DevBuf& vecs_buf, DevBuf& rhs_buf) {
+// cluster p.  `work` holds one region per problem, laid out by L.  With C == 1 and `stage` the gather vectors are staged
+// in shared memory.
+int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& states, int C, bool stage, double* work,
+                             const LsqrBatchLayout& L, LsqrParams prm, double zero_below, DevBuf& ops_buf, DevBuf& vecs_buf,
+                             DevBuf& rhs_buf) {
     const int B = (int)states.size();
     if (B == 0) return 0;
     const int n = (int)states[0].n, m = (int)states[0].m, N = n + m + 1;
@@ -1596,10 +1524,9 @@ int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& sta
         o.nrows = o.ncols = N;
         ops[(size_t)p] = o;
         std::swap(ctx->conic, states[(size_t)p]);
-        double* base = work + (size_t)p * stride;
+        double* base = work + (size_t)p * L.stride;
         rhs[(size_t)p] = base;
-        vecs[(size_t)p] = LsqrVectors{base + (N + 1) + N, base + (N + 1) + 2 * (size_t)N, base + (N + 1) + 3 * (size_t)N, base + (N + 1),
-                                      base + (N + 1) + 4 * (size_t)N, base + (N + 1) + 4 * (size_t)N + (size_t)NSLOTS * C};
+        vecs[(size_t)p] = LsqrVectors{base + L.u, base + L.v, base + L.w, base + L.x, base + L.partials, base + L.stats};
     }
     DO_CUDA(ctx, ops_buf.reserve(sizeof(OpArgs) * (size_t)B));
     DO_CUDA(ctx, vecs_buf.reserve(sizeof(LsqrVectors) * (size_t)B));
@@ -1618,18 +1545,8 @@ int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& sta
     const double* const* drhs = rhs_buf.as<const double*>();
     const LsqrVectors* dvecs = vecs_buf.as<LsqrVectors>();
     void* args[] = {(void*)&dops, (void*)&drhs, &prm, (void*)&dvecs, &C, &zero_below};
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(B * C));
-    cfg.blockDim = dim3(CL_THREADS);
-    cfg.dynamicSmemBytes = dyn2;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = (unsigned)C;
-    at[0].val.clusterDim.y = 1;
-    at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
+    cudaLaunchAttribute at;
+    const cudaLaunchConfig_t cfg = cluster_config((unsigned)(B * C), (unsigned)C, dyn2, ctx->stream, at);
     DO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     DO_CUDA(ctx, cudaLaunchKernelExC(&cfg, kern, args));
     ctx->launches++;

@@ -4,7 +4,10 @@
 //              `lsqr(M, g)` at ConicProgram.jl:323,372 -- the dense Dpi blocks are never formed.
 // One kernel runs the whole iteration: vectors stay in L2/HBM, Golub-Kahan scalars live replicated in
 // registers, norms are reduced deterministically (per-CTA partials + fixed-order sum), grid.sync()
-// separates the phases; there is no host round-trip per iteration.
+// separates the phases; there is no host round-trip per iteration.  Large conic operators run the same
+// iteration as one kernel per phase (the streaming driver).  Every driver shares one copy of the arithmetic
+// in lsqr.cu: the scalar recurrences and stop tests (LsqrScalars), the vector initialisation and deferred
+// x / w update, and the row-block phases of M and M'.
 #pragma once
 #include "common.cuh"
 
@@ -56,10 +59,22 @@ struct LsqrParams {
     long long maxiter;
 };
 
+constexpr int LSQR_NSLOTS = 8;  // partial-sum slots per CTA
+
 struct LsqrVectors {
     double *u, *v, *w, *x;  // lengths nrows, ncols, ncols, ncols
-    double* partials;       // [NSLOTS][gridDim.x]
+    double* partials;       // [LSQR_NSLOTS][gridDim.x]
     double* stats;          // out: istop, itn, rnorm, arnorm, anorm, acond, xnorm
+};
+
+// Work region of one problem of the lock-step batch, offsets in doubles for an operator of order N solved by C CTAs:
+// rhs (N + 1) | x, u, v, w (N each) | partial sums (LSQR_NSLOTS * C) | statistics (8).  `stride` (even: every region
+// stays 16-byte aligned) separates consecutive problems.
+struct LsqrBatchLayout {
+    size_t x, u, v, w, partials, stats, stride;
+    LsqrBatchLayout(int64_t N, int C)
+        : x((size_t)N + 1), u(x + (size_t)N), v(u + (size_t)N), w(v + (size_t)N), partials(w + (size_t)N),
+          stats(partials + (size_t)LSQR_NSLOTS * C), stride((stats + 8 + 1) & ~(size_t)1) {}
 };
 
 int32_t lsqr_run_csr(diffopt_b200_ctx* ctx, const CsrDev& M, bool trans, const double* rhs_dev, LsqrParams prm,
@@ -68,8 +83,8 @@ int32_t lsqr_run_conic(diffopt_b200_ctx* ctx, const double* rhs_dev, LsqrParams 
                        double* stats_host7);
 int32_t conic_apply_M(diffopt_b200_ctx* ctx, const double* t_dev, bool transpose, double* out_dev);
 int32_t conic_apply_dpi(diffopt_b200_ctx* ctx, const double* t_dev, bool transpose, double* out_dev);
-int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& states, int C, bool stage, double* work, size_t stride,
-                             LsqrParams prm, double zero_below, DevBuf& ops_buf, DevBuf& vecs_buf, DevBuf& rhs_buf);
-constexpr int LSQR_NSLOTS = 8;  // == NSLOTS of lsqr.cu (partial-sum slots per CTA)
+int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& states, int C, bool stage, double* work,
+                             const LsqrBatchLayout& L, LsqrParams prm, double zero_below, DevBuf& ops_buf, DevBuf& vecs_buf,
+                             DevBuf& rhs_buf);
 int32_t csr_from_csc_host(diffopt_b200_ctx* ctx, int64_t nrows, int64_t ncols, const int64_t* colptr,
                           const int64_t* rowval, const double* nzval, CsrDev& out);

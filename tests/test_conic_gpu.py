@@ -522,6 +522,31 @@ def test_streaming_lsqr_matches_persistent_kernel(ctx, monkeypatch):
         assert a[1] == pytest.approx(b[1], rel=1e-5 if k in (1, 2, 3, 4, 10) else 5e-2), (k, a[1], b[1])
 
 
+@pytest.mark.parametrize("tol, istop", [(dict(atol=0.0, btol=1e-9, conlim=0.0), 1),
+                                        (dict(atol=0.0, btol=0.0, conlim=100.0), 3)])
+def test_lsqr_stop_tests_persistent_and_streaming(ctx, monkeypatch, tol, istop):
+    """LSQR's own stopping rule -- ||r|| small (istop 1), cond(M) beyond conlim (istop 3) -- through the persistent and
+    the streaming driver on a well-conditioned, consistent config-4 problem: both stop where the oracle stops, with the
+    oracle's answer.  (The oracle's acond crosses conlim = 100 between 98.7 and 103.2, so rounding cannot move the stop.)"""
+    cm = diffopt_b200.submodule("conic")
+    d = bench_data.conic_config4_conditioned(n=150, n_zero=15, n_nonneg=130, n_soc=9, soc_dim=8, nnz_per_row=5, seed=100)
+    cache = _oracle_cache(d)
+    dz = np.concatenate([d["seed"], np.zeros(d["A"].shape[0]), [-(d["x"] @ d["seed"])]])
+    kw = dict(tol, maxiter=4 * dz.size)
+    g, info = olsqr.lsqr(cache.M, dz, return_info=True, **kw)
+    assert info.istop == istop
+    for mode in ("persistent", "stream"):
+        monkeypatch.setenv("DIFFOPT_B200_LSQR", mode)
+        model = cm.ConicModel(ctx, d["A"], d["b"], d["c"], d["cone_types"], d["cone_dims"])
+        model.set_variable_primal(d["x"]); model.set_constraint_primal(d["s"]); model.set_constraint_dual(d["y"])
+        model.tolerances = kw
+        model.reverse_differentiate(d["seed"])
+        st = model.last_stats
+        assert st["istop"] == info.istop, (mode, st, info)
+        assert abs(st["itn"] - info.itn) <= max(3, info.itn // 50), (mode, st, info)
+        assert rel(model.back_grad_cache["g"], g) <= RTOL_LSQR, mode
+
+
 @pytest.mark.parametrize("ctas", [1, 4])
 @pytest.mark.parametrize("stage", ["1", "0"])
 def test_conic_lockstep_batch_matches_single_problem_solves(ctx, monkeypatch, ctas, stage):
