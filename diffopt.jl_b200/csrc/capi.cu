@@ -71,7 +71,6 @@ int32_t diffopt_b200_destroy(diffopt_b200_ctx* ctx) {
     LsqrWork& l = ctx->lsqr;
     for (DevBuf* b : {&l.u, &l.v, &l.w, &l.x, &l.tmp, &l.scal}) b->release();
     release_csr(ctx->lsqr_mat);
-    for (DevBuf* b : {&ctx->sparse.AB, &ctx->sparse.ipiv, &ctx->sparse.perm, &ctx->sparse.work}) b->release();
     sparse_mf_release(ctx);
     conic_batch_release(ctx);
     nccl_release(ctx);

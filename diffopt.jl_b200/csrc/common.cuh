@@ -89,14 +89,6 @@ struct ConicState {
     DevBuf w1, w2, w3;
 };
 
-// factorisation kept by diffopt_b200_sparse_setup (banded LU after RCM ordering)
-struct SparseBandState {
-    bool valid = false;
-    int64_t N = 0;
-    int kl = 0, ku = 0;
-    DevBuf AB, ipiv, perm, work;
-};
-
 struct NcclUniqueIdBytes { char internal[128]; };  // ncclUniqueId (nccl.h), passed by value to ncclCommInitRank
 void nccl_release(struct diffopt_b200_ctx* ctx);
 
@@ -146,7 +138,6 @@ struct diffopt_b200_ctx {
     ConicState conic;
     LsqrWork lsqr;
     CsrDev lsqr_mat;
-    SparseBandState sparse;
     void* nccl_comm = nullptr;    // ncclComm_t of diffopt_b200_nccl_init (one rank per ctx)
     int nccl_ranks = 0, nccl_rank = 0;
     DevBuf qp_unpacked[2];        // Q / dQ expanded from packed lower triangles (qp_batch_solve_ex)
@@ -155,7 +146,7 @@ struct diffopt_b200_ctx {
     ConicBatchImpl* conic_batch = nullptr;
     int csr_cluster_ctas = 0;     // CTAs the cluster-kernel row blocks of csr_from_csc_host are cut for (0: default 16)
     SparseMfImpl* sparse_mf = nullptr;
-    int sparse_method = 0;        // factorisation currently held: 0 none, 1 banded LU (RCM), 2 multifrontal LU
+    int sparse_method = 0;        // factorisation currently held: 0 none, 2 multifrontal LU
     int64_t sparse_N = 0;
 };
 

@@ -27,10 +27,6 @@
 
 #include "common.cuh"
 
-int32_t sparse_band_setup(diffopt_b200_ctx* ctx, int64_t N, const int64_t* colptr, const int64_t* rowval, const double* nzval,
-                          int32_t trans, int64_t* bandwidth_out);
-int32_t sparse_band_solve(diffopt_b200_ctx* ctx, int64_t nrhs, const double* rhs, double* x_out, int32_t memspace);
-
 namespace {
 
 constexpr int MF_TC = 64;            // right-hand sides per solve CTA (one thread each)
@@ -373,24 +369,16 @@ __global__ void __launch_bounds__(MF_TC) mf_backward_kernel(const int* list, con
 // Row interchanges enter as the NET permutation of the front (psrc / pdst, mf_netperm_kernel).
 constexpr int MF_TT = 256;
 constexpr int MF_RG = MF_TT / MF_TC;   // row groups
-#ifndef MF_NB_W
-#define MF_NB_W 8                      // columns per block step of the tiled sweeps (16 measured slower: registers)
-#endif
-constexpr int MF_NB = MF_NB_W;
+constexpr int MF_NB = 8;               // columns per block step of the tiled sweeps (16 measured slower: registers)
 constexpr int MF_LDT = MF_TC + 1;      // leading dimension of YW: conflict-free by row and by column
-#ifndef MF_BT_MINB
-#define MF_BT_MINB 4                   // resident CTAs per SM the backward tiled kernel is compiled for (64 registers, 24 bytes of spills)
-#endif
+constexpr int MF_BT_MIN_BLOCKS = 4;    // resident CTAs per SM the backward tiled kernel is compiled for (64 registers, 24 bytes of spills)
 constexpr int MF_US_CAP = 8192;        // update lists up to this many entries are staged in shared memory
-#ifndef MF_HINTS
-#define MF_HINTS 0                     // bit 0: evict-first loads of B, bit 1: evict-first stores of X
-#endif
 __device__ __forceinline__ void cp_async8(double* smem_dst, const double* gsrc) {   // one double, global -> shared, no register staging
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ double ld_b(const double* p) { return (MF_HINTS & 1) ? __ldcs(p) : __ldg(p); }
-__device__ __forceinline__ void st_x(double* p, const double v) { if (MF_HINTS & 2) __stcs(p, v); else *p = v; }
+__device__ __forceinline__ double ld_b(const double* p) { return __ldg(p); }
+__device__ __forceinline__ void st_x(double* p, const double v) { *p = v; }
 
 // one CTA per front: net effect of the front's row interchanges.  psrc[first + r] = row (0..k-1, before the interchanges)
 // that ends at position r; pdst = inverse.
@@ -573,7 +561,7 @@ __global__ void __launch_bounds__(MF_TT) mf_forward_tiled_kernel(const int* list
     }
 }
 
-__global__ void __launch_bounds__(MF_TT, MF_BT_MINB) mf_backward_tiled_kernel(const int* list, const MfFront* fronts, const int* strct, const int* perm,
+__global__ void __launch_bounds__(MF_TT, MF_BT_MIN_BLOCKS) mf_backward_tiled_kernel(const int* list, const MfFront* fronts, const int* strct, const int* perm,
                                                                   const double* Lp, const double* Up, double* Y, double* X,
                                                                   const long long N, const int nrhs) {
     extern __shared__ __align__(16) double mf_smem[];
@@ -1327,7 +1315,7 @@ bool mf_symbolic(const Graph& g, const std::vector<std::vector<int32_t>>& snodes
             L.count = (int)(j - i);
             // within a size class the fronts run in the order of their rows in the caller's numbering: neighbouring fronts
             // share the sectors at the ends of their row runs (gathers of b, scatters of x), which then meet in L2
-            if (!big && !getenv("DIFFOPT_B200_MF_NO_LOCALITY_SORT"))
+            if (!big)
                 std::sort(H.lists.begin() + L.offset, H.lists.begin() + L.offset + L.count, [&](int32_t a, int32_t b) {
                     const int32_t ra = H.perm[(size_t)H.fronts[(size_t)a].first], rb = H.perm[(size_t)H.fronts[(size_t)b].first];
                     return ra != rb ? ra < rb : a < b;
@@ -1568,10 +1556,8 @@ int32_t mf_numeric(diffopt_b200_ctx* ctx, SparseMfImpl& M, int64_t nnz, std::vec
                     M.status.as<int>());
                 return cudaSuccess;
             };
-            const char* ft = getenv("DIFFOPT_B200_MF_FACT_THREADS");
-            const int want = ft ? atoi(ft) : (smem > 100 * 1024 ? 1024 : smem > 50 * 1024 ? 512 : MF_FACT_THREADS);
-            if (want >= 1024) DO_CUDA(ctx, launch(mf_factor_kernel<1024>, 1024));
-            else if (want >= 512) DO_CUDA(ctx, launch(mf_factor_kernel<512>, 512));
+            if (smem > 100 * 1024) DO_CUDA(ctx, launch(mf_factor_kernel<1024>, 1024));
+            else if (smem > 50 * 1024) DO_CUDA(ctx, launch(mf_factor_kernel<512>, 512));
             else DO_CUDA(ctx, launch(mf_factor_kernel<MF_FACT_THREADS>, MF_FACT_THREADS));
         } else {
             mf_factor_big_kernel<<<(unsigned)L.count, MF_BIG_THREADS, 0, ctx->stream>>>(
@@ -1620,17 +1606,10 @@ int32_t mf_numeric(diffopt_b200_ctx* ctx, SparseMfImpl& M, int64_t nnz, std::vec
 extern "C" int32_t diffopt_b200_sparse_setup(diffopt_b200_ctx* ctx, int64_t N, const int64_t* colptr, const int64_t* rowval,
                                              const double* nzval, int32_t trans, int64_t* bandwidth_out) {
     if (!ctx) return -1;
-    ctx->sparse.valid = false;
     ctx->sparse_method = 0;
     if (N <= 0 || !colptr || !rowval || !nzval) BAD_ARG(ctx, "sparse_setup: bad argument");
     if (colptr[0] != 1) BAD_ARG(ctx, "sparse_setup: colptr must be 1-based (Julia SparseMatrixCSC)");
     if (N >= (int64_t)1 << 31) BAD_ARG(ctx, "sparse_setup: N too large");
-    const char* force = getenv("DIFFOPT_B200_SPARSE");
-    if (force && strcmp(force, "band") == 0) {
-        int32_t rc = sparse_band_setup(ctx, N, colptr, rowval, nzval, trans, bandwidth_out);
-        if (rc == 0) ctx->sparse_method = 1;
-        return rc;
-    }
     if (bandwidth_out) *bandwidth_out = -1;
     DeviceGuard guard_(ctx->device);
     const auto t0 = std::chrono::steady_clock::now();
@@ -1681,8 +1660,9 @@ extern "C" int32_t diffopt_b200_sparse_setup(diffopt_b200_ctx* ctx, int64_t N, c
             fprintf(stderr, "sparse_setup: pass %d, %zu of %zu fronts need a delayed pivot (first: front %d, k %d, s %d, level-0 leaf %d)\n",
                     M.retries, failed.size(), M.H.fronts.size(), failed[0], f0.k, f0.s, f0.leaf);
         }
-        // delayed pivots: merge every failing front into its parent (its columns become fully summed there) and repeat
-        if (++M.retries > 8) break;
+        // delayed pivots: merge every failing front into its parent (its columns become fully summed there) and repeat.
+        // This ends: a root has no boundary rows, so it never reports a delayed pivot, and every pass removes a front.
+        ++M.retries;
         std::vector<char> drop(M.snodes.size(), 0);
         bool progress = false;
         for (int32_t f : failed) {
@@ -1700,11 +1680,9 @@ extern "C" int32_t diffopt_b200_sparse_setup(diffopt_b200_ctx* ctx, int64_t N, c
             if (!drop[s]) kept.push_back(std::move(M.snodes[s]));
         M.snodes.swap(kept);
     }
-    if (rc == -5) {  // pivoting inside the fronts was not enough: banded LU with full partial pivoting if the pattern allows
-        int32_t rb = sparse_band_setup(ctx, N, colptr, rowval, nzval, trans, bandwidth_out);
-        if (rb == 0) ctx->sparse_method = 1;
-        else if (rb == -3) ctx->err = "sparse_setup: no acceptable pivots inside the fronts after merging, and the pattern is not banded";
-        return rb;
+    if (rc == -5) {   // only if every failing front were a root, which cannot report a delayed pivot
+        ctx->err = "sparse_setup: a delayed pivot could not be merged into a parent front";
+        return -3;
     }
     if (rc != 0) return rc;
     ctx->sparse_method = 2;
@@ -1714,7 +1692,6 @@ extern "C" int32_t diffopt_b200_sparse_setup(diffopt_b200_ctx* ctx, int64_t N, c
 
 extern "C" int32_t diffopt_b200_sparse_solve(diffopt_b200_ctx* ctx, int64_t nrhs, const double* rhs, double* x_out, int32_t memspace) {
     if (!ctx) return -1;
-    if (ctx->sparse_method == 1) return sparse_band_solve(ctx, nrhs, rhs, x_out, memspace);
     if (ctx->sparse_method != 2 || !ctx->sparse_mf) BAD_ARG(ctx, "sparse_solve: no factorisation (call diffopt_b200_sparse_setup first)");
     if (nrhs <= 0 || !rhs || !x_out) BAD_ARG(ctx, "sparse_solve: bad argument");
     if (nrhs > 65535 * MF_TC) BAD_ARG(ctx, "sparse_solve: too many right-hand sides in one call");
@@ -1732,9 +1709,8 @@ extern "C" int32_t diffopt_b200_sparse_solve(diffopt_b200_ctx* ctx, int64_t nrhs
     const unsigned tiles = (unsigned)((nrhs + MF_TC - 1) / MF_TC);
     DO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     const unsigned ltiles = (unsigned)((nrhs + MF_LEAF_TC - 1) / MF_LEAF_TC);
-    const bool use_leaf = getenv("DIFFOPT_B200_MF_NO_LEAF_KERNELS") == nullptr;
     auto leaf_group = [&](const MfLaunch& L) {
-        return use_leaf && L.level == 0 && !L.big && L.max_k <= MF_KMAX && sizeof(double) * (size_t)(MF_KMAX + L.max_nf) * MF_LLD <= MF_SMEM_CAP;
+        return L.level == 0 && !L.big && L.max_k <= MF_KMAX && sizeof(double) * (size_t)(MF_KMAX + L.max_nf) * MF_LLD <= MF_SMEM_CAP;
     };
     auto smem_fwd = [](const MfLaunch& L) {
         return ((size_t)L.max_nf * L.max_k + (size_t)MF_TC * (L.max_k | 1) + (size_t)MF_TC * (L.max_s | 1)) * sizeof(double);
@@ -1743,12 +1719,11 @@ extern "C" int32_t diffopt_b200_sparse_solve(diffopt_b200_ctx* ctx, int64_t nrhs
         return ((size_t)L.max_k * L.max_k + (size_t)L.max_k * L.max_s + (size_t)MF_TC * (L.max_k | 1) + (size_t)MF_TC * (L.max_s | 1)) *
                sizeof(double);
     };
-    const bool use_tiled = M.netperm && getenv("DIFFOPT_B200_MF_OLD_SOLVE") == nullptr;
     auto tiled_smem = [](const MfLaunch& L, bool fwd) {
         return sizeof(double) * ((size_t)L.max_nf * MF_LDT + 1 + (size_t)(fwd ? L.max_nf : L.max_k) * MF_NB) + (fwd ? sizeof(int) * (2 * (size_t)L.max_k + (size_t)L.max_nf + 1 + (size_t)std::min(L.max_u, MF_US_CAP)) : 0);
     };
     auto tiled_group = [&](const MfLaunch& L) {
-        return use_tiled && L.max_nf <= MF_TT && tiled_smem(L, true) <= MF_SMEM_CAP && tiled_smem(L, false) <= MF_SMEM_CAP;
+        return M.netperm && L.max_nf <= MF_TT && tiled_smem(L, true) <= MF_SMEM_CAP && tiled_smem(L, false) <= MF_SMEM_CAP;
     };
     for (const MfLaunch& L : H.launches) {
         if (L.count == 0) continue;

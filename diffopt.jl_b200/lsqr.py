@@ -71,7 +71,7 @@ def sparse_analyze(M, trans=False):
 
 class SparseFactorization:
     """``diffopt_b200_sparse_setup`` / ``_sparse_solve``: one factorisation of a large sparse KKT matrix (or of its
-    adjoint) on the device (multifrontal LU; banded LU as fallback), reused for any number of right-hand sides -- the
+    adjoint) on the device (multifrontal LU), reused for any number of right-hand sides -- the
     direct ``LHS \\ RHS`` of QuadraticProgram.jl:490 for systems beyond the dense kernels (BASELINE config 3)."""
 
     def __init__(self, ctx: Context, M, trans=False):
@@ -79,16 +79,14 @@ class SparseFactorization:
         self.ctx = ctx
         self.N = M.shape[0]
         colptr, rowval, nzval = julia_csc(M)
-        bw = np.zeros(1, dtype=np.int64)
-        rc = ctx.lib.diffopt_b200_sparse_setup(ctx.h, self.N, ptr(colptr), ptr(rowval), ptr(nzval), int(trans), ptr(bw))
+        rc = ctx.lib.diffopt_b200_sparse_setup(ctx.h, self.N, ptr(colptr), ptr(rowval), ptr(nzval), int(trans), None)
         ctx.check(rc)
         if rc > 0:
             raise SingularException(rc)
-        self.bandwidth = int(bw[0])          # -1: multifrontal path (no band involved)
         self.factor_ms = ctx.last_kernel_ms
         st = np.zeros(8)
         ctx.check(ctx.lib.diffopt_b200_sparse_stats(ctx.h, ptr(st)))
-        self.stats = dict(method={0: "none", 1: "band", 2: "multifrontal"}[int(st[0])], fronts=int(st[1]), levels=int(st[2]),
+        self.stats = dict(method={0: "none", 2: "multifrontal"}[int(st[0])], fronts=int(st[1]), levels=int(st[2]),
                           max_front=int(st[3]), nnz_lu=int(st[4]), factor_flops=float(st[5]), analysis_ms=float(st[6]),
                           delayed_pivot_retries=int(st[7]))
 

@@ -240,17 +240,17 @@ int32_t diffopt_b200_kkt_solve_csc(
  * reference's refactorisation per direction (:438).  Method: multifrontal LU for general patterns -- nested-dissection
  * ordering and symbolic factorisation on the host, fronts factorised level by level on the device with partial
  * pivoting inside each front (a front that needs a delayed pivot is merged into its parent and the factorisation
- * repeated).  If that still finds no acceptable pivots, a banded LU with full partial pivoting (reverse Cuthill-McKee
- * ordering) is used when the pattern is banded (DIFFOPT_B200_SPARSE=band forces it).
+ * repeated until no front delays a pivot).
  * sparse_solve then solves for nrhs columns (rhs / x_out are N x nrhs column-major, host or device per memspace).
- * Returns 0; > 0: the matrix is singular (SingularException in the reference); -3: no acceptable pivot order found.
- * bandwidth_out (may be NULL) receives the half bandwidth when the banded path was used, -1 otherwise. */
+ * Returns 0; > 0: the matrix is singular (SingularException in the reference); -3: the factorisation cannot be held
+ * (a front or the factor structure is too large).
+ * bandwidth_out (may be NULL) receives -1. */
 int32_t diffopt_b200_sparse_setup(
     diffopt_b200_ctx* ctx, int64_t N, const int64_t* colptr, const int64_t* rowval, const double* nzval,
     int32_t trans, int64_t* bandwidth_out);
 int32_t diffopt_b200_sparse_solve(
     diffopt_b200_ctx* ctx, int64_t nrhs, const double* rhs, double* x_out, int32_t memspace);
-/* out8 = {method (0 none, 1 banded, 2 multifrontal), fronts, tree levels, largest front order, nnz(L+U) stored,
+/* out8 = {method (0 none, 2 multifrontal), fronts, tree levels, largest front order, nnz(L+U) stored,
  * factorisation flop, host analysis ms, delayed-pivot repetitions} of the factorisation held by the ctx. */
 int32_t diffopt_b200_sparse_stats(diffopt_b200_ctx* ctx, double* out8);
 /* Host-only analysis (ordering + symbolic factorisation, no GPU involved): out8 as above with out8[7] = number of

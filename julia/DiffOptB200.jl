@@ -89,23 +89,21 @@ end
     SparseFactorization(ctx, LHS)            # LHS::SparseMatrixCSC or its Adjoint
 
 One device factorisation of a large sparse KKT matrix (multifrontal LU: nested dissection + partial pivoting inside the
-fronts; banded LU as fallback), reused for any number of right-hand sides: `F \\ RHS` with `RHS::Matrix` (N x nrhs).  Replaces the per-direction `LHS' \\ RHS` of
+fronts), reused for any number of right-hand sides: `F \\ RHS` with `RHS::Matrix` (N x nrhs).  Replaces the per-direction `LHS' \\ RHS` of
 `forward_differentiate!` (QuadraticProgram.jl:438) when many directions are differentiated against one solution.
 """
 struct SparseFactorization
     ctx::Context
     n::Int
-    bandwidth::Int
     function SparseFactorization(ctx::Context, LHS)
         A, trans = _csc(LHS)
-        bw = Ref{Int64}(0)
         GC.@preserve A begin
             rc = ccall((:diffopt_b200_sparse_setup, LIB), Int32,
                        (Ptr{Cvoid}, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Int32, Ptr{Int64}),
-                       ctx.handle, size(A, 1), A.colptr, A.rowval, A.nzval, trans, bw)
+                       ctx.handle, size(A, 1), A.colptr, A.rowval, A.nzval, trans, C_NULL)
         end
         check(ctx, rc)
-        return new(ctx, size(A, 1), Int(bw[]))
+        return new(ctx, size(A, 1))
     end
 end
 

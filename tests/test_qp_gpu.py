@@ -372,92 +372,6 @@ def test_direct_solve_system_kkt_and_singular(ctx, kat):
         lsq.solve_csc(ctx, S, np.ones(3))
 
 
-def _banded_random(N, bw, seed):
-    import scipy.sparse as sp
-    rng = np.random.default_rng(seed)
-    diags = {k: rng.standard_normal(N - abs(k)) * (rng.random(N - abs(k)) < 0.6) for k in range(-bw, bw + 1)}
-    M = sp.diags([diags[k] for k in diags], list(diags), format="csc")
-    # weak diagonal (partial pivoting must do real work) and a random symmetric permutation (RCM must find the band again)
-    M = M + sp.diags(rng.uniform(0.01, 0.1, N) * rng.choice([-1, 1], N))
-    P = rng.permutation(N)
-    return sp.csc_matrix(M[P][:, P])
-
-
-@pytest.mark.parametrize("N,bw,nrhs", [(1, 0, 1), (50, 3, 2), (400, 17, 9), (333, 30, 3), (1000, 31, 5), (3000, 40, 33)])
-def test_sparse_band_factorization(ctx, N, bw, nrhs, monkeypatch):
-    """Banded fallback of the sparse direct path (LU after RCM): LHS and LHS', many right-hand sides, against a
-    dense/sparse CPU solve."""
-    import scipy.sparse.linalg as spla
-    monkeypatch.setenv("DIFFOPT_B200_SPARSE", "band")
-    lsq = diffopt_b200.submodule("lsqr")
-    M = _banded_random(N, bw, seed=N)
-    R = np.random.default_rng(1).standard_normal((N, nrhs))
-    for trans in (False, True):
-        F = lsq.SparseFactorization(ctx, M, trans=trans)
-        assert F.bandwidth <= 255
-        X = F.solve(R)
-        ref = spla.splu(M.T.tocsc() if trans else M).solve(R)
-        assert (np.linalg.norm(X - ref, axis=0) / np.linalg.norm(ref, axis=0)).max() <= RTOL_DIRECT
-    assert np.allclose(F.solve(R[:, 0]), ref[:, 0], rtol=1e-7, atol=1e-10)
-
-
-def test_sparse_mpc_kkt_forward_directions(ctx):
-    """BASELINE config 3 at reduced horizon (T = 300, N = 7200): the reference's LHS of an MPC QP, forward mode uses
-    LHS' (QuadraticProgram.jl:438); 16 directions against one factorisation vs SuperLU (stand-in for UMFPACK)."""
-    import scipy.sparse.linalg as spla
-    lsq = diffopt_b200.submodule("lsqr")
-    d = bench_data.mpc_config3(T=300)
-    K = d["K"]
-    N = K.shape[0]
-    R = np.random.default_rng(2).standard_normal((N, 16))
-    F = lsq.SparseFactorization(ctx, K, trans=True)
-    X = F.solve(R)
-    ref = spla.splu(K.T.tocsc()).solve(R)
-    assert (np.linalg.norm(X - ref, axis=0) / np.linalg.norm(ref, axis=0)).max() <= RTOL_DIRECT
-    res = np.linalg.norm(K.T @ X - R, axis=0) / np.linalg.norm(R, axis=0)
-    assert res.max() < 1e-9
-
-
-def test_sparse_band_kernel_variants_agree(ctx, monkeypatch):
-    """Narrow bands run the one-barrier LU and the register-window sweeps; the general kernels (any band up to 255)
-    must give the same factorisation and solutions (same pivots: identical up to the reciprocal-vs-division rounding)."""
-    import scipy.sparse.linalg as spla
-    lsq = diffopt_b200.submodule("lsqr")
-    monkeypatch.setenv("DIFFOPT_B200_SPARSE", "band")
-    d = bench_data.mpc_config3(T=150)
-    K = d["K"]
-    R = np.random.default_rng(4).standard_normal((K.shape[0], 7))
-    ref = spla.splu(K.tocsc()).solve(R)
-    sols = {}
-    for name, env in (("new", {}), ("old_lu", {"DIFFOPT_B200_BAND_LU_OLD": "1"}),
-                      ("old_solve", {"DIFFOPT_B200_BAND_SOLVE_OLD": "1"})):
-        for k in ("DIFFOPT_B200_BAND_LU_OLD", "DIFFOPT_B200_BAND_SOLVE_OLD"):
-            monkeypatch.delenv(k, raising=False)
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        F = lsq.SparseFactorization(ctx, K)
-        assert F.bandwidth <= 31
-        sols[name] = F.solve(R)
-        assert (np.linalg.norm(sols[name] - ref, axis=0) / np.linalg.norm(ref, axis=0)).max() <= RTOL_DIRECT
-    for other in ("old_lu", "old_solve"):
-        assert np.linalg.norm(sols["new"] - sols[other]) <= 1e-12 * np.linalg.norm(sols["new"])
-
-
-def test_sparse_setup_rejects_and_reports(ctx, monkeypatch):
-    import scipy.sparse as sp
-    lsq = diffopt_b200.submodule("lsqr")
-    monkeypatch.setenv("DIFFOPT_B200_SPARSE", "band")
-    # exactly singular (two identical rows) -> SingularException like the reference's `\\`
-    S = sp.csc_matrix(np.array([[1.0, 2.0, 0.0], [1.0, 2.0, 0.0], [0.0, 1.0, 1.0]]))
-    with pytest.raises(diffopt_b200.SingularException):
-        lsq.SparseFactorization(ctx, S)
-    # arrow matrix: no narrow band exists -> clean error, not a wrong answer
-    N = 2000
-    Aw = sp.lil_matrix((N, N)); Aw.setdiag(2.0); Aw[0, :] = 1.0; Aw[:, 0] = 1.0
-    with pytest.raises(diffopt_b200.DiffOptB200Error):
-        lsq.SparseFactorization(ctx, sp.csc_matrix(Aw))
-
-
 def test_extended_entry_shared_matrices_and_packed_triangles(ctx):
     """diffopt_b200_qp_batch_solve_ex: (a) Q, G, A (and the direction dQ, dG, dA) given once for the whole batch
     (OptNet layer with shared weights, SURVEY 8d) and (b) Q / dQ as packed lower triangles give exactly the results of
