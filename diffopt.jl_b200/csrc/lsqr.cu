@@ -91,77 +91,6 @@ __device__ double total_of(Dev& d, int slot) {
     return warp_sum_all(s);
 }
 
-// dot product of sparse row `row` with x, computed by a group of T lanes (T = 1,2,4,...,32; groups are
-// aligned inside the warp).  All 32 lanes must call this together.
-template <bool kScaleNone = true>
-__device__ __forceinline__ double row_dot(const CsrView& A, int row, bool valid, const double* __restrict__ x,
-                                          int lane_in_group, int T) {
-    double acc = 0.0;
-    if (valid) {
-        int s = A.rowptr[row], e = A.rowptr[row + 1];
-        for (int k = s + lane_in_group; k < e; k += T) acc += A.val[k] * __ldcg(x + A.colind[k]);
-    }
-    for (int o = T >> 1; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    return acc;
-}
-
-__device__ __forceinline__ int pick_T(const CsrView& A) {
-    int nnz = A.rowptr[A.nrows];
-    int avg = A.nrows > 0 ? nnz / A.nrows : 1;
-    int T = 1;
-    while (T < 32 && T * 2 <= avg) T <<= 1;
-    return T;
-}
-
-
-// y_row = (sparse row) . x for every row of A, `epi(row, value)` called once per row (by the first lane of the row's
-// lane group).  Each group of T lanes keeps RU rows in flight at once (RU independent rowptr -> (val, colind) -> x gather
-// chains per lane) so that a persistent grid of a few hundred CTAs still covers the HBM latency on large matrices;
-// consecutive groups take consecutive rows, so val / colind accesses of a warp stay contiguous.
-template <int RU, class F>
-__device__ __forceinline__ void spmv_rows(const Dev& d, const CsrView& A, const double* __restrict__ x, F&& epi) {
-    const int T = pick_T(A);
-    const int lig = d.lane & (T - 1), ngroups = d.gthreads / T, g = d.gtid / T;
-    for (int base = 0; base < A.nrows; base += ngroups * RU) {
-        int s[RU], len[RU];
-        int maxlen = 0;
-#pragma unroll
-        for (int r = 0; r < RU; ++r) {
-            const int row = base + r * ngroups + g;
-            s[r] = 0;
-            len[r] = 0;
-            if (row < A.nrows) {
-                s[r] = A.rowptr[row];
-                len[r] = A.rowptr[row + 1] - s[r];
-            }
-            maxlen = max(maxlen, len[r]);
-        }
-        maxlen = __reduce_max_sync(0xffffffffu, maxlen);  // keep the warp converged for the shuffles below
-        double acc[RU];
-#pragma unroll
-        for (int r = 0; r < RU; ++r) acc[r] = 0.0;
-        for (int k = lig; k < maxlen; k += T) {
-            double av[RU];
-            int ci[RU];
-#pragma unroll
-            for (int r = 0; r < RU; ++r) {
-                const bool ok = k < len[r];
-                av[r] = ok ? A.val[s[r] + k] : 0.0;
-                ci[r] = ok ? A.colind[s[r] + k] : 0;
-            }
-#pragma unroll
-            for (int r = 0; r < RU; ++r) acc[r] = fma(av[r], __ldcg(x + ci[r]), acc[r]);
-        }
-#pragma unroll
-        for (int r = 0; r < RU; ++r) {
-            double t = acc[r];
-            for (int o = T >> 1; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-            const int row = base + r * ngroups + g;
-            if (row < A.nrows && lig == 0) epi(row, t);
-        }
-    }
-}
-
 constexpr int SP_THREADS = 128;                   // threads of a streaming-SpMV CTA (8 CTAs per SM)
 constexpr int ST_NPT = 8;                         // nonzeros per thread in flight
 constexpr int ST_CHUNK = SP_THREADS * ST_NPT;     // nonzeros per row block
@@ -173,14 +102,18 @@ constexpr int CL_THREADS = CL_THREADS_DEF;
 constexpr int CL_NPT = 8;
 constexpr int CL_CHUNK = CL_THREADS * CL_NPT;
 constexpr int CL_MAX_CTAS = 16;
+// the 256-thread persistent kernel (problems with PSD cones) and conic_M_kernel run on the row blocks of the streaming
+// driver (CsrDev::blk / t_blk): <= ST_CHUNK nonzeros and <= SP_THREADS rows per block, or one longer row
+constexpr int LSQR_NPT = 4;
+static_assert(LSQR_THREADS * LSQR_NPT == ST_CHUNK && LSQR_THREADS >= SP_THREADS, "shape does not fit the blk lists");
 constexpr int ST_STRIDE = 2048;  // capacity of one partial slot = upper bound of every streaming grid
 
-// Row-block ("CSR-stream") SpMV for matrices beyond L2.  The host cuts the rows into blocks of <= ST_CHUNK
-// nonzeros (and <= SP_THREADS rows, or one longer row) and stores (first row, first nonzero) per block.  A CTA owns a
-// CONTIGUOUS range of blocks, so the part of x it gathers from slides slowly and stays in L1 when the matrix has any
-// locality (the kernels keep shared memory small to leave L1 its capacity).  Per block: NPT independent, fully
-// coalesced (val, colind) loads per thread -- no dependence on row pointers, so the HBM pipe stays full regardless of
-// the row lengths -- then the x gathers (read-only path) with the row's epilogue operands loaded underneath them
+// Row-block ("CSR-stream") SpMV, the sparse product of every LSQR driver.  The host cuts the rows into blocks of
+// <= THREADS * NPT nonzeros (and <= THREADS rows, or one longer row) and stores (first row, first nonzero) per block.
+// A CTA owns a CONTIGUOUS range of blocks, so the part of x it gathers from slides slowly and stays in L1 when the
+// matrix has any locality (the kernels keep shared memory small to leave L1 its capacity).  Per block: NPT independent,
+// fully coalesced (val, colind) loads per thread -- no dependence on row pointers, so the HBM pipe stays full regardless
+// of the row lengths -- then the x gathers (read-only path) with the row's epilogue operands loaded underneath them
 // (`pre(b, row)`), products parked in shared memory, one row per thread reduced in storage order (deterministic),
 // `epi(b, row, value, operands)` once per row.
 // sel(b, A, x, lb): matrix, gather vector and local block index of global block b.
@@ -446,8 +379,8 @@ __device__ void psd_apply_all(Dev& d, const ConicOpView& op, const double* __res
 }
 
 // Dpi (or Dpi') applied to y -> out, for all cones; ends WITHOUT a grid sync when there is no PSD cone
-// PSD = false compiles the PSD-cone phases out (the cluster / row-block variants and the streaming driver never run
-// problems with PSD cones; their kernels stay small).
+// PSD = false compiles the PSD-cone phases out (the cluster, gstream and batch kernels and the streaming driver never
+// run problems with PSD cones; their kernels stay small).
 template <bool PSD>
 __device__ void dpi_apply(Dev& d, const ConicOpView& op, const double* __restrict__ y, double* out, bool transpose) {
     for (int i = d.gtid; i < op.m; i += d.gthreads) {
@@ -479,34 +412,25 @@ __device__ void dpi_apply(Dev& d, const ConicOpView& op, const double* __restric
 // CONIC: OP = M or M'.
 // All functions are called by the whole grid and contain grid syncs.
 
-extern __shared__ double cl_prod[];  // CL_CHUNK products (dynamic shared memory of the cluster launch)
+extern __shared__ double cl_prod[];  // THREADS * NPT products (dynamic shared memory of the persistent launches)
 
-// CL = cluster-synchronised launch: the SpMVs run as row-block streams (every load of a thread's share is issued up
-// front: two L2 latencies per product instead of two per lane-group step), see spmv_stream.
-template <bool CL>
+// THREADS / NPT: row-block shape of the launch (the block list the host hands over is cut for it), see spmv_stream.
+template <int THREADS, int NPT>
 __device__ void csr_apply(Dev& d, const CsrView& A, const double* __restrict__ src, double s_src, double* dst,
                           double s_dst, int slot) {
     double acc = 0.0;
-    if constexpr (CL) {
-        spmv_stream<CL_THREADS, CL_NPT, 1>(
-            d.rank(), d.nblk, A.nblk, cl_prod, d.red, [&](int b, const CsrView*& M, const double*& x, int& lb) { M = &A; x = src; lb = b; },
-            [&](int, int row) { return make_double4(s_dst != 0.0 ? __ldcg(dst + row) : 0.0, 0.0, 0.0, 0.0); },
-            [&](int, int row, double t, const double4& o) {
-                t = t * s_src + s_dst * o.x;
-                dst[row] = t;
-                acc += t * t;
-            });
-    } else {
-        spmv_rows<4>(d, A, src, [&](int row, double t) {
-            t = t * s_src + s_dst * dst[row];
+    spmv_stream<THREADS, NPT, 1>(
+        d.rank(), d.nblk, A.nblk, cl_prod, d.red, [&](int b, const CsrView*& M, const double*& x, int& lb) { M = &A; x = src; lb = b; },
+        [&](int, int row) { return make_double4(s_dst != 0.0 ? __ldcg(dst + row) : 0.0, 0.0, 0.0, 0.0); },
+        [&](int, int row, double t, const double4& o) {
+            t = t * s_src + s_dst * o.x;
             dst[row] = t;
             acc += t * t;
         });
-    }
     block_partial(d, slot, acc);
 }
 
-// ---- Row-block phases of the conic operator, shared by conic_apply<CL = true> and the streaming kernels.  The CTAs
+// ---- Row-block phases of the conic operator, shared by conic_apply and the streaming kernels.  The CTAs
 // that share the row blocks number `ncta`, this one is `cta`; prod / red: shared scratch of spmv_stream.  xw / xs: the
 // vectors the products gather from (wc and src or src + n, or their copies staged in shared memory for XM = 2).
 // Partial sums accumulate into acc (||dst||^2) and dot.  dst is read with ld.global.cg where other CTAs of the same
@@ -591,120 +515,54 @@ __device__ __forceinline__ void conic_Mt_rows(const ConicOpView& op, int cta, in
 // identically): nobody reads those entries from memory, so thread 0 may store the new one right after the barrier
 // that publishes the partial sums, and ||dst||^2 (returned in `norm2`) is complete without another barrier.
 // SM (batched launches, one problem per CTA): the vectors the products gather from are first copied into shared memory
-// (behind the CL_CHUNK products: n + m doubles), see spmv_stream XM = 2.
-template <bool CL, bool PSD, bool SM = false>
-__device__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const double* __restrict__ src,
+// (behind the THREADS * NPT products: n + m doubles), see spmv_stream XM = 2.
+template <int THREADS, int NPT, bool PSD, bool SM = false>
+__device__ __forceinline__ void conic_apply(Dev& d, const ConicOpView& op, bool transpose, const double* __restrict__ src,
                             double s_src, double* dst, double s_dst, int slot, double src_last, double& dst_last,
                             double& norm2) {
     const int n = op.n, m = op.m, N = n + m + 1;
-    double dotacc = 0.0;
-    if constexpr (CL) {
-        double* xs_m = cl_prod + CL_CHUNK;  // staged gather vectors (SM): m entries, then n entries
-        double* xs_n = xs_m + m;
-        constexpr int XM = SM ? 2 : 1;
-        // (one problem per CTA: every producer of these vectors ran on this SM, so the L1-allocating cp.async sees them;
-        // the copies are in flight together, each thread waits for its own and the caller's barrier publishes them)
-        auto stage = [&](double* to, const double* from, int len) {
-            for (int i = d.tid; i < len; i += CL_THREADS)
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(to + i)), "l"(from + i)
-                             : "memory");
-            asm volatile("cp.async.commit_group;\n\tcp.async.wait_all;" ::: "memory");
-        };
-        double acc = 0.0;
-        if (!transpose) {
-            dpi_apply<PSD>(d, op, src + n, op.wc, false);  // wc = Dpi t2
-            d.sync();
-            if constexpr (SM) {
-                stage(xs_m, op.wc, m);
-                stage(xs_n, src, n);
-                __syncthreads();
-            }
-            conic_M_rows<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : op.wc, SM ? xs_n : src,
-                                                 src_last, s_src, dst, s_dst, acc, dotacc);
-            block_partial(d, slot, acc);
-            block_partial(d, slot + 1, dotacc);
-            d.sync();
-            const double last = -total_of(d, slot + 1) * s_src + s_dst * dst_last;  // -(c't1 + b'wc)
-            dst_last = last;
-            if (d.gtid == 0) dst[N - 1] = last;
-            norm2 = total_of(d, slot) + last * last;
-        } else {
-            const double u3 = src_last;
-            if constexpr (SM) {
-                stage(xs_n, src, n);
-                __syncthreads();
-            }
-            conic_Mt_A<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_n : src, u3, dotacc);
-            d.sync();
-            dpi_apply<PSD>(d, op, op.wc, op.wc + m, true);
-            if constexpr (SM) stage(xs_m, src + n, m);   // (src is not touched by dpi_apply: no barrier needed before)
-            d.sync();
-            conic_Mt_rows<CL_THREADS, CL_NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : src + n, u3, s_src,
-                                                  dst, s_dst, acc, dotacc);
-            block_partial(d, slot, acc);
-            block_partial(d, slot + 1, dotacc);
-            d.sync();
-            const double last = total_of(d, slot + 1) * s_src + s_dst * dst_last;
-            dst_last = last;
-            if (d.gtid == 0) dst[N - 1] = last;
-            norm2 = total_of(d, slot) + last * last;
-        }
-        return;
-    }
+    double* xs_m = cl_prod + THREADS * NPT;  // staged gather vectors (SM): m entries, then n entries
+    double* xs_n = xs_m + m;
+    constexpr int XM = SM ? 2 : 1;
+    // (one problem per CTA: every producer of these vectors ran on this SM, so the L1-allocating cp.async sees them;
+    // the copies are in flight together, each thread waits for its own and the caller's barrier publishes them)
+    auto stage = [&](double* to, const double* from, int len) {
+        for (int i = d.tid; i < len; i += THREADS)
+            asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(to + i)), "l"(from + i)
+                         : "memory");
+        asm volatile("cp.async.commit_group;\n\tcp.async.wait_all;" ::: "memory");
+    };
+    double acc = 0.0, dotacc = 0.0;
     if (!transpose) {
-        // wc = Dpi t2
-        dpi_apply<PSD>(d, op, src + n, op.wc, false);
+        dpi_apply<PSD>(d, op, src + n, op.wc, false);  // wc = Dpi t2
         d.sync();
-        const double t3 = src_last;
-        double acc = 0.0;
-        // rows 0..n-1:  (A' wc)_j + c_j t3
-        spmv_rows<4>(d, op.At, op.wc, [&](int row, double t) {
-            t = (t + op.c[row] * t3) * s_src + s_dst * dst[row];
-            dst[row] = t;
-            acc += t * t;
-            dotacc += op.c[row] * __ldcg(src + row);
-        });
-        // rows n..n+m-1:  -(A t1)_i + t2_i - wc_i + b_i t3
-        spmv_rows<4>(d, op.A, src, [&](int row, double t) {
-            const double wci = __ldcg(op.wc + row);
-            t = (-t + __ldcg(src + n + row) - wci + op.b[row] * t3) * s_src + s_dst * dst[n + row];
-            dst[n + row] = t;
-            acc += t * t;
-            dotacc += op.b[row] * wci;
-        });
+        if constexpr (SM) {
+            stage(xs_m, op.wc, m);
+            stage(xs_n, src, n);
+            __syncthreads();
+        }
+        conic_M_rows<THREADS, NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : op.wc, SM ? xs_n : src, src_last,
+                                       s_src, dst, s_dst, acc, dotacc);
         block_partial(d, slot, acc);
         block_partial(d, slot + 1, dotacc);
         d.sync();
-        // last row: -(c't1 + b'wc)
-        const double last = -total_of(d, slot + 1) * s_src + s_dst * dst_last;
+        const double last = -total_of(d, slot + 1) * s_src + s_dst * dst_last;  // -(c't1 + b'wc)
         dst_last = last;
         if (d.gtid == 0) dst[N - 1] = last;
         norm2 = total_of(d, slot) + last * last;
     } else {
-        // r = A u1 - u2 - b u3  -> wc
         const double u3 = src_last;
-        spmv_rows<4>(d, op.A, src, [&](int row, double t) {
-            const double u2 = __ldcg(src + n + row);
-            op.wc[row] = t - u2 - op.b[row] * u3;
-            dotacc += op.b[row] * u2;
-        });
-        d.sync();
-        double* r2 = op.wc + m;  // second half of the 2m scratch
-        dpi_apply<PSD>(d, op, op.wc, r2, true);
-        d.sync();
-        double acc = 0.0;
-        // rows 0..n-1: -(A' u2)_j - c_j u3
-        spmv_rows<4>(d, op.At, src + n, [&](int row, double t) {
-            t = (-t - op.c[row] * u3) * s_src + s_dst * dst[row];
-            dst[row] = t;
-            acc += t * t;
-            dotacc += op.c[row] * __ldcg(src + row);
-        });
-        for (int i = d.gtid; i < m; i += d.gthreads) {
-            double t = (__ldcg(r2 + i) + __ldcg(src + n + i)) * s_src + s_dst * dst[n + i];
-            dst[n + i] = t;
-            acc += t * t;
+        if constexpr (SM) {
+            stage(xs_n, src, n);
+            __syncthreads();
         }
+        conic_Mt_A<THREADS, NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_n : src, u3, dotacc);
+        d.sync();
+        dpi_apply<PSD>(d, op, op.wc, op.wc + m, true);
+        if constexpr (SM) stage(xs_m, src + n, m);   // (src is not touched by dpi_apply: no barrier needed before)
+        d.sync();
+        conic_Mt_rows<THREADS, NPT, XM>(op, d.rank(), d.nblk, cl_prod, d.red, src, SM ? xs_m : src + n, u3, s_src, dst, s_dst,
+                                        acc, dotacc);
         block_partial(d, slot, acc);
         block_partial(d, slot + 1, dotacc);
         d.sync();
@@ -724,17 +582,18 @@ struct OpArgs {
 };
 
 // Returns ||dst||^2 (after the update).  The conic operator ends behind its own barrier; the CSR one needs a barrier
-// here before its partial sums can be read.
-template <bool CL, bool PSD, bool SM = false>
-__device__ double op_apply(Dev& d, const OpArgs& o, bool adjoint, const double* src, double s_src, double* dst,
+// here before its partial sums can be read.  Inlined with conic_apply: called out of line, they make the kernel copy
+// its OpArgs parameter to a stack frame (600 B in the PSD build).
+template <int THREADS, int NPT, bool PSD, bool SM = false>
+__device__ __forceinline__ double op_apply(Dev& d, const OpArgs& o, bool adjoint, const double* src, double s_src, double* dst,
                            double s_dst, int slot, double src_last, double& dst_last) {
     if (o.kind == 0) {
-        csr_apply<CL>(d, adjoint ? o.adj : o.fwd, src, s_src, dst, s_dst, slot);
+        csr_apply<THREADS, NPT>(d, adjoint ? o.adj : o.fwd, src, s_src, dst, s_dst, slot);
         d.sync();
         return total_of(d, slot);
     }
     double norm2 = 0.0;
-    conic_apply<CL, PSD, SM>(d, o.conic, adjoint != (o.conic_trans != 0), src, s_src, dst, s_dst, slot, src_last, dst_last, norm2);
+    conic_apply<THREADS, NPT, PSD, SM>(d, o.conic, adjoint != (o.conic_trans != 0), src, s_src, dst, s_dst, slot, src_last, dst_last, norm2);
     return norm2;
 }
 
@@ -896,7 +755,7 @@ __device__ __forceinline__ void lsqr_update(Dev& d, const LsqrScalars& s, bool f
 // The whole LSQR iteration (Paige-Saunders) for one operator; called by every thread of the CTAs that share the problem
 // (the whole grid, one cluster, or -- batched launches -- one cluster / CTA per problem).  zero_below: right-hand sides of
 // norm <= zero_below give x = 0 without iterating (ConicProgram.jl:369 tests 1e-4 on the reverse seed; -1 disables).
-template <bool STREAM, bool PSD, bool SM>
+template <int THREADS, int NPT, bool PSD, bool SM>
 __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rhs, const LsqrParams prm, const LsqrVectors vec,
                           const double zero_below) {
     const int nr = o.nrows, nc = o.ncols;
@@ -908,7 +767,7 @@ __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rh
     d.sync();
     LsqrScalars s;
     const bool op1 = s.start(total_of(d, 0), zero_below);
-    s.first_alpha(op1 ? op_apply<STREAM, PSD, SM>(d, o, true, u, s.su, v, 0.0, 2, u_last, v_last) : 0.0);  // v_mem = A' u_true
+    s.first_alpha(op1 ? op_apply<THREADS, NPT, PSD, SM>(d, o, true, u, s.su, v, 0.0, 2, u_last, v_last) : 0.0);  // v_mem = A' u_true
     bool first = true;
     bool pending = false;  // an iteration whose x/w update and stop tests are still to be applied
 
@@ -919,7 +778,7 @@ __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rh
             lsqr_update(d, s, first, nc, vec, o.kind == 1 ? nc - 1 : -1, v_last);
             const bool more = s.itn < prm.maxiter;
             double unorm2 = 0.0;
-            if (more) unorm2 = op_apply<STREAM, PSD, SM>(d, o, false, v, s.sv, u, -s.alpha * s.su, 0, v_last, u_last);  // u_mem = A v_true - alpha u_true
+            if (more) unorm2 = op_apply<THREADS, NPT, PSD, SM>(d, o, false, v, s.sv, u, -s.alpha * s.su, 0, v_last, u_last);  // u_mem = A v_true - alpha u_true
             else d.sync();  // the partial sums of the update above
             if (pending) {
                 s.stop_tests(total_of(d, 4), prm);
@@ -928,7 +787,7 @@ __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rh
             first = false;
             if (s.istop > 0 || !more) break;
             if (s.next_beta(unorm2))
-                s.next_alpha(op_apply<STREAM, PSD, SM>(d, o, true, u, s.su, v, -s.beta * s.sv, 2, u_last, v_last));  // v_mem = A' u_true - beta v_true
+                s.next_alpha(op_apply<THREADS, NPT, PSD, SM>(d, o, true, u, s.su, v, -s.beta * s.sv, 2, u_last, v_last));  // v_mem = A' u_true - beta v_true
             s.rotate();
             pending = true;
         }
@@ -944,7 +803,7 @@ __device__ void lsqr_body(Dev& d, const OpArgs& o, const double* __restrict__ rh
     if (d.gtid == 0) s.write_stats(vec.stats);
 }
 
-template <int THREADS, int MINB, bool CLUSTER, bool STREAM, bool PSD>
+template <int THREADS, int NPT, int MINB, bool CLUSTER, bool PSD>
 __global__ void __launch_bounds__(THREADS, MINB) lsqr_kernel_t(OpArgs o, const double* __restrict__ rhs, LsqrParams prm,
                                                                LsqrVectors vec) {
     __shared__ double red[64];
@@ -952,7 +811,7 @@ __global__ void __launch_bounds__(THREADS, MINB) lsqr_kernel_t(OpArgs o, const d
     Dev d{cg::this_grid(), vec.partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
           (int)(blockDim.x >> 5), (int)gridDim.x, (int)(blockIdx.x * blockDim.x + threadIdx.x),
           (int)(gridDim.x * blockDim.x), CLUSTER};
-    lsqr_body<STREAM, PSD, false>(d, o, rhs, prm, vec, -1.0);
+    lsqr_body<THREADS, NPT, PSD, false>(d, o, rhs, prm, vec, -1.0);
 }
 
 // Lock-step batch: problem p = blockIdx.x / C is solved by the C CTAs of one cluster (C = 1: one CTA, the gather vectors
@@ -973,7 +832,7 @@ __global__ void __launch_bounds__(CL_THREADS, 1) lsqr_batch_kernel(const OpArgs*
     __syncthreads();
     Dev d{cg::this_grid(), sv.partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
           (int)(blockDim.x >> 5), C, (int)(cta * blockDim.x + threadIdx.x), (int)(C * blockDim.x), true, cta, C == 1};
-    lsqr_body<true, false, SM>(d, so, rhs[p], prm, sv, zero_below);
+    lsqr_body<CL_THREADS, CL_NPT, false, SM>(d, so, rhs[p], prm, sv, zero_below);
 }
 
 // stand-alone operator kernels (C-ABI conic_M_apply / conic_dpi_apply; also used by tests)
@@ -982,7 +841,7 @@ __global__ void __launch_bounds__(LSQR_THREADS) conic_M_kernel(ConicOpView op, i
     __shared__ double red[64];
     Dev d = make_dev(partials, red, (int)gridDim.x);
     double last = 0.0, norm2 = 0.0;
-    conic_apply<false, true>(d, op, transpose != 0, t, 1.0, out, 0.0, 0, __ldcg(t + op.n + op.m), last, norm2);
+    conic_apply<LSQR_THREADS, LSQR_NPT, true>(d, op, transpose != 0, t, 1.0, out, 0.0, 0, __ldcg(t + op.n + op.m), last, norm2);
 }
 
 __global__ void __launch_bounds__(LSQR_THREADS) conic_dpi_kernel(ConicOpView op, int transpose, const double* t, double* out,
@@ -1247,9 +1106,9 @@ ConicOpView conic_view(diffopt_b200_ctx* ctx, bool stream_blocks = false) {
     return o;
 }
 
-static int coop_grid(diffopt_b200_ctx* ctx, const void* kernel, int64_t work) {
+static int coop_grid(diffopt_b200_ctx* ctx, const void* kernel, size_t dyn, int64_t work) {
     int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, LSQR_THREADS, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, LSQR_THREADS, dyn);
     if (per_sm < 1) per_sm = 1;
     int64_t want = (work + LSQR_THREADS * 4 - 1) / (LSQR_THREADS * 4);
     // small problems: one CTA per SM keeps grid.sync cheap; large ones (beyond L2) need every resident CTA to cover HBM latency
@@ -1261,7 +1120,6 @@ static int coop_grid(diffopt_b200_ctx* ctx, const void* kernel, int64_t work) {
 
 // Cluster-synchronised variant for operators that a single cluster can chew through (a few 10^5 nonzeros, everything
 // L2 resident): ONE cluster of 16 (or 8) CTAs x 1024 threads, every phase boundary is a hardware cluster barrier.
-constexpr int64_t CL_MAX_WORK = (int64_t)1 << 20;
 constexpr int64_t CL_CLUSTER_WORK = (int64_t)512 << 10;
 
 // launch of `grid` CL_THREADS-thread CTAs in thread-block clusters of `cs`; `at` stores the cluster attribute
@@ -1309,38 +1167,34 @@ static int32_t lsqr_launch(diffopt_b200_ctx* ctx, OpArgs& o, int64_t work, const
     DO_CUDA(ctx, wk.u.reserve(d * (size_t)o.nrows));
     DO_CUDA(ctx, wk.v.reserve(d * (size_t)o.ncols));
     DO_CUDA(ctx, wk.w.reserve(d * (size_t)o.ncols));
-    const void* k_grid = (const void*)lsqr_kernel_t<LSQR_THREADS, 4, false, false, false>;
-    const void* k_cluster = (const void*)lsqr_kernel_t<CL_THREADS, 1, true, true, false>;
-    const void* k_gstream = (const void*)lsqr_kernel_t<CL_THREADS, 1, false, true, false>;
-    // Three persistent variants, by size of the operator (`work` ~ nonzeros + vector lengths):
-    //   cluster : <= CL_CLUSTER_WORK  one 16-CTA cluster, hardware barriers, row-block SpMV (16 SMs are enough)
-    //   gstream : <= CL_MAX_WORK      one CTA per SM, grid.sync(), row-block SpMV (L1 gather rate of 16 SMs is not)
-    //   grid    : larger / PSD cones  lane-group SpMV, up to 4 CTAs per SM
+    const void* k_cluster = (const void*)lsqr_kernel_t<CL_THREADS, CL_NPT, 1, true, false>;
+    const void* k_gstream = (const void*)lsqr_kernel_t<CL_THREADS, CL_NPT, 1, false, false>;
+    // problems with PSD cones: 256 threads (the GEMM phases of the PSD apply are written for them), 2 CTAs per SM
+    const void* k_grid = (const void*)lsqr_kernel_t<LSQR_THREADS, LSQR_NPT, 2, false, true>;
+    // Three persistent variants, all with the row-block SpMV (`work` ~ nonzeros + vector lengths):
+    //   cluster : <= CL_CLUSTER_WORK  one 16-CTA cluster, hardware barriers (16 SMs are enough)
+    //   gstream : larger              one CTA per SM, grid.sync() (L1 gather rate of 16 SMs is not enough)
+    //   grid    : PSD cones           256-thread CTAs, up to 2 per SM, grid.sync()
     const char* mode = getenv("DIFFOPT_B200_LSQR");
-    const bool psd = o.kind == 1 && o.conic.npsd > 0;  // PSD applies are GEMM phases written for the lane-group grid
-    int variant = 0;  // 0 grid, 1 cluster, 2 gstream
-    if (!psd && work <= CL_MAX_WORK) variant = work <= CL_CLUSTER_WORK ? 1 : 2;
-    if (mode && strcmp(mode, "grid") == 0) variant = 0;
+    const bool psd = o.kind == 1 && o.conic.npsd > 0;
+    int variant = psd || (mode && strcmp(mode, "grid") == 0) ? 0 : work <= CL_CLUSTER_WORK ? 1 : 2;  // 0 grid, 1 cluster, 2 gstream
     if (mode && strcmp(mode, "cluster") == 0 && !psd) variant = 1;
     if (mode && strcmp(mode, "gstream") == 0 && !psd) variant = 2;
     int cs = variant == 1 ? cluster_size_for(ctx, k_cluster) : 0;
     if (variant == 1 && cs == 0) variant = 2;
-    const size_t dyn = variant ? CL_CHUNK * sizeof(double) : 0;
-    // problems with PSD cones: same kernel compiled for 2 CTAs per SM (128 registers: the GEMM phases of the PSD apply
-    // spill badly under the 64-register cap of the 4-CTA build)
-    const void* k_psd = (const void*)lsqr_kernel_t<LSQR_THREADS, 2, false, false, true>;
-    const void* k_lane = psd ? k_psd : k_grid;
+    const size_t dyn = (variant ? CL_CHUNK : ST_CHUNK) * sizeof(double);
     int grid = cs;
-    if (variant == 0) grid = coop_grid(ctx, k_lane, work);
+    if (variant == 0) grid = coop_grid(ctx, k_grid, dyn, work);
     if (variant == 2) {
         DO_CUDA(ctx, cudaFuncSetAttribute(k_gstream, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
         grid = ctx->sm_count;
     }
-    {   // the row-block lists that match the launch
+    {   // the row-block lists cut for the launch's block shape
         auto pick = [&](CsrView& v, const CsrDev& M, bool t) {
-            const bool g = variant == 2;
-            v.blk = (t ? (g ? M.t_gblk : M.t_cblk) : (g ? M.gblk : M.cblk)).as<int>();
-            v.nblk = (int)(t ? (g ? M.t_ngblk : M.t_ncblk) : (g ? M.ngblk : M.ncblk));
+            const DevBuf* lists[3][2] = {{&M.blk, &M.t_blk}, {&M.cblk, &M.t_cblk}, {&M.gblk, &M.t_gblk}};
+            const int64_t counts[3][2] = {{M.nblk, M.t_nblk}, {M.ncblk, M.t_ncblk}, {M.ngblk, M.t_ngblk}};
+            v.blk = lists[variant][t]->as<int>();
+            v.nblk = (int)counts[variant][t];
         };
         if (o.kind == 1) {
             pick(o.conic.A, ctx->conic.A, false);
@@ -1365,7 +1219,7 @@ static int32_t lsqr_launch(diffopt_b200_ctx* ctx, OpArgs& o, int64_t work, const
     } else if (variant == 2) {
         DO_CUDA(ctx, cudaLaunchCooperativeKernel(k_gstream, dim3(grid), dim3(CL_THREADS), args, dyn, ctx->stream));
     } else {
-        DO_CUDA(ctx, cudaLaunchCooperativeKernel(k_lane, dim3(grid), dim3(LSQR_THREADS), args, 0, ctx->stream));
+        DO_CUDA(ctx, cudaLaunchCooperativeKernel(k_grid, dim3(grid), dim3(LSQR_THREADS), args, dyn, ctx->stream));
     }
     ctx->launches++;
     DO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
@@ -1481,26 +1335,27 @@ int32_t lsqr_run_conic(diffopt_b200_ctx* ctx, const double* rhs_dev, LsqrParams 
     return lsqr_launch(ctx, o, work, rhs_dev, prm, x_dev, stats_host7);
 }
 
-static int32_t conic_small_launch(diffopt_b200_ctx* ctx, const void* kernel, const double* t_dev, bool transpose,
+// dyn: dynamic shared memory of the kernel (conic_M_kernel: the products of its row blocks)
+static int32_t conic_small_launch(diffopt_b200_ctx* ctx, const void* kernel, size_t dyn, const double* t_dev, bool transpose,
                                   double* out_dev) {
     ConicState& s = ctx->conic;
-    ConicOpView op = conic_view(ctx);
+    ConicOpView op = conic_view(ctx, true);  // the streaming row blocks, cut for the LSQR_THREADS x LSQR_NPT shape
     int64_t work = s.A.nnz * 2 + s.n + 2 * s.m + s.psd_sumd2 * 8;
-    int grid = coop_grid(ctx, kernel, work);
+    int grid = coop_grid(ctx, kernel, dyn, work);
     DO_CUDA(ctx, ctx->lsqr.tmp.reserve(sizeof(double) * (size_t)LSQR_NSLOTS * (size_t)grid));
     double* partials = ctx->lsqr.tmp.as<double>();
     int tr = transpose ? 1 : 0;
     void* args[] = {&op, &tr, (void*)&t_dev, &out_dev, &partials};
-    DO_CUDA(ctx, cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(LSQR_THREADS), args, 0, ctx->stream));
+    DO_CUDA(ctx, cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(LSQR_THREADS), args, dyn, ctx->stream));
     ctx->launches++;
     return 0;
 }
 
 int32_t conic_apply_M(diffopt_b200_ctx* ctx, const double* t_dev, bool transpose, double* out_dev) {
-    return conic_small_launch(ctx, (const void*)conic_M_kernel, t_dev, transpose, out_dev);
+    return conic_small_launch(ctx, (const void*)conic_M_kernel, ST_CHUNK * sizeof(double), t_dev, transpose, out_dev);
 }
 int32_t conic_apply_dpi(diffopt_b200_ctx* ctx, const double* t_dev, bool transpose, double* out_dev) {
-    return conic_small_launch(ctx, (const void*)conic_dpi_kernel, t_dev, transpose, out_dev);
+    return conic_small_launch(ctx, (const void*)conic_dpi_kernel, 0, t_dev, transpose, out_dev);
 }
 
 // Lock-step batch of conic problems (diffopt_b200_conic_batch_reverse): one persistent kernel, problem p on the C CTAs of

@@ -50,31 +50,38 @@ def test_lsqr_csc_matches_oracle(ctx):
 
 @pytest.mark.parametrize("mode", ["cluster", "gstream", "grid"])
 def test_persistent_lsqr_variants_match_oracle(ctx, monkeypatch, mode):
-    """The three persistent LSQR drivers (single cluster with hardware barriers / one CTA per SM with row-block SpMV /
-    lane-group grid) on an explicit CSC matrix and on the conic operator: same iterates as the oracle at matched
-    iteration counts, same answer at convergence."""
+    """The three persistent LSQR drivers (single cluster with hardware barriers / one CTA per SM / the 256-thread build
+    of problems with PSD cones, all with the row-block SpMV) on explicit CSC matrices and on the conic operator: same
+    iterates as the oracle at matched iteration counts, same answer at convergence."""
     monkeypatch.setenv("DIFFOPT_B200_LSQR", mode)
     lsqr = diffopt_b200.submodule("lsqr")
     cm = diffopt_b200.submodule("conic")
     rng = np.random.default_rng(8)
     A = (sp.random(700, 450, density=0.03, random_state=3) + sp.eye(700, 450)).tocsc()
     A = sp.vstack([A, sp.csc_matrix((3, 450))]).tocsc()          # empty rows
-    A[5, :] = rng.normal(size=450)                                # one dense row (long-row path of the row-block SpMV)
+    A[5, :] = rng.normal(size=450)                                # one dense row
     A = A.tocsc()
     b = rng.normal(size=703)
-    for mi in (1, 3, 6):
-        xg, sg = lsqr.lsqr_csc(ctx, A, b, maxiter=mi)
-        xc, ic = olsqr.lsqr(A, b, maxiter=mi, return_info=True)
-        assert sg["itn"] == ic.itn == mi
-        # the dense row makes this matrix ill conditioned: rounding differences (summation order) grow quickly with
-        # the iteration count (1e-7 .. 3e-4 at 30 iterations depending on the build), so iterates are compared at
-        # small counts and the answer at convergence
-        assert rel(xg, xc) <= 1e-10, (mi, rel(xg, xc))
-    x, st = lsqr.lsqr_csc(ctx, A, b)
-    assert rel(x, olsqr.lsqr(A, b)) <= RTOL_LSQR
     bt = rng.normal(size=450)
-    xt, _ = lsqr.lsqr_csc(ctx, A, bt, trans=True, maxiter=4)
-    assert rel(xt, olsqr.lsqr(A.T.tocsc(), bt, maxiter=4)) <= 1e-10
+    # a row of 5000 nonzeros, longer than the row blocks of every driver (<= 4096): the one-row, whole-CTA branch of the
+    # row-block SpMV (scaled so that it does not dominate the spectrum: at full scale the iterates of this matrix move by
+    # 1e-9 under 1e-16 perturbations of A after 6 iterations, at 0.1 by 3e-14)
+    rng = np.random.default_rng(9)
+    L = (sp.random(400, 5000, density=0.03, random_state=4) + sp.eye(400, 5000)).tolil()
+    L[7, :] = 0.1 * rng.normal(size=5000)
+    for A, b, bt in ((A, b, bt), (L.tocsc(), rng.normal(size=400), rng.normal(size=5000))):
+        for mi in (1, 3, 6):
+            xg, sg = lsqr.lsqr_csc(ctx, A, b, maxiter=mi)
+            xc, ic = olsqr.lsqr(A, b, maxiter=mi, return_info=True)
+            assert sg["itn"] == ic.itn == mi
+            # the dense rows make these matrices ill conditioned: rounding differences (summation order) grow quickly
+            # with the iteration count (1e-7 .. 3e-4 at 30 iterations depending on the build), so iterates are compared
+            # at small counts and the answer at convergence
+            assert rel(xg, xc) <= 1e-10, (A.shape, mi, rel(xg, xc))
+        x, st = lsqr.lsqr_csc(ctx, A, b)
+        assert rel(x, olsqr.lsqr(A, b)) <= RTOL_LSQR
+        xt, _ = lsqr.lsqr_csc(ctx, A, bt, trans=True, maxiter=4)
+        assert rel(xt, olsqr.lsqr(A.T.tocsc(), bt, maxiter=4)) <= 1e-10
     d = bench_data.conic_config4(n=300, n_zero=30, n_nonneg=200, n_soc=20, soc_dim=6, nnz_per_row=5, seed=31)
     model = cm.ConicModel(ctx, d["A"], d["b"], d["c"], d["cone_types"], d["cone_dims"])
     model.set_variable_primal(d["x"]); model.set_constraint_primal(d["s"]); model.set_constraint_dual(d["y"])

@@ -87,8 +87,9 @@ def _exp_problem(**kw):
 
 @pytest.mark.parametrize("mode,psd_sides", [("cluster", ()), ("gstream", ()), ("grid", ()), ("stream", ()), ("grid", (6,))])
 def test_exp_forward_reverse_every_driver(ctx, monkeypatch, mode, psd_sides):
-    """Forward / reverse against the oracle at matched tight tolerances through each LSQR driver (the PSD variant runs
-    the PSD grid build); at fixed small iteration counts the iterates match the oracle's."""
+    """Forward / reverse against the oracle at matched tight tolerances through each LSQR driver (`grid` is the
+    256-thread build of problems with PSD cones, run here without and with one); at fixed small iteration counts the
+    iterates match the oracle's."""
     monkeypatch.setenv("DIFFOPT_B200_LSQR", mode)
     d = _exp_problem(psd_sides=psd_sides)
     model = _model(ctx, d)
