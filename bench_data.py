@@ -162,18 +162,22 @@ def conic_config4(n=5000, n_zero=500, n_nonneg=4000, n_soc=300, soc_dim=10, nnz_
 
 
 def conic_exp_problem(n=5000, n_zero=500, n_nonneg=4000, n_soc=0, soc_dim=10, n_exp=500, n_dual_exp=500, nnz_per_row=10,
-                      seed=7, psd_sides=(), solution_scale=1.0):
+                      seed=7, psd_sides=(), solution_scale=1.0, n_pow=0, n_dual_pow=0):
     """Config-4-like sparse conic program with ``n_exp`` ExponentialCone and ``n_dual_exp`` DualExponentialCone
-    constraints (3 rows each) after the zero, nonnegative and SOC rows (and PSD cones, if any), solved by construction
-    like ``conic_config4``: zeta ~ N(0,1)^m, s = Pi_K(zeta) onto the primal cone K (the listed sets), y = s - zeta in
-    K*, b = A x + s, c = -A'y.  The exponential cones are not self-dual: exp_cone_oracle.project(., t) projects onto the
-    DUAL of set t, so the primal projection of an EXP slice is project(., DUAL_EXP) and vice versa.  Every third exp
-    slice is drawn on the cone's curved boundary side (|zeta| mixed in scale) so that all four projection cases
-    occur."""
+    constraints (3 rows each) after the zero, nonnegative and SOC rows (and PSD cones, if any), then ``n_pow`` PowerCone
+    and ``n_dual_pow`` DualPowerCone constraints (3 rows each), solved by construction like ``conic_config4``:
+    zeta ~ N(0,1)^m, s = Pi_K(zeta) onto the primal cone K (the listed sets), y = s - zeta in K*, b = A x + s,
+    c = -A'y.  The exponential and power cones are not self-dual: pow_cone_oracle.project(., t) projects onto the DUAL
+    of set t, so the primal projection of an EXP slice is project(., DUAL_EXP) and vice versa (POW likewise).  Every
+    third exp / power slice is drawn with |zeta| mixed in scale so that all curved-cone cases occur.  The power cones'
+    exponents (uniform in [0.05, 0.95]), their order and scales come from a second generator seeded from ``seed``, so
+    the data without power cones is what it always was.  ``cone_params`` holds each cone's exponent (0 for the other
+    cones)."""
     import scipy.sparse as sp
 
-    import exp_cone_oracle as oc  # projection only used to *construct* the data set
+    import pow_cone_oracle as oc  # projection only used to *construct* the data set
     rng = np.random.default_rng(seed)
+    prng = np.random.default_rng([seed, 6])
     cone_types = [oc.ZERO] * (1 if n_zero else 0) + [oc.NONNEG] * (1 if n_nonneg else 0) + [oc.SOC] * n_soc + \
         [oc.PSD] * len(psd_sides)
     cone_dims = ([n_zero] if n_zero else []) + ([n_nonneg] if n_nonneg else []) + [soc_dim] * n_soc + \
@@ -182,6 +186,13 @@ def conic_exp_problem(n=5000, n_zero=500, n_nonneg=4000, n_soc=0, soc_dim=10, n_
     kinds = kinds[rng.permutation(kinds.size)]
     cone_types += kinds.tolist()
     cone_dims += [3] * kinds.size
+    cone_params = [0.0] * len(cone_types)
+    if n_pow or n_dual_pow:
+        pkinds = np.array([oc.POW] * n_pow + [oc.DUAL_POW] * n_dual_pow)
+        pkinds = pkinds[prng.permutation(pkinds.size)]
+        cone_types += pkinds.tolist()
+        cone_dims += [3] * pkinds.size
+        cone_params += prng.uniform(0.05, 0.95, pkinds.size).tolist()
     m = int(sum(cone_dims))
     rows = np.repeat(np.arange(m), nnz_per_row)
     cols = rng.integers(0, n, size=m * nnz_per_row)
@@ -193,16 +204,18 @@ def conic_exp_problem(n=5000, n_zero=500, n_nonneg=4000, n_soc=0, soc_dim=10, n_
     for k, t in enumerate(cone_types):
         if t in (oc.EXP, oc.DUAL_EXP) and k % 3 == 0:
             zeta[off[k]:off[k + 1]] *= 10.0 ** rng.uniform(-1, 1, 3)
+        elif t in (oc.POW, oc.DUAL_POW) and k % 3 == 0:
+            zeta[off[k]:off[k + 1]] *= 10.0 ** prng.uniform(-1, 1, 3)
     zeta *= solution_scale
-    dual_of = {oc.EXP: oc.DUAL_EXP, oc.DUAL_EXP: oc.EXP}
+    dual_of = {oc.EXP: oc.DUAL_EXP, oc.DUAL_EXP: oc.EXP, oc.POW: oc.DUAL_POW, oc.DUAL_POW: oc.POW}
     s = np.empty(m)
     for k, t in enumerate(cone_types):
         sl = slice(off[k], off[k + 1])
-        s[sl] = 0.0 if t == oc.ZERO else oc.project(zeta[sl], dual_of.get(t, t))
+        s[sl] = 0.0 if t == oc.ZERO else oc.project(zeta[sl], dual_of.get(t, t), cone_params[k])
     y = s - zeta
     x = rng.standard_normal(n) * solution_scale
     return dict(A=A, b=A @ x + s, c=-(A.T @ y), x=x, s=s, y=y, cone_types=cone_types, cone_dims=cone_dims,
-                seed=rng.standard_normal(n))
+                cone_params=cone_params, seed=rng.standard_normal(n))
 
 
 def conic_config4_conditioned(**kw):

@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("DIFFOPT_B200_LIB") or os.path.join(HERE, "lib", "libd
 
 HOST, DEVICE = 0, 1
 QP_SHARED_MATRICES, QP_SHARED_DIRECTION, QP_PACKED_Q, QP_ASYNC, QP_ALLREDUCE = 1, 2, 4, 8, 16
-CONE_ZERO, CONE_NONNEG, CONE_SOC, CONE_PSD, CONE_EXP, CONE_DUAL_EXP = 0, 1, 2, 3, 4, 5
+CONE_ZERO, CONE_NONNEG, CONE_SOC, CONE_PSD, CONE_EXP, CONE_DUAL_EXP, CONE_POW, CONE_DUAL_POW = 0, 1, 2, 3, 4, 5, 6, 7
 
 _lib = None
 
@@ -56,6 +56,7 @@ SIGNATURES = {
     "diffopt_b200_lsqr_csc": (C.c_int32, [vp, C.c_int64, C.c_int64, vp, vp, vp, C.c_int32, vp, C.c_double,
                                           C.c_double, C.c_double, C.c_int64, vp, vp, C.c_int32]),
     "diffopt_b200_conic_setup": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, C.c_int32]),
+    "diffopt_b200_conic_setup_ex": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, vp, C.c_int32]),
     "diffopt_b200_conic_get_vp": (C.c_int32, [vp, vp, C.c_int32]),
     "diffopt_b200_conic_dpi_apply": (C.c_int32, [vp, vp, C.c_int32, vp, C.c_int32]),
     "diffopt_b200_conic_M_apply": (C.c_int32, [vp, vp, C.c_int32, vp, C.c_int32]),
@@ -65,6 +66,7 @@ SIGNATURES = {
                                                C.c_int32]),
     "diffopt_b200_conic_batch_begin": (C.c_int32, [vp, C.c_int64, C.c_int32]),
     "diffopt_b200_conic_batch_add": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, C.c_int32]),
+    "diffopt_b200_conic_batch_add_ex": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, vp, C.c_int32]),
     "diffopt_b200_conic_batch_reverse": (C.c_int32, [vp, vp, C.c_double, C.c_double, C.c_double, C.c_int64, vp, vp, vp, vp,
                                                      C.c_int32]),
     "diffopt_b200_sparse_setup_inertia": (C.c_int32, [vp, C.c_int64, vp, vp, vp, C.c_int64, C.c_int64, C.c_double, C.c_int32, vp]),

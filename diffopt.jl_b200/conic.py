@@ -9,15 +9,18 @@ import time
 
 import numpy as np
 
-from ._capi import CONE_DUAL_EXP, CONE_EXP, CONE_NONNEG, CONE_PSD, CONE_SOC, CONE_ZERO, HOST, Context, ptr  # noqa: F401
+from ._capi import (CONE_DUAL_EXP, CONE_DUAL_POW, CONE_EXP, CONE_NONNEG, CONE_POW, CONE_PSD, CONE_SOC,  # noqa: F401
+                    CONE_ZERO, HOST, Context, ptr)
 from .lsqr import DEFAULTS, julia_csc
 
 
 class ConicModel:
     """Geometric conic form  A x + s = b, s in K  with the reference's conventions:
-    ``A = -coefficients`` (:179-183), ``b = constants``, ``c`` negated for MAX sense (:206-208)."""
+    ``A = -coefficients`` (:179-183), ``b = constants``, ``c`` negated for MAX sense (:206-208).
+    ``cone_params``: one number per cone, the exponent of each ``PowerCone`` / ``DualPowerCone`` (other entries are not
+    read); None when the list has no power cone."""
 
-    def __init__(self, ctx: Context, A, b, c, cone_types, cone_dims):
+    def __init__(self, ctx: Context, A, b, c, cone_types, cone_dims, cone_params=None):
         import scipy.sparse as sp
         self.ctx = ctx
         self.A = sp.csc_matrix(A, dtype=np.float64)
@@ -26,6 +29,9 @@ class ConicModel:
         self.c = np.ascontiguousarray(c, dtype=np.float64).reshape(self.n)
         self.cone_types = np.ascontiguousarray(cone_types, dtype=np.int32)
         self.cone_dims = np.ascontiguousarray(cone_dims, dtype=np.int64)
+        self.cone_params = None if cone_params is None else np.ascontiguousarray(cone_params, dtype=np.float64)
+        if self.cone_params is not None and self.cone_params.shape != self.cone_types.shape:
+            raise ValueError("cone_params needs one entry per cone")
         self.x = np.full(self.n, np.nan)
         self.s = np.full(self.m, np.nan)
         self.y = np.full(self.m, np.nan)
@@ -37,12 +43,12 @@ class ConicModel:
         self.last_stats = None
 
     @classmethod
-    def from_moi(cls, ctx, coefficients, constants, c, cone_types, cone_dims, max_sense=False):
+    def from_moi(cls, ctx, coefficients, constants, c, cone_types, cone_dims, max_sense=False, cone_params=None):
         """From MOI-style data (function = coefficients x + constants in K), applying the
         reference's sign handling."""
         import scipy.sparse as sp
         return cls(ctx, -sp.csc_matrix(coefficients, dtype=np.float64), constants,
-                   -np.asarray(c, float) if max_sense else c, cone_types, cone_dims)
+                   -np.asarray(c, float) if max_sense else c, cone_types, cone_dims, cone_params)
 
     # MOI.set(model, VariablePrimalStart / ConstraintPrimalStart / ConstraintDualStart, ...)
     def set_variable_primal(self, x):
@@ -65,10 +71,10 @@ class ConicModel:
         if np.isnan(self.s).any():
             raise ValueError("Some constraints are missing a value for the `ConstraintPrimalStart` attribute.")
         colptr, rowval, nzval = julia_csc(self.A)
-        rc = self.ctx.lib.diffopt_b200_conic_setup(
+        rc = self.ctx.lib.diffopt_b200_conic_setup_ex(
             self.ctx.h, self.n, self.m, ptr(colptr), ptr(rowval), ptr(nzval), ptr(self.b), ptr(self.c),
             ptr(self.x), ptr(self.s), ptr(self.y), len(self.cone_types), ptr(self.cone_types),
-            ptr(self.cone_dims), HOST)
+            ptr(self.cone_dims), ptr(self.cone_params), HOST)
         self.ctx.check(rc)
         self.setup_ms = self.ctx.last_kernel_ms
         self.gradient_cache = True
@@ -178,9 +184,9 @@ class ConicBatch:
         ctx.check(ctx.lib.diffopt_b200_conic_batch_begin(ctx.h, self.B, int(ctas_per_problem)))
         for mdl in self.models:
             colptr, rowval, nzval = julia_csc(mdl.A)
-            ctx.check(ctx.lib.diffopt_b200_conic_batch_add(
+            ctx.check(ctx.lib.diffopt_b200_conic_batch_add_ex(
                 ctx.h, mdl.n, mdl.m, ptr(colptr), ptr(rowval), ptr(nzval), ptr(mdl.b), ptr(mdl.c), ptr(mdl.x), ptr(mdl.s),
-                ptr(mdl.y), len(mdl.cone_types), ptr(mdl.cone_types), ptr(mdl.cone_dims), HOST))
+                ptr(mdl.y), len(mdl.cone_types), ptr(mdl.cone_types), ptr(mdl.cone_dims), ptr(mdl.cone_params), HOST))
 
     def reverse_differentiate(self, dx_seeds):
         """dx_seeds: (B, n).  Returns dict(g (B, n+m+1), dc (B, n), db (B, m), stats (B, 4))."""

@@ -46,7 +46,7 @@ void conic_state_release(ConicState& c) {
     for (DevBuf* b : {&c.b, &c.c, &c.x, &c.s, &c.y, &c.v, &c.vp, &c.row_kind, &c.nn_scale, &c.soc_off, &c.soc_dim,
                       &c.soc_case, &c.soc_nx, &c.psd_off, &c.psd_d, &c.psd_uoff, &c.psd_U, &c.psd_Bm, &c.psd_ident,
                       &c.psd_work, &c.psd_lam, &c.psd_loff, &c.psd_tri, &c.psd_toff, &c.w1, &c.w2, &c.w3, &c.exp_off,
-                      &c.exp_neg, &c.blk3})
+                      &c.exp_neg, &c.blk3, &c.pow_off, &c.pow_neg, &c.pow_alpha})
         b->release();
 }
 

@@ -75,6 +75,9 @@ struct ConicState {
     // pi onto K* = -(pi onto K°)(-v)); blk3: 3 coefficients per row of such a cone (row i: blk3[3 i .. 3 i + 2])
     DevBuf exp_off, exp_neg, blk3;
     int64_t nexp = 0;
+    // power cones (same blk3 rows): first row, v negated (DIFFOPT_CONE_POW: pi onto K*), exponent
+    DevBuf pow_off, pow_neg, pow_alpha;
+    int64_t npow = 0;
     // PSD cones
     DevBuf psd_off, psd_d, psd_uoff;  // per PSD cone: row offset, side d, offset into U/B storage
     DevBuf psd_U, psd_Bm, psd_ident;  // eigenvectors (col-major d x d), B matrix, identity flag

@@ -5,6 +5,7 @@
 #include <vector>
 
 #include "exp_cone.cuh"
+#include "pow_cone.cuh"
 #include "lsqr.cuh"
 
 ConicOpView conic_view(diffopt_b200_ctx* ctx, bool stream_blocks);
@@ -271,10 +272,16 @@ int32_t diffopt_b200_lsqr_csc(diffopt_b200_ctx* ctx, int64_t nrows, int64_t ncol
     return 0;
 }
 
-int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
-                                 const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
-                                 const double* x, const double* s, const double* y, int64_t ncones,
-                                 const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace) {
+}  // extern "C"
+
+namespace {
+
+// conic_setup and conic_setup_ex: cone_param (one exponent per cone, read for power cones) may be NULL when the list
+// has no power cone.
+int32_t conic_setup_impl(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr, const int64_t* A_rowval,
+                         const double* A_nzval, const double* b, const double* c, const double* x, const double* s,
+                         const double* y, int64_t ncones, const int32_t* cone_type, const int64_t* cone_dim,
+                         const double* cone_param, int32_t memspace) {
     if (!ctx) return -1;
     DeviceGuard guard_(ctx->device);
     ConicState& S = ctx->conic;
@@ -282,20 +289,24 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     if (n <= 0 || m < 0 || ncones < 0) BAD_ARG(ctx, "conic_setup: bad sizes");
     if (!A_colptr || !b || !c || !x || !s || !y || (ncones > 0 && (!cone_type || !cone_dim)))
         BAD_ARG(ctx, "conic_setup: null argument");
-    std::vector<char> t0, t1, t2, t3, t4;
-    const void *hc, *hr, *hv, *hct, *hcd;
+    std::vector<char> t0, t1, t2, t3, t4, t5;
+    const void *hc, *hr, *hv, *hct, *hcd, *hcp = nullptr;
     if (int32_t rc = to_host_copy(ctx, A_colptr, sizeof(int64_t) * (size_t)(n + 1), memspace, t0, &hc)) return rc;
     const int64_t nnz = ((const int64_t*)hc)[n] - 1;
     if (int32_t rc = to_host_copy(ctx, A_rowval, sizeof(int64_t) * (size_t)nnz, memspace, t1, &hr)) return rc;
     if (int32_t rc = to_host_copy(ctx, A_nzval, sizeof(double) * (size_t)nnz, memspace, t2, &hv)) return rc;
     if (int32_t rc = to_host_copy(ctx, cone_type, sizeof(int32_t) * (size_t)ncones, memspace, t3, &hct)) return rc;
     if (int32_t rc = to_host_copy(ctx, cone_dim, sizeof(int64_t) * (size_t)ncones, memspace, t4, &hcd)) return rc;
+    if (cone_param && ncones > 0)
+        if (int32_t rc = to_host_copy(ctx, cone_param, sizeof(double) * (size_t)ncones, memspace, t5, &hcp)) return rc;
     const int32_t* ct = (const int32_t*)hct;
     const int64_t* cd = (const int64_t*)hcd;
+    const double* cp = (const double*)hcp;
     // cone bookkeeping (host): row kinds and per-cone index lists
     std::vector<signed char> kind((size_t)m, 0), rowtype((size_t)m, 0);
-    std::vector<int> soc_off, soc_dim, psd_off, psd_d, exp_off;
-    std::vector<signed char> exp_neg;
+    std::vector<int> soc_off, soc_dim, psd_off, psd_d, exp_off, pow_off;
+    std::vector<signed char> exp_neg, pow_neg;
+    std::vector<double> pow_alpha;
     std::vector<long long> psd_uoff;
     int64_t row = 0, sumd2 = 0, maxd = 0;
     for (int64_t k = 0; k < ncones; ++k) {
@@ -330,6 +341,18 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
                 exp_off.push_back((int)row);
                 exp_neg.push_back(ct[k] == DIFFOPT_CONE_EXP ? 1 : 0);
                 break;
+            case DIFFOPT_CONE_POW:
+            case DIFFOPT_CONE_DUAL_POW: {
+                if (dim != 3) BAD_ARG(ctx, "conic_setup: power cone dimension must be 3");
+                if (!cp) BAD_ARG(ctx, "conic_setup: power cones need their exponents: call conic_setup_ex with cone_param");
+                const double a = cp[k];
+                if (!(std::isfinite(a) && a > 0.0 && a < 1.0))
+                    BAD_ARG(ctx, "conic_setup: power cone exponent must be finite and in (0, 1)");
+                for (int64_t i = 0; i < 3; ++i) kind[(size_t)(row + i)] = (signed char)(4 + i);
+                pow_off.push_back((int)row);
+                pow_neg.push_back(ct[k] == DIFFOPT_CONE_POW ? 1 : 0);
+                pow_alpha.push_back(a);
+            } break;
             default:
                 BAD_ARG(ctx, "conic_setup: unknown cone type");
         }
@@ -340,6 +363,7 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     S.nsoc = (int64_t)soc_off.size();
     S.npsd = (int64_t)psd_off.size();
     S.nexp = (int64_t)exp_off.size();
+    S.npow = (int64_t)pow_off.size();
     S.psd_sumd2 = sumd2;
     S.psd_maxd = maxd;
     if (int32_t rc = csr_from_csc_host(ctx, m, n, (const int64_t*)hc, (const int64_t*)hr, (const double*)hv, S.A))
@@ -365,7 +389,11 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     DO_CUDA(ctx, keep(S.psd_uoff, psd_uoff.data(), sizeof(long long) * psd_uoff.size(), cudaMemcpyHostToDevice));
     DO_CUDA(ctx, keep(S.exp_off, exp_off.data(), sizeof(int) * exp_off.size(), cudaMemcpyHostToDevice));
     DO_CUDA(ctx, keep(S.exp_neg, exp_neg.data(), exp_neg.size(), cudaMemcpyHostToDevice));
-    DO_CUDA(ctx, S.blk3.reserve(exp_off.empty() ? 8 : d8 * 3 * (size_t)m));
+    DO_CUDA(ctx, keep(S.pow_off, pow_off.data(), sizeof(int) * pow_off.size(), cudaMemcpyHostToDevice));
+    DO_CUDA(ctx, keep(S.pow_neg, pow_neg.data(), pow_neg.size(), cudaMemcpyHostToDevice));
+    DO_CUDA(ctx, keep(S.pow_alpha, pow_alpha.data(), d8 * pow_alpha.size(), cudaMemcpyHostToDevice));
+    // (blk3 holds 3 coefficients for every row when any cone has a 3 x 3 block: exponential or power)
+    DO_CUDA(ctx, S.blk3.reserve(exp_off.empty() && pow_off.empty() ? 8 : d8 * 3 * (size_t)m));
     {   // flattened list of 32 x 32 output tiles of the PSD apply
         std::vector<int> toff(psd_d.size() + 1, 0);
         for (size_t k = 0; k < psd_d.size(); ++k) {
@@ -411,6 +439,14 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
                                                           S.v.as<double>(), S.vp.as<double>(), S.blk3.as<double>(), nullptr);
         ctx->launches++;
     }
+    if (S.npow > 0) {
+        int blocks = (int)((S.npow + 127) / 128);
+        if (blocks > ctx->sm_count * 16) blocks = ctx->sm_count * 16;
+        cone_pow_kernel<<<blocks, 128, 0, ctx->stream>>>((int)S.npow, S.pow_off.as<int>(), S.pow_neg.as<signed char>(),
+                                                          S.pow_alpha.as<double>(), S.v.as<double>(), S.vp.as<double>(),
+                                                          S.blk3.as<double>(), nullptr);
+        ctx->launches++;
+    }
     if (S.npsd > 0)
         if (int32_t rc = psd_eig_launch(ctx, psd_d, psd_uoff, psd_off)) return rc;
     DO_CUDA(ctx, cudaGetLastError());
@@ -420,6 +456,27 @@ int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, co
     if (cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1) == cudaSuccess) ctx->last_ms = ms;
     S.valid = true;
     return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int32_t diffopt_b200_conic_setup(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
+                                 const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
+                                 const double* x, const double* s, const double* y, int64_t ncones,
+                                 const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace) {
+    return conic_setup_impl(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim, nullptr,
+                            memspace);
+}
+
+int32_t diffopt_b200_conic_setup_ex(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
+                                    const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
+                                    const double* x, const double* s, const double* y, int64_t ncones,
+                                    const int32_t* cone_type, const int64_t* cone_dim, const double* cone_param,
+                                    int32_t memspace) {
+    return conic_setup_impl(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim,
+                            cone_param, memspace);
 }
 
 int32_t diffopt_b200_conic_get_vp(diffopt_b200_ctx* ctx, double* vp_out, int32_t memspace) {
@@ -611,10 +668,15 @@ int32_t diffopt_b200_conic_batch_begin(diffopt_b200_ctx* ctx, int64_t B, int32_t
     return 0;
 }
 
-int32_t diffopt_b200_conic_batch_add(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
-                                     const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
-                                     const double* x, const double* s, const double* y, int64_t ncones,
-                                     const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace) {
+}  // extern "C"
+
+namespace {
+
+int32_t conic_batch_add_impl(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
+                             const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
+                             const double* x, const double* s, const double* y, int64_t ncones,
+                             const int32_t* cone_type, const int64_t* cone_dim, const double* cone_param,
+                             int32_t memspace) {
     if (!ctx) return -1;
     ConicBatchImpl* bt = ctx->conic_batch;
     if (!bt) BAD_ARG(ctx, "conic_batch_add: call conic_batch_begin first");
@@ -627,7 +689,8 @@ int32_t diffopt_b200_conic_batch_add(diffopt_b200_ctx* ctx, int64_t n, int64_t m
     ctx->conic = ConicState{};
     const int prev_ctas = ctx->csr_cluster_ctas;
     ctx->csr_cluster_ctas = bt->C;
-    int32_t rc = diffopt_b200_conic_setup(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim, memspace);
+    int32_t rc = conic_setup_impl(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim,
+                                  cone_param, memspace);
     ctx->csr_cluster_ctas = prev_ctas;
     ConicState fresh = ctx->conic;
     ctx->conic = parked;
@@ -643,6 +706,27 @@ int32_t diffopt_b200_conic_batch_add(diffopt_b200_ctx* ctx, int64_t n, int64_t m
     bt->m = m;
     bt->states.push_back(fresh);
     return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int32_t diffopt_b200_conic_batch_add(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
+                                     const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
+                                     const double* x, const double* s, const double* y, int64_t ncones,
+                                     const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace) {
+    return conic_batch_add_impl(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim,
+                                nullptr, memspace);
+}
+
+int32_t diffopt_b200_conic_batch_add_ex(diffopt_b200_ctx* ctx, int64_t n, int64_t m, const int64_t* A_colptr,
+                                        const int64_t* A_rowval, const double* A_nzval, const double* b, const double* c,
+                                        const double* x, const double* s, const double* y, int64_t ncones,
+                                        const int32_t* cone_type, const int64_t* cone_dim, const double* cone_param,
+                                        int32_t memspace) {
+    return conic_batch_add_impl(ctx, n, m, A_colptr, A_rowval, A_nzval, b, c, x, s, y, ncones, cone_type, cone_dim,
+                                cone_param, memspace);
 }
 
 int32_t diffopt_b200_conic_batch_reverse(diffopt_b200_ctx* ctx, const double* dx_seeds, double atol, double btol,

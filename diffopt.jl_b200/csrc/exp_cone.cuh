@@ -27,6 +27,16 @@
 #define __device__
 #endif
 
+// Leading 3 x 3 block of [[M, g], [g', 0]]^-1 from Mi = M^-1 (symmetric): D = Mi - Mi g g' Mi / (g' Mi g).  The
+// projection Jacobian of every cone with one curved boundary surface f = 0 (exponential, power).
+__host__ __device__ inline void sym3_bordered_block(const double* Mi, const double* g, double* D) {
+    double u[3];
+    for (int i = 0; i < 3; ++i) u[i] = Mi[3 * i] * g[0] + Mi[3 * i + 1] * g[1] + Mi[3 * i + 2] * g[2];
+    const double gu = g[0] * u[0] + g[1] * u[1] + g[2] * u[2];
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) D[3 * i + j] = Mi[3 * i + j] - u[i] * u[j] / gu;
+}
+
 // scaled h and h' at rho: both times e^-|rho|, so G / Gp is the Newton step of h
 __host__ __device__ inline void exp_cone_h(double rho, double r, double s, double t, double& G, double& Gp) {
     const double a = (rho - 1.0) * r + s, b = r - rho * s, q = rho * rho - rho + 1.0;
@@ -173,11 +183,7 @@ __host__ __device__ inline int exp_cone_project(double r, double s, double t, do
     }
     const double sc = rho > 0.0 ? exp(-rho) : 1.0, er = rho > 0.0 ? 1.0 : exp(rho);
     const double g[3] = {er, er * (1.0 - rho), -sc};
-    double u[3];
-    for (int i = 0; i < 3; ++i) u[i] = Mi[3 * i] * g[0] + Mi[3 * i + 1] * g[1] + Mi[3 * i + 2] * g[2];
-    const double gu = g[0] * u[0] + g[1] * u[1] + g[2] * u[2];
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) D[3 * i + j] = Mi[3 * i + j] - u[i] * u[j] / gu;
+    sym3_bordered_block(Mi, g, D);
     return evals;
 }
 

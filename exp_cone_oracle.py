@@ -202,13 +202,18 @@ def Dpi_dense(v, cone_types, cone_dims):
 def gradient_cache(A, b, c, x, s, y, cone_types, cone_dims):
     """``oracle.conic.gradient_cache`` with exponential cones among the cones; the result feeds ``oracle.conic.forward``,
     ``reverse`` and ``reverse_param_grads`` as is."""
+    v = np.asarray(y, float) - np.asarray(s, float)                 # ConicProgram.jl:222
+    return assemble_cache(A, b, c, x, s, y, Dpi_blocks(v, cone_types, cone_dims), pi(v, cone_types, cone_dims))
+
+
+def assemble_cache(A, b, c, x, s, y, blocks, vp):
+    """The gradient cache of ``oracle.conic`` from the dense Dpi blocks of every cone and vp = pi(y - s)."""
     A = sp.csc_matrix(A, dtype=np.float64)
     m, n = A.shape
     b = np.asarray(b, float)
     c = np.asarray(c, float)
     x, s, y = (np.asarray(t, float) for t in (x, s, y))
-    v = y - s                                                        # ConicProgram.jl:222
-    Dpi = sp.block_diag([sp.csc_matrix(B) for B in Dpi_blocks(v, cone_types, cone_dims)], format="csc")
+    Dpi = sp.block_diag([sp.csc_matrix(B) for B in blocks], format="csc")
     cc = sp.csc_matrix(c.reshape(n, 1))
     bb = sp.csc_matrix(b.reshape(m, 1))
     M = sp.bmat([                                                    # :243-247
@@ -216,4 +221,4 @@ def gradient_cache(A, b, c, x, s, y, cone_types, cone_dims):
         [-A, sp.identity(m, format="csc") - Dpi, bb],
         [-cc.T, -(bb.T @ Dpi), sp.csc_matrix((1, 1))],
     ], format="csc")
-    return ConicCache(M, pi(v, cone_types, cone_dims), Dpi, A, b, c, x, s, y)
+    return ConicCache(M, vp, Dpi, A, b, c, x, s, y)

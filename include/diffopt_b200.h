@@ -51,6 +51,15 @@ typedef struct diffopt_b200_ctx diffopt_b200_ctx;
  * v in -K* -> 0, 0; r <= 0 and s <= 0 -> (r, 0, max(t, 0)), diag(1, 0, [t > 0]);
  * else the curved boundary (root of Friberg's univariate h), symmetric 3 x 3 Jacobian. */
 #define DIFFOPT_CONE_DUAL_EXP 5
+/* MOI.PowerCone(a) K_a = {(x, y, z) : x >= 0, y >= 0, x^a y^(1-a) >= |z|}, dimension 3, 0 < a < 1 (the exponent of
+ * each power cone is passed in cone_param of conic_setup_ex); pi onto K_a* (Moreau: Pi_K*(v) = v + Pi_K(-v),
+ * DPi_K*(v) = I - DPi_K(-v)) */
+#define DIFFOPT_CONE_POW 6
+/* MOI.DualPowerCone(a) K_a* = {(u, v, w) : u >= 0, v >= 0, (u/a)^a (v/(1-a))^(1-a) >= |w|}, dimension 3; pi onto K_a.
+ * Pi_K(v), v = (x0, y0, z0), cases in this order (the order decides ties): v in K -> v, I; v in -K* -> 0, 0;
+ * z0 = 0 -> (max(x0, 0), max(y0, 0), 0), diag([x0 > 0], [y0 > 0], 0); else the curved boundary (root of Hien's
+ * univariate psi), symmetric 3 x 3 Jacobian. */
+#define DIFFOPT_CONE_DUAL_POW 7
 
 /* ---- lifetime ------------------------------------------------------------------- */
 int32_t diffopt_b200_version(void);
@@ -284,6 +293,14 @@ int32_t diffopt_b200_conic_setup(
     const int64_t* A_colptr, const int64_t* A_rowval, const double* A_nzval,
     const double* b, const double* c, const double* x, const double* s, const double* y,
     int64_t ncones, const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace);
+/* conic_setup with one parameter per cone: cone_param[i] (in memspace, like cone_type) is the exponent a of cone i,
+ * read only for DIFFOPT_CONE_POW / DIFFOPT_CONE_DUAL_POW, which need it (finite, 0 < a < 1; the end points are not
+ * supported).  cone_param may be NULL when the list has no power cone; conic_setup is conic_setup_ex with NULL. */
+int32_t diffopt_b200_conic_setup_ex(
+    diffopt_b200_ctx* ctx, int64_t n, int64_t m,
+    const int64_t* A_colptr, const int64_t* A_rowval, const double* A_nzval,
+    const double* b, const double* c, const double* x, const double* s, const double* y,
+    int64_t ncones, const int32_t* cone_type, const int64_t* cone_dim, const double* cone_param, int32_t memspace);
 /* vp = pi(y - s) of the current setup (length m) */
 int32_t diffopt_b200_conic_get_vp(diffopt_b200_ctx* ctx, double* vp_out, int32_t memspace);
 /* out = Dpi(v) * t or Dpi(v)' * t (length m): the `Dπ` operator on its own */
@@ -322,6 +339,12 @@ int32_t diffopt_b200_conic_batch_add(
     const int64_t* A_colptr, const int64_t* A_rowval, const double* A_nzval,
     const double* b, const double* c, const double* x, const double* s, const double* y,
     int64_t ncones, const int32_t* cone_type, const int64_t* cone_dim, int32_t memspace);
+/* conic_batch_add with the per-cone parameters of conic_setup_ex (cone_param may be NULL without power cones) */
+int32_t diffopt_b200_conic_batch_add_ex(
+    diffopt_b200_ctx* ctx, int64_t n, int64_t m,
+    const int64_t* A_colptr, const int64_t* A_rowval, const double* A_nzval,
+    const double* b, const double* c, const double* x, const double* s, const double* y,
+    int64_t ncones, const int32_t* cone_type, const int64_t* cone_dim, const double* cone_param, int32_t memspace);
 int32_t diffopt_b200_conic_batch_reverse(
     diffopt_b200_ctx* ctx, const double* dx_seeds,
     double atol, double btol, double conlim, int64_t maxiter,

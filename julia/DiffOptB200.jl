@@ -201,16 +201,18 @@ synchronize(ctx::Context) = check(ctx, ccall((:diffopt_b200_synchronize, LIB), I
 
 # ------------------------------------------------------------------------------------------------
 # (3) ConicProgram backend: _gradient_cache / forward / reverse (src/ConicProgram/ConicProgram.jl:172-394)
-#     cone_type: 0 Zeros, 1 Nonnegatives, 2 SecondOrderCone, 3 PositiveSemidefiniteConeTriangle (row order of A)
+#     cone_type: 0 Zeros, 1 Nonnegatives, 2 SecondOrderCone, 3 PositiveSemidefiniteConeTriangle, 4 ExponentialCone,
+#     5 DualExponentialCone, 6 PowerCone, 7 DualPowerCone (row order of A); cone_param: the exponent of each power cone
 # ------------------------------------------------------------------------------------------------
 function conic_setup(ctx::Context, A::SparseArrays.SparseMatrixCSC{Float64,Int}, b, c, x, s, y,
-                     cone_type::Vector{Int32}, cone_dim::Vector{Int64})
+                     cone_type::Vector{Int32}, cone_dim::Vector{Int64}, cone_param::Vector{Float64} = zeros(length(cone_type)))
     m, n = size(A)
-    GC.@preserve A b c x s y cone_type cone_dim begin
-        rc = ccall((:diffopt_b200_conic_setup, LIB), Int32,
+    GC.@preserve A b c x s y cone_type cone_dim cone_param begin
+        rc = ccall((:diffopt_b200_conic_setup_ex, LIB), Int32,
                    (Ptr{Cvoid}, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
-                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Int64}, Int32),
-                   ctx.handle, n, m, A.colptr, A.rowval, A.nzval, b, c, x, s, y, length(cone_type), cone_type, cone_dim, HOST)
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}, Int32),
+                   ctx.handle, n, m, A.colptr, A.rowval, A.nzval, b, c, x, s, y, length(cone_type), cone_type, cone_dim,
+                   cone_param, HOST)
     end
     check(ctx, rc)
 end
@@ -317,19 +319,26 @@ _cone_code(::Type{MOI.SecondOrderCone}) = Int32(2)
 _cone_code(::Type{MOI.PositiveSemidefiniteConeTriangle}) = Int32(3)
 _cone_code(::Type{MOI.ExponentialCone}) = Int32(4)
 _cone_code(::Type{MOI.DualExponentialCone}) = Int32(5)
+_cone_code(::Type{MOI.PowerCone{Float64}}) = Int32(6)
+_cone_code(::Type{MOI.DualPowerCone{Float64}}) = Int32(7)
 _cone_code(::Type{S}) where {S} = error("DiffOptB200.ConicModel: unsupported set $S")
 
-"cone list in row order (cone_type, cone_dim) from the ProductOfSets -- what `Dπ` / `π` iterate over (diff_opt.jl:491-519)"
+"the per-cone parameter passed through conic_setup_ex: the exponent of a power cone, 0 for every other set"
+_cone_param(set::Union{MOI.PowerCone{Float64},MOI.DualPowerCone{Float64}}) = set.exponent
+_cone_param(::MOI.AbstractVectorSet) = 0.0
+
+"cone list in row order (cone_type, cone_dim, cone_param) from the ProductOfSets -- what `Dπ` / `π` iterate over (diff_opt.jl:491-519)"
 function _cone_list(model::ConicModel)
-    entries = Tuple{Int,Int32,Int64}[]
+    entries = Tuple{Int,Int32,Int64,Float64}[]
     for (F, S) in MOI.get(model.model, MOI.ListOfConstraintTypesPresent())
         for ci in MOI.get(model.model, MOI.ListOfConstraintIndices{F,S}())
             r = MOI.Utilities.rows(model.model.constraints, ci)
-            push!(entries, (first(r), _cone_code(S), Int64(length(r))))
+            set = MOI.get(model.model, MOI.ConstraintSet(), ci)
+            push!(entries, (first(r), _cone_code(S), Int64(length(r)), _cone_param(set)))
         end
     end
     sort!(entries; by = first)
-    return Int32[e[2] for e in entries], Int64[e[3] for e in entries]
+    return Int32[e[2] for e in entries], Int64[e[3] for e in entries], Float64[e[4] for e in entries]
 end
 
 # _gradient_cache (ConicProgram.jl:172-255): A = -coefficients, b = constants, c (negated for MAX, zero for FEASIBILITY)
@@ -351,8 +360,8 @@ function _gradient_cache(model::ConicModel)
         cc = Vector{Float64}(DiffOpt.sparse_array_representation(obj, n).terms)
         MOI.get(model, MOI.ObjectiveSense()) == MOI.MAX_SENSE ? -cc : cc
     end
-    cone_type, cone_dim = _cone_list(model)
-    conic_setup(model.ctx, A, Vector{Float64}(b), c, model.x, model.s, model.y, cone_type, cone_dim)
+    cone_type, cone_dim, cone_param = _cone_list(model)
+    conic_setup(model.ctx, A, Vector{Float64}(b), c, model.x, model.s, model.y, cone_type, cone_dim, cone_param)
     model.vp = Vector{Float64}(undef, length(b))
     rc = ccall((:diffopt_b200_conic_get_vp, LIB), Int32, (Ptr{Cvoid}, Ptr{Float64}, Int32), model.ctx.handle, model.vp, HOST)
     check(model.ctx, rc)
@@ -526,7 +535,7 @@ end
     conic_batch_reverse(ctx, problems, dx; atol, btol, conlim, maxiter)
 
 `reverse_differentiate!` (ConicProgram.jl:336-394) of B conic problems of equal size in ONE persistent kernel.  `problems`:
-vector of named tuples `(A, b, c, x, s, y, cone_type, cone_dim)`; `dx[n, B]`.  Returns `(g[n+m+1, B], dc[n, B], db[m, B], stats[4, B])`.
+vector of named tuples `(A, b, c, x, s, y, cone_type, cone_dim)` (and `cone_param` with power cones); `dx[n, B]`.  Returns `(g[n+m+1, B], dc[n, B], db[m, B], stats[4, B])`.
 """
 function conic_batch_reverse(ctx::Context, problems::Vector, dx::Matrix{Float64};
                              atol = sqrt(eps()), btol = sqrt(eps()), conlim = 1 / sqrt(eps()), maxiter = 0)
@@ -536,11 +545,12 @@ function conic_batch_reverse(ctx::Context, problems::Vector, dx::Matrix{Float64}
     m, n = size(problems[1].A)
     for pr in problems
         A = pr.A::SparseArrays.SparseMatrixCSC{Float64,Int}
-        rc = ccall((:diffopt_b200_conic_batch_add, LIB), Int32,
+        cone_param = hasproperty(pr, :cone_param) ? Vector{Float64}(pr.cone_param) : zeros(length(pr.cone_type))
+        rc = ccall((:diffopt_b200_conic_batch_add_ex, LIB), Int32,
                    (Ptr{Cvoid}, Int64, Int64, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
-                    Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Int64}, Int32),
+                    Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Int32}, Ptr{Int64}, Ptr{Float64}, Int32),
                    ctx.handle, n, m, A.colptr, A.rowval, A.nzval, pr.b, pr.c, pr.x, pr.s, pr.y, length(pr.cone_type), pr.cone_type,
-                   pr.cone_dim, HOST)
+                   pr.cone_dim, cone_param, HOST)
         check(ctx, rc)
     end
     g = Matrix{Float64}(undef, n + m + 1, B); dc = Matrix{Float64}(undef, n, B); db = Matrix{Float64}(undef, m, B)
