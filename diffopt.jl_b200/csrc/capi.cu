@@ -67,6 +67,7 @@ int32_t diffopt_b200_destroy(diffopt_b200_ctx* ctx) {
         if (ev) cudaEventDestroy(ev);
     QpBatchState& q = ctx->qp;
     q.Q.release(); q.G.release(); q.A.release(); q.h.release(); q.z.release(); q.lam.release(); q.nu.release();
+    for (DevBuf* b : {&ctx->qpf.f, &ctx->qpf.fb, &ctx->qpf.gin, &ctx->qpf.gout}) b->release();
     conic_state_release(ctx->conic);
     LsqrWork& l = ctx->lsqr;
     for (DevBuf* b : {&l.u, &l.v, &l.w, &l.x, &l.tmp, &l.scal}) b->release();
@@ -111,7 +112,7 @@ int32_t qp_batch_launch(diffopt_b200_ctx* ctx, const QpSolveArgs& a) {
 }
 
 // Scan info[] (device) after the solve: returns first failing instance + 1, or 0.
-static int32_t finish_info(diffopt_b200_ctx* ctx, int64_t B, int* dinfo, int32_t* info_user, int memspace,
+int32_t finish_info(diffopt_b200_ctx* ctx, int64_t B, int* dinfo, int32_t* info_user, int memspace,
                            std::vector<int>& hinfo) {
     hinfo.resize((size_t)B);
     cudaError_t e = cudaMemcpyAsync(hinfo.data(), dinfo, sizeof(int) * (size_t)B, cudaMemcpyDeviceToHost, ctx->stream);
@@ -248,6 +249,7 @@ int32_t diffopt_b200_qp_batch_last_stats(diffopt_b200_ctx* ctx, int64_t* out3) {
     out3[0] = 0;
     out3[1] = ctx->qp_last_hint;
     out3[2] = ctx->qp_last_kernel;
+    if (ctx->qp_last_kernel == 3) out3[0] = ctx->qpf.nrej;
     if (ctx->qp_last_kernel == 2 && ctx->qp_fb.ptr) {
         int nfb = 0;
         DO_CUDA(ctx, cudaMemcpyAsync(&nfb, ctx->qp_fb.ptr, sizeof nfb, cudaMemcpyDeviceToHost, ctx->stream));
@@ -297,6 +299,7 @@ int32_t diffopt_b200_qp_batch_setup(diffopt_b200_ctx* ctx, int64_t B, int32_t n,
         BAD_ARG(ctx, "qp_batch_setup: Q, z (and G, h, lam when m > 0; A, nu when p > 0) are required");
     QpBatchState& s = ctx->qp;
     s.valid = false;
+    ctx->qpf.valid = false;
     s.B = B; s.n = n; s.m = m; s.p = p;
     const size_t d = sizeof(double);
     cudaMemcpyKind kind = memspace == DIFFOPT_B200_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
@@ -318,13 +321,17 @@ int32_t diffopt_b200_qp_batch_setup(diffopt_b200_ctx* ctx, int64_t B, int32_t n,
     return 0;
 }
 
-static void fill_from_state(const QpBatchState& s, QpSolveArgs& a) {
+}  // extern "C"
+
+void fill_from_state(const QpBatchState& s, QpSolveArgs& a) {
     a.B = s.B; a.n = s.n; a.m = s.m; a.p = s.p;
     a.Q = s.Q.as<double>();
     a.G = s.m ? s.G.as<double>() : nullptr;
     a.A = s.p ? s.A.as<double>() : nullptr;
     a.h = s.h.as<double>(); a.z = s.z.as<double>(); a.lam = s.lam.as<double>(); a.nu = s.nu.as<double>();
 }
+
+extern "C" {
 
 int32_t diffopt_b200_qp_batch_reverse(diffopt_b200_ctx* ctx, const double* dl_dz, double* rev_out, int32_t* info,
                                       int32_t memspace) {

@@ -46,6 +46,17 @@ struct QpBatchState {
                  *dlam_ = nullptr, *dnu_ = nullptr;  // device pointers actually used
 };
 
+// LDL' factors of the setup's instances kept by qp_batch_factorize (FactorLayout in qp_sqd_dev.cuh); a new setup drops them.
+struct QpFactorState {
+    bool valid = false;
+    int nt_cap = 0;      // tile order the factors were stored for (0: no instance fits, the pivoted LU serves the batch)
+    int64_t stride = 0;  // doubles per instance
+    int nrej = 0;        // instances served by the pivoted LU (listed in fb)
+    DevBuf f;            // [B][stride] factors
+    DevBuf fb;           // [count, list...] of those instances
+    DevBuf gin, gout;    // one direction of the listed instances in the [B][...] layout the pivoted-LU kernel reads and writes
+};
+
 struct CsrDev {  // device CSR (0-based, int32 indices) of a sparse matrix and of its transpose
     int64_t nrows = 0, ncols = 0, nnz = 0;
     DevBuf rowptr, colind, val;     // A   (nrows x ncols)
@@ -127,7 +138,8 @@ struct diffopt_b200_ctx {
     cudaEvent_t qp_hmax_ev[4] = {nullptr, nullptr, nullptr, nullptr};
     int64_t qp_hmax_call[4] = {-1, -1, -1, -1};  // host-side call counter of the copy in flight in each slot (-1: none)
     int64_t qp_calls = 0;
-    int qp_last_kernel = -1;      // kernel of the last qp_batch call: 0 generic pivoted LU, 1 tuned pivoted LU, 2 LDL' fast path
+    int qp_last_kernel = -1;      // kernel of the last qp_batch call: 0 generic pivoted LU, 1 tuned pivoted LU, 2 LDL' fast path,
+                                  // 3 stored LDL' (qp_batch_factorize)
     int qp_last_hint = -1;        // active-set size that launch was configured for
     int qp_seq = 0;               // call number, tags the active-set word written by the LDL' kernel
     int qp_hint = -1;             // active-set size the next launch of the LDL' fast path is configured for (-1: unknown)
@@ -138,6 +150,7 @@ struct diffopt_b200_ctx {
     unsigned async_calls = 0;     // calls enqueued since the last synchronize
     bool async_pending = false;
     QpBatchState qp;
+    QpFactorState qpf;
     ConicState conic;
     LsqrWork lsqr;
     CsrDev lsqr_mat;

@@ -142,8 +142,13 @@ __device__ __forceinline__ void prefetch_l2(const void* p, const size_t bytes) {
     for (size_t o = (size_t)threadIdx.x * 128; o < bytes; o += (size_t)THREADS * 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(c + o));
 }
 
+// STORE (qp_batch_factorize): no right-hand sides and no outputs; the factor of every instance that passes the pivot test is
+// written to `store` (FactorLayout, `stride` doubles per instance) instead of being used, every other instance is listed in
+// fb_list and marked in the store.
+template <bool STORE>
 __global__ void __launch_bounds__(THREADS, 4) qp_kkt_sqd_any_kernel(QpSolveArgs a, int* fb_list, int* fb_count, const int nt_cap,
-                                                                     int* max_active, const int max_tag) {
+                                                                     int* max_active, const int max_tag, double* store,
+                                                                     const int64_t stride) {
     extern __shared__ __align__(16) double sm[];
     const int n = a.n, m = a.m, p = a.p, N = n + m + p;
     const Layout lay(n, m, p, nt_cap);
@@ -158,7 +163,7 @@ __global__ void __launch_bounds__(THREADS, 4) qp_kkt_sqd_any_kernel(QpSolveArgs 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int g = lane >> 2, t = lane & 3;
     const int fo = el(g, 2 * t);
-    const bool do_fwd = a.fwd != nullptr, do_rev = a.rev != nullptr;
+    const bool do_fwd = !STORE && a.fwd != nullptr, do_rev = !STORE && a.rev != nullptr;
 #ifdef QP_PROFILE
     long long sub[6] = {0, 0, 0, 0, 0, 0};
     long long pc[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
@@ -213,7 +218,10 @@ __global__ void __launch_bounds__(THREADS, 4) qp_kkt_sqd_any_kernel(QpSolveArgs 
         const int ma = scal[0], nt = scal[1];
         const int nred = n8 + ma + p, np = nt << 3;
         if (nt > nt_cap) {  // larger than this launch was configured for: the pivoted-LU kernel takes it
-            if (tid == 0) fb_list[atomicAdd(fb_count, 1)] = (int)inst;
+            if (tid == 0) {
+                fb_list[atomicAdd(fb_count, 1)] = (int)inst;
+                if (STORE) reinterpret_cast<int*>(store + b * stride)[0] = -1;
+            }
             __syncthreads();
             continue;
         }
@@ -323,6 +331,31 @@ __global__ void __launch_bounds__(THREADS, 4) qp_kkt_sqd_any_kernel(QpSolveArgs 
         factor<0>(T, V, nt, np, ntz, tid, lane, warp, g, t, fo SQD_SUB_ARG);
         __syncthreads();
         APROF(4);
+        if constexpr (STORE) {
+            double* F = store + b * stride;
+            int* Fi = reinterpret_cast<int*>(F);
+            const FactorLayout fl(m, nt_cap);
+            if (scal[2] == 0) {
+                const double2* T2 = reinterpret_cast<const double2*>(T);
+                double2* F2 = reinterpret_cast<double2*>(F + fl.tiles);
+                const int cnt = ((nt * (nt + 1)) >> 1) * 32;
+                for (int i = tid; i < cnt; i += THREADS) F2[i] = T2[i];
+                for (int i = tid; i < np; i += THREADS) F[fl.rd + i] = V.rd[i];
+                for (int i = tid; i < m; i += THREADS) {
+                    F[fl.dvec + i] = dvec[i];
+                    Fi[1 + i] = apos[i];
+                }
+                if (tid == 0) {
+                    Fi[0] = ma;
+                    if (a.info) a.info[inst] = 0;
+                }
+            } else if (tid == 0) {
+                fb_list[atomicAdd(fb_count, 1)] = (int)inst;
+                Fi[0] = -1;
+            }
+            __syncthreads();
+            continue;
+        }
         {
             const int lines = (int)(((size_t)m * n * sizeof(double) + 127) / 128);
             backward(T, V, nt, lane, warp, (do_rev && G) ? (const char*)G : nullptr, lines < 1024 ? lines : 1024);
@@ -435,7 +468,7 @@ int32_t qp_sqd_any_launch(diffopt_b200_ctx* ctx, const QpSolveArgs& a, int nt_ca
     int* fb_list = fb_count + 1;
     DO_CUDA(ctx, cudaMemsetAsync(fb_count, 0, sizeof(int), ctx->stream));
     int per_sm = 1;
-    DO_CUDA(ctx, kernel_config((const void*)qp_kkt_sqd_any_kernel, ctx->device, THREADS, smem, &per_sm));
+    DO_CUDA(ctx, kernel_config((const void*)qp_kkt_sqd_any_kernel<false>, ctx->device, THREADS, smem, &per_sm));
     if (per_sm < 1) per_sm = 1;
     int64_t grid = (int64_t)ctx->sm_count * per_sm;
     if (grid > a.B) grid = a.B;
@@ -448,7 +481,8 @@ int32_t qp_sqd_any_launch(diffopt_b200_ctx* ctx, const QpSolveArgs& a, int nt_ca
         DO_CUDA(ctx, cudaMemsetAsync(dprof, 0, 16 * sizeof(long long), ctx->stream));
         aa.prof = dprof;
     }
-    qp_kkt_sqd_any_kernel<<<(unsigned)grid, THREADS, smem, ctx->stream>>>(aa, fb_list, fb_count, nt_cap, max_active, max_tag);
+    qp_kkt_sqd_any_kernel<false><<<(unsigned)grid, THREADS, smem, ctx->stream>>>(aa, fb_list, fb_count, nt_cap, max_active, max_tag,
+                                                                                 nullptr, 0);
     ctx->launches++;
     DO_CUDA(ctx, cudaGetLastError());
     if (profile) {  // per-phase clocks of CTA 0 (profile build: DIFFOPT_B200_BUILD_PROFILE=1)
@@ -463,4 +497,26 @@ int32_t qp_sqd_any_launch(diffopt_b200_ctx* ctx, const QpSolveArgs& a, int nt_ca
     }
     *handled = true;
     return qp_generic_launch_list(ctx, a, fb_list, fb_count);
+}
+
+// Store mode (qp_batch_factorize): the same factorisation of every instance of `a` (no right-hand sides), factors written to
+// `store` (FactorLayout(m, nt_cap), `stride` doubles per instance); instances that fail the pivot test or exceed nt_cap are
+// appended to fb_list / *fb_count (cleared here).  a.info[b] = 0 for every stored instance.
+int32_t qp_sqd_any_store_launch(diffopt_b200_ctx* ctx, const QpSolveArgs& a, int nt_cap, double* store, int64_t stride, int* fb_list,
+                                int* fb_count) {
+    const size_t smem = (size_t)Layout(a.n, a.m, a.p, nt_cap).total * sizeof(double);
+    DO_CUDA(ctx, cudaMemsetAsync(fb_count, 0, sizeof(int), ctx->stream));
+    int per_sm = 1;
+    DO_CUDA(ctx, kernel_config((const void*)qp_kkt_sqd_any_kernel<true>, ctx->device, THREADS, smem, &per_sm));
+    if (per_sm < 1) per_sm = 1;
+    int64_t grid = (int64_t)ctx->sm_count * per_sm;
+    if (grid > a.B) grid = a.B;
+    if (grid < 1) grid = 1;
+    QpSolveArgs aa = a;
+    aa.fwd = aa.rev = nullptr;
+    aa.prof = nullptr;
+    qp_kkt_sqd_any_kernel<true><<<(unsigned)grid, THREADS, smem, ctx->stream>>>(aa, fb_list, fb_count, nt_cap, nullptr, 0, store, stride);
+    ctx->launches++;
+    DO_CUDA(ctx, cudaGetLastError());
+    return 0;
 }

@@ -17,6 +17,7 @@
 
 int32_t qp_solve_common(diffopt_b200_ctx* ctx, QpSolveArgs a, double* fwd_user, double* rev_user, int32_t* info_user, int memspace,
                         bool async);
+int32_t qp_factored_run(diffopt_b200_ctx* ctx, int64_t k, const double* in, double* out_user, int memspace, bool fwd);
 
 namespace {
 
@@ -36,25 +37,27 @@ __global__ void unpack_lower_kernel(const double* __restrict__ packed, double* _
 
 // Forward right-hand side [dQ z + dq + dG'lam + dA'nu; dG z - dh; dA z - db] (QuadraticProgram.jl:429-433, the middle block
 // before its scaling by lam) from the direction's sparse triplets -- what the reference holds after diff_opt.jl:594-656 and
-// SparseArrays.sparse (duplicates add up).  One thread per instance walks its triplets in storage order (a fixed
-// summation order); an index outside its matrix raises *err and is skipped.
+// SparseArrays.sparse (duplicates add up).  One thread per slot walks its triplets in storage order (a fixed summation
+// order); an index outside its matrix raises *err and is skipped.  k directions per instance: slot s = b k + j is direction j
+// of instance b (triplets, dq, dh, db and rhs are per slot; z, lam, nu per instance).
 struct CooDev {
     const int64_t *ptr, *I, *J;
     const double* V;
 };
 
-__global__ void qp_coo_rhs_kernel(const int64_t B, const int n, const int m, const int p, const double* __restrict__ z,
+__global__ void qp_coo_rhs_kernel(const int64_t B, const int64_t k, const int n, const int m, const int p, const double* __restrict__ z,
                                   const double* __restrict__ lam, const double* __restrict__ nu, const CooDev cq, const CooDev cg,
                                   const CooDev ca, const double* __restrict__ dq, const double* __restrict__ dh,
                                   const double* __restrict__ db, const int shared_dir, double* __restrict__ rhs, int* err) {
     const int N = n + m + p;
-    for (int64_t b = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; b < B; b += (int64_t)gridDim.x * blockDim.x) {
-        double* r = rhs + b * N;
+    for (int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; s < B * k; s += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = s / k;
+        double* r = rhs + s * N;
         const double* zb = z + b * n;
-        const int64_t bt = shared_dir ? 0 : b;
-        for (int i = 0; i < n; ++i) r[i] = dq ? dq[b * n + i] : 0.0;
-        for (int i = 0; i < m; ++i) r[n + i] = dh ? -dh[b * m + i] : 0.0;
-        for (int i = 0; i < p; ++i) r[n + m + i] = db ? -db[b * p + i] : 0.0;
+        const int64_t bt = shared_dir ? 0 : s;
+        for (int i = 0; i < n; ++i) r[i] = dq ? dq[s * n + i] : 0.0;
+        for (int i = 0; i < m; ++i) r[n + i] = dh ? -dh[s * m + i] : 0.0;
+        for (int i = 0; i < p; ++i) r[n + m + i] = db ? -db[s * p + i] : 0.0;
         if (cq.ptr)
             for (int64_t k = cq.ptr[bt]; k < cq.ptr[bt + 1]; ++k) {
                 const int64_t i = cq.I[k] - 1, j = cq.J[k] - 1;
@@ -78,6 +81,39 @@ __global__ void qp_coo_rhs_kernel(const int64_t B, const int n, const int m, con
                 r[j] += v * nu[b * p + i];
             }
     }
+}
+
+// The triplets of dQ, dG, dA on the device: used in place (device memspace) or, after their offsets were checked, staged into
+// ctx->qp_coo[0..2] as ptr | I | J | V back to back (host memspace).  `slots` = entries of ptr minus one.
+int32_t stage_triplets(diffopt_b200_ctx* ctx, const char* who, const diffopt_b200_coo_batch* const src[3], const int lim_rows[3],
+                       const int64_t slots, const int memspace, CooDev dev[3]) {
+    for (int q = 0; q < 3; ++q) {
+        const diffopt_b200_coo_batch* c = src[q];
+        dev[q] = CooDev{};
+        if (!c || !c->ptr || lim_rows[q] == 0) continue;
+        if (memspace == DIFFOPT_B200_DEVICE) {
+            dev[q] = CooDev{c->ptr, c->I, c->J, c->V};
+            continue;
+        }
+        const int64_t nnz = c->ptr[slots];
+        if (c->ptr[0] != 0 || nnz < 0 || (nnz > 0 && (!c->I || !c->J || !c->V)))
+            BAD_ARG(ctx, std::string(who) + ": triplet offsets must start at 0 and I, J, V must be given");
+        for (int64_t b = 0; b < slots; ++b)
+            if (c->ptr[b + 1] < c->ptr[b]) BAD_ARG(ctx, std::string(who) + ": triplet offsets must be nondecreasing");
+        const size_t np8 = sizeof(int64_t) * (size_t)(slots + 1), nz8 = sizeof(int64_t) * (size_t)nnz;
+        DevBuf& buf = ctx->qp_coo[q];
+        DO_CUDA(ctx, buf.reserve(np8 + 3 * nz8 + 8));
+        char* base = buf.as<char>();
+        DO_CUDA(ctx, cudaMemcpyAsync(base, c->ptr, np8, cudaMemcpyHostToDevice, ctx->stream));
+        if (nnz > 0) {
+            DO_CUDA(ctx, cudaMemcpyAsync(base + np8, c->I, nz8, cudaMemcpyHostToDevice, ctx->stream));
+            DO_CUDA(ctx, cudaMemcpyAsync(base + np8 + nz8, c->J, nz8, cudaMemcpyHostToDevice, ctx->stream));
+            DO_CUDA(ctx, cudaMemcpyAsync(base + np8 + 2 * nz8, c->V, nz8, cudaMemcpyHostToDevice, ctx->stream));
+        }
+        dev[q] = CooDev{(const int64_t*)base, (const int64_t*)(base + np8), (const int64_t*)(base + np8 + nz8),
+                        (const double*)(base + np8 + 2 * nz8)};
+    }
+    return 0;
 }
 
 constexpr int GR_THREADS = 256;
@@ -400,42 +436,17 @@ int32_t diffopt_b200_qp_batch_solve_coo(diffopt_b200_ctx* ctx, int64_t B, int32_
     STAGE_COO(12, ddb, db, (size_t)B * p)
     if (rev_out) { STAGE_COO(13, a.seed, dl_dz, (size_t)B * n) }
 #undef STAGE_COO
-    // triplets: one staging buffer per matrix holding ptr | I | J | V back to back (host memspace), or used in place
-    CooDev dev[3] = {};
+    CooDev dev[3];
     const diffopt_b200_coo_batch* src[3] = {dQ, dG, dA};
     const int lim_rows[3] = {n, m, p};
-    for (int q = 0; q < 3; ++q) {
-        const diffopt_b200_coo_batch* c = src[q];
-        if (!c || !c->ptr || lim_rows[q] == 0) continue;
-        if (memspace == DIFFOPT_B200_DEVICE) {
-            dev[q] = CooDev{c->ptr, c->I, c->J, c->V};
-            continue;
-        }
-        const int64_t nnz = c->ptr[Bd];
-        if (c->ptr[0] != 0 || nnz < 0 || (nnz > 0 && (!c->I || !c->J || !c->V)))
-            BAD_ARG(ctx, "qp_batch_solve_coo: triplet offsets must start at 0 and I, J, V must be given");
-        for (int64_t b = 0; b < Bd; ++b)
-            if (c->ptr[b + 1] < c->ptr[b]) BAD_ARG(ctx, "qp_batch_solve_coo: triplet offsets must be nondecreasing");
-        const size_t np8 = sizeof(int64_t) * (size_t)(Bd + 1), nz8 = sizeof(int64_t) * (size_t)nnz;
-        DevBuf& buf = ctx->qp_coo[q];
-        DO_CUDA(ctx, buf.reserve(np8 + 3 * nz8 + 8));
-        char* base = buf.as<char>();
-        DO_CUDA(ctx, cudaMemcpyAsync(base, c->ptr, np8, cudaMemcpyHostToDevice, ctx->stream));
-        if (nnz > 0) {
-            DO_CUDA(ctx, cudaMemcpyAsync(base + np8, c->I, nz8, cudaMemcpyHostToDevice, ctx->stream));
-            DO_CUDA(ctx, cudaMemcpyAsync(base + np8 + nz8, c->J, nz8, cudaMemcpyHostToDevice, ctx->stream));
-            DO_CUDA(ctx, cudaMemcpyAsync(base + np8 + 2 * nz8, c->V, nz8, cudaMemcpyHostToDevice, ctx->stream));
-        }
-        dev[q] = CooDev{(const int64_t*)base, (const int64_t*)(base + np8), (const int64_t*)(base + np8 + nz8),
-                        (const double*)(base + np8 + 2 * nz8)};
-    }
+    if (int32_t rc = stage_triplets(ctx, "qp_batch_solve_coo", src, lim_rows, Bd, memspace, dev)) return rc;
     const int N = n + m + p;
     DO_CUDA(ctx, ctx->qp_coo[3].reserve(d * (size_t)B * N + sizeof(int)));
     double* rhs = ctx->qp_coo[3].as<double>();
     int* derr = reinterpret_cast<int*>(rhs + (size_t)B * N);
     DO_CUDA(ctx, cudaMemsetAsync(derr, 0, sizeof(int), ctx->stream));
     const int64_t blocks = std::min<int64_t>((B + 63) / 64, (int64_t)ctx->sm_count * 8);
-    qp_coo_rhs_kernel<<<(unsigned)blocks, 64, 0, ctx->stream>>>(B, n, m, p, a.z, a.lam, a.nu, dev[0], dev[1], dev[2], ddq, ddh, ddb,
+    qp_coo_rhs_kernel<<<(unsigned)blocks, 64, 0, ctx->stream>>>(B, 1, n, m, p, a.z, a.lam, a.nu, dev[0], dev[1], dev[2], ddq, ddh, ddb,
                                                               shd ? 1 : 0, rhs, derr);
     ctx->launches++;
     DO_CUDA(ctx, cudaGetLastError());
@@ -445,6 +456,46 @@ int32_t diffopt_b200_qp_batch_solve_coo(diffopt_b200_ctx* ctx, int64_t B, int32_
     int herr = 0;  // the blocking call has synchronised: out-of-range triplet indices are an argument error
     DO_CUDA(ctx, cudaMemcpy(&herr, derr, sizeof(int), cudaMemcpyDeviceToHost));
     if (herr) BAD_ARG(ctx, "qp_batch_solve_coo: a triplet index lies outside its matrix (1-based I, J expected)");
+    return rc;
+}
+
+int32_t diffopt_b200_qp_batch_forward_multi(diffopt_b200_ctx* ctx, int64_t k, const diffopt_b200_coo_batch* dQ, const double* dq,
+                                            const diffopt_b200_coo_batch* dG, const double* dh, const diffopt_b200_coo_batch* dA,
+                                            const double* db, double* fwd_out, int32_t memspace) {
+    if (!ctx) return -1;
+    DeviceGuard guard_(ctx->device);
+    if (!ctx->qpf.valid) BAD_ARG(ctx, "qp_batch_forward_multi: call qp_batch_factorize first (qp_batch_setup drops the stored factor)");
+    if (k < 0) BAD_ARG(ctx, "qp_batch_forward_multi: need k >= 0");
+    const QpBatchState& s = ctx->qp;
+    const int64_t B = s.B;
+    const int n = s.n, m = s.m, p = s.p, N = n + m + p;
+    if (k == 0 || B == 0) return 0;
+    if (!fwd_out) BAD_ARG(ctx, "qp_batch_forward_multi: fwd_out is required");
+    const int64_t S = B * k;  // direction j of instance b is slot b k + j
+    const size_t d = sizeof(double);
+    const void *ddq, *ddh, *ddb;
+    DO_CUDA(ctx, stage_in(ctx, ctx->in[8], dq, d * (size_t)S * n, memspace, &ddq));
+    DO_CUDA(ctx, stage_in(ctx, ctx->in[10], dh, d * (size_t)S * m, memspace, &ddh));
+    DO_CUDA(ctx, stage_in(ctx, ctx->in[12], db, d * (size_t)S * p, memspace, &ddb));
+    CooDev dev[3];
+    const diffopt_b200_coo_batch* src[3] = {dQ, dG, dA};
+    const int lim_rows[3] = {n, m, p};
+    if (int32_t rc = stage_triplets(ctx, "qp_batch_forward_multi", src, lim_rows, S, memspace, dev)) return rc;
+    DO_CUDA(ctx, ctx->qp_coo[3].reserve(d * (size_t)S * N + sizeof(int)));
+    double* rhs = ctx->qp_coo[3].as<double>();
+    int* derr = reinterpret_cast<int*>(rhs + (size_t)S * N);
+    DO_CUDA(ctx, cudaMemsetAsync(derr, 0, sizeof(int), ctx->stream));
+    const int64_t blocks = std::max<int64_t>(1, std::min<int64_t>((S + 63) / 64, (int64_t)ctx->sm_count * 8));
+    qp_coo_rhs_kernel<<<(unsigned)blocks, 64, 0, ctx->stream>>>(B, k, n, m, p, s.z.as<double>(), s.lam.as<double>(), s.nu.as<double>(),
+                                                              dev[0], dev[1], dev[2], (const double*)ddq, (const double*)ddh,
+                                                              (const double*)ddb, 0, rhs, derr);
+    ctx->launches++;
+    DO_CUDA(ctx, cudaGetLastError());
+    const int32_t rc = qp_factored_run(ctx, k, rhs, fwd_out, memspace, true);
+    if (rc < 0) return rc;
+    int herr = 0;  // qp_factored_run has synchronised: out-of-range triplet indices are an argument error
+    DO_CUDA(ctx, cudaMemcpy(&herr, derr, sizeof(int), cudaMemcpyDeviceToHost));
+    if (herr) BAD_ARG(ctx, "qp_batch_forward_multi: a triplet index lies outside its matrix (1-based I, J expected)");
     return rc;
 }
 

@@ -17,6 +17,25 @@ constexpr double PIV_RTOL = 1e-12;
 
 __device__ __forceinline__ int tix(int I, int J) { return ((I * (I + 1)) >> 1) + J; }
 
+// One instance's stored LDL' factor (qp_batch_factorize; written by the store mode of qp_kkt_sqd_any_kernel, read by
+// qp_batch_factored.cu), `stride` doubles per instance, every segment 16-byte aligned:
+//   ints  [0] = ma, the active-set size (-1: the instance is served by the pivoted LU), [1 .. m] = apos (reduced row of
+//         inequality i minus n8, -1 when inactive)
+//   dvec  D = G z - h (m)
+//   rd    1 / d of every reduced row (8 nt_cap)
+//   tiles the lower-triangular tile grid (tix order) exactly as factor<>() leaves it: strict lower triangles of the
+//         diagonal tiles hold L_jj, the tiles below the diagonal W(I, j) = L(I, j) D_j, in-tile swizzle of el()
+struct FactorLayout {
+    int ints, dvec, rd, tiles, stride;
+    __host__ __device__ FactorLayout(int m, int nt_cap) {
+        ints = 0;
+        dvec = (((m + 2) >> 1) + 1) & ~1;
+        rd = dvec + ((m + 1) & ~1);
+        tiles = rd + 8 * nt_cap;
+        stride = (tiles + (nt_cap * (nt_cap + 1) / 2) * 64 + 15) & ~15;
+    }
+};
+
 // Offset of element (r, c) inside an 8 x 8 tile.  Rows are 64 B; the four 16-byte chunks of row r are stored at
 // chunk ^ ((r >> 1) & 3).  DMMA fragment accesses (lane (g, t) -> chunk t of row g) and whole-row accesses (one lane
 // per row, chunk q of rows 0..7) are then both free of shared-memory bank conflicts.

@@ -86,6 +86,49 @@ class QPBatch:
         self._raise_if_singular(rc)
         return self._split(out)
 
+    def factorize(self):
+        """``diffopt_b200_qp_batch_factorize``: keep every instance's LDL' factor on the device for ``reverse_multi`` /
+        ``forward_multi`` (until the next setup).  Raises SingularException for a singular instance (``info`` is kept: the
+        multi calls raise for the same instance)."""
+        rc = self.ctx.lib.diffopt_b200_qp_batch_factorize(self.ctx.h, ptr(self.info), HOST)
+        self._raise_if_singular(rc)
+
+    def reverse_multi(self, seeds):
+        """k reverse seeds per instance, ``seeds`` (B, k, n) -> (dz, dλ, dν), each (B, k, ·): one ``reverse`` per seed."""
+        seeds = np.asarray(seeds, float)
+        k = seeds.shape[1]
+        seeds = np.ascontiguousarray(seeds.reshape(self.B, k, self.n))
+        out = np.empty((self.B, k, self.N))
+        rc = self.ctx.lib.diffopt_b200_qp_batch_reverse_multi(self.ctx.h, k, ptr(seeds), ptr(out), HOST)
+        self._raise_if_singular(rc)
+        return self._split_multi(out)
+
+    def forward_multi(self, k, dQ=None, dq=None, dG=None, dh=None, dA=None, db=None):
+        """k forward directions per instance: dq (B, k, n), dh (B, k, m), db (B, k, p); dQ, dG, dA as B*k scipy.sparse
+        matrices in slot order (direction j of instance b at b*k + j, see ``coo_batch``); any may be None (zero).
+        Returns (dz, dλ, dν), each (B, k, ·): one ``forward`` per direction."""
+        B, n, m, p = self.B, self.n, self.m, self.p
+        vec = lambda v, r: None if v is None or r == 0 else np.ascontiguousarray(np.asarray(v, float).reshape(B, k, r))
+        keep = []
+
+        def coo(mats, rows):
+            arrs = coo_batch(mats, B * k) if rows else None
+            if arrs is None:
+                return None
+            st = _capi.CooBatch(*[a.ctypes.data for a in arrs])
+            keep.append((arrs, st))
+            return _capi.C.addressof(st)
+        dvecs = [vec(dq, n), vec(dh, m), vec(db, p)]
+        out = np.empty((B, k, self.N))
+        rc = self.ctx.lib.diffopt_b200_qp_batch_forward_multi(self.ctx.h, k, coo(dQ, n), ptr(dvecs[0]), coo(dG, m), ptr(dvecs[1]),
+                                                              coo(dA, p), ptr(dvecs[2]), ptr(out), HOST)
+        self._raise_if_singular(rc)
+        return self._split_multi(out)
+
+    def _split_multi(self, out):
+        n, m = self.n, self.m
+        return out[..., :n], out[..., n:n + m], out[..., n + m:]
+
     def param_grads(self, rev, reduce_over_batch=False):
         """dQ, dq, dG, dh, dA, db from rev = concatenated (dz, dlam, dnu) (B, N)."""
         B, n, m, p = self.B, self.n, self.m, self.p

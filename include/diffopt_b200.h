@@ -132,7 +132,8 @@ int32_t diffopt_b200_synchronize(diffopt_b200_ctx* ctx);
 /* Diagnostics of the last qp_batch call on this ctx (waits for the stream): out3[0] = instances the pivot-free LDL'
  * fast path handed to the partially pivoted LU kernel (semidefinite Q, rank-deficient active set, ... -- results are
  * the same, throughput is not), out3[1] = active-set size the launch was configured for, out3[2] = kernel that served
- * the call (0 generic pivoted LU, 1 tuned pivoted LU, 2 LDL' fast path). */
+ * the call (0 generic pivoted LU, 1 tuned pivoted LU, 2 LDL' fast path, 3 stored LDL' of qp_batch_factorize -- then out3[0]
+ * counts the instances the multi calls serve with the pivoted LU and out3[1] is the tile order the factors were stored for). */
 int32_t diffopt_b200_qp_batch_last_stats(diffopt_b200_ctx* ctx, int64_t* out3);
 
 /* Extended form of qp_batch_solve.  flags (OR of):
@@ -216,6 +217,30 @@ int32_t diffopt_b200_qp_batch_forward(
     diffopt_b200_ctx* ctx, const double* dQ, const double* dq, const double* dG,
     const double* dh, const double* dA, const double* db,
     double* fwd_out, int32_t* info, int32_t memspace);
+
+/* Factorise once, solve many directions.  qp_batch_factorize (after qp_batch_setup) computes the LDL' factor of every
+ * instance's reduced KKT system and keeps it on the device (about 40 KB per instance at n=64, m=64, p=16 with 16 active
+ * rows); a new qp_batch_setup drops it, destroy frees it.  The multi calls then take k directions per instance and cost two
+ * triangular sweeps over the stored factor per direction instead of a full assembly and factorisation.  Instances the
+ * pivot-free factorisation rejects (semidefinite Q, rank-deficient active set, wrong-sign duals, an active set beyond shared
+ * memory) are listed at factorize time and solved by the pivoted LU, one launch per direction.
+ *   factorize: info[B] (may be NULL) as in qp_batch_solve.  Returns 0, first singular instance + 1, -3 when the factor
+ *     storage cannot be allocated.
+ *   reverse_multi: dl_dz[B][k][n] (instance-major, then direction: Julia's Array{Float64,3} of size (n, k, B)) ->
+ *     rev_out[B][k][N], direction j of instance b = what qp_batch_reverse returns for that seed (to rounding: the sums run
+ *     in another order).
+ *   forward_multi: dq[B][k][n], dh[B][k][m], db[B][k][p] (any may be NULL = zero); dQ, dG, dA as in qp_batch_solve_coo
+ *     with B*k+1 offsets (direction j of instance b is slot b*k + j) -> fwd_out[B][k][N], direction j of instance b = what
+ *     qp_batch_forward returns for that direction.  -1 when a triplet index lies outside its matrix.
+ *   Both return 0, first singular instance + 1, or < 0 (a call before factorize, or after a new setup, is -1 and
+ *   diffopt_b200_last_error names the missing step); k = 0 returns 0. */
+int32_t diffopt_b200_qp_batch_factorize(diffopt_b200_ctx* ctx, int32_t* info, int32_t memspace);
+int32_t diffopt_b200_qp_batch_reverse_multi(
+    diffopt_b200_ctx* ctx, int64_t k, const double* dl_dz, double* rev_out, int32_t memspace);
+int32_t diffopt_b200_qp_batch_forward_multi(
+    diffopt_b200_ctx* ctx, int64_t k,
+    const diffopt_b200_coo_batch* dQ, const double* dq, const diffopt_b200_coo_batch* dG, const double* dh,
+    const diffopt_b200_coo_batch* dA, const double* db, double* fwd_out, int32_t memspace);
 
 /* Reverse-mode gradients w.r.t. the problem data from rev = (dz, dlam, dnu)
  * (getters QuadraticProgram.jl:307-314, :448-473; signs as the reference's tests read

@@ -199,6 +199,68 @@ end
 
 synchronize(ctx::Context) = check(ctx, ccall((:diffopt_b200_synchronize, LIB), Int32, (Ptr{Cvoid},), ctx.handle))
 
+# Factorise once, solve many directions: setup keeps the batch resident, factorize stores every instance's LDL' factor, the
+# multi calls take k directions per instance as Array{Float64,3} of size (rows, k, B) and return (N, k, B) blocks.
+function qp_batch_setup(ctx::Context, Q, G, A, h, z, lam, nu)
+    n, B = size(z)
+    m = size(lam, 1)
+    p = size(nu, 1)
+    GC.@preserve Q G A h z lam nu begin
+        rc = ccall((:diffopt_b200_qp_batch_setup, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Int32, Int32, Int32,
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32),
+                   ctx.handle, B, n, m, p, _p(Q), _p(G), _p(A), _p(h), _p(z), _p(lam), _p(nu), HOST)
+    end
+    check(ctx, rc)
+    return (B = B, n = n, m = m, p = p)
+end
+
+function qp_batch_factorize(ctx::Context, B::Integer)
+    info = zeros(Int32, B)
+    rc = ccall((:diffopt_b200_qp_batch_factorize, LIB), Int32, (Ptr{Cvoid}, Ptr{Int32}, Int32), ctx.handle, info, HOST)
+    check(ctx, rc)
+    return info
+end
+
+function qp_batch_reverse_multi(ctx::Context, shape, dl_dz::Array{Float64,3})
+    n, k, B = size(dl_dz)
+    N = shape.n + shape.m + shape.p
+    rev = Array{Float64,3}(undef, N, k, B)
+    GC.@preserve dl_dz rev begin
+        rc = ccall((:diffopt_b200_qp_batch_reverse_multi, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Int32), ctx.handle, k, dl_dz, rev, HOST)
+    end
+    check(ctx, rc)
+    return rev
+end
+
+# dQ, dG, dA: (ptr, I, J, V) of the B*k direction slots (0-based offsets, 1-based I, J), or nothing
+struct CooBatch
+    ptr::Ptr{Int64}
+    I::Ptr{Int64}
+    J::Ptr{Int64}
+    V::Ptr{Float64}
+end
+_coo(t::Nothing) = nothing
+_coo(t::Tuple) = Ref(CooBatch(pointer(t[1]), pointer(t[2]), pointer(t[3]), pointer(t[4])))
+_cp(r::Nothing) = Ptr{CooBatch}(C_NULL)
+_cp(r::Ref{CooBatch}) = Base.unsafe_convert(Ptr{CooBatch}, r)
+
+function qp_batch_forward_multi(ctx::Context, shape, k::Integer; dQ = nothing, dq = nothing, dG = nothing, dh = nothing,
+                                dA = nothing, db = nothing)
+    N = shape.n + shape.m + shape.p
+    fwd = Array{Float64,3}(undef, N, k, shape.B)
+    cq, cg, ca = _coo(dQ), _coo(dG), _coo(dA)
+    GC.@preserve dQ dq dG dh dA db cq cg ca fwd begin
+        rc = ccall((:diffopt_b200_qp_batch_forward_multi, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Ptr{CooBatch}, Ptr{Float64}, Ptr{CooBatch}, Ptr{Float64}, Ptr{CooBatch}, Ptr{Float64},
+                    Ptr{Float64}, Int32),
+                   ctx.handle, k, _cp(cq), _p(dq), _cp(cg), _p(dh), _cp(ca), _p(db), fwd, HOST)
+    end
+    check(ctx, rc)
+    return fwd
+end
+
 # ------------------------------------------------------------------------------------------------
 # (3) ConicProgram backend: _gradient_cache / forward / reverse (src/ConicProgram/ConicProgram.jl:172-394)
 #     cone_type: 0 Zeros, 1 Nonnegatives, 2 SecondOrderCone, 3 PositiveSemidefiniteConeTriangle, 4 ExponentialCone,
