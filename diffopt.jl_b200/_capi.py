@@ -67,6 +67,10 @@ SIGNATURES = {
                                                C.c_int64, vp, vp, vp, C.c_int32]),
     "diffopt_b200_conic_reverse": (C.c_int32, [vp, vp, C.c_double, C.c_double, C.c_double, C.c_int64, vp, vp, vp, vp,
                                                C.c_int32]),
+    "diffopt_b200_conic_forward_multi": (C.c_int32, [vp, C.c_int64, vp, vp, vp, C.c_double, C.c_double, C.c_double,
+                                                     C.c_int64, vp, vp, vp, C.c_int32]),
+    "diffopt_b200_conic_reverse_multi": (C.c_int32, [vp, C.c_int64, vp, C.c_double, C.c_double, C.c_double, C.c_int64,
+                                                     vp, vp, vp, vp, C.c_int32]),
     "diffopt_b200_conic_batch_begin": (C.c_int32, [vp, C.c_int64, C.c_int32]),
     "diffopt_b200_conic_batch_add": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, C.c_int32]),
     "diffopt_b200_conic_batch_add_ex": (C.c_int32, [vp, C.c_int64, C.c_int64] + [vp] * 8 + [C.c_int64, vp, vp, vp, C.c_int32]),

@@ -9,6 +9,7 @@ import time
 
 import numpy as np
 
+from . import _capi
 from ._capi import (CONE_DUAL_EXP, CONE_DUAL_POW, CONE_EXP, CONE_NONNEG, CONE_POW, CONE_PSD, CONE_SOC,  # noqa: F401
                     CONE_ZERO, HOST, Context, ptr)
 from .lsqr import DEFAULTS, julia_csc
@@ -131,6 +132,49 @@ class ConicModel:
         self.last_stats = dict(istop=int(stats[0]), itn=int(stats[1]), rnorm=stats[2], arnorm=stats[3],
                                kernel_ms=self.ctx.last_kernel_ms)
         self.diff_time = time.perf_counter() - t0
+
+    def forward_differentiate_multi(self, dAs=None, dbs=None, dcs=None, k=None):
+        """k forward directions in one call (``diffopt_b200_conic_forward_multi``): dAs a list of k sparse / dense (m x n)
+        matrices or None entries (zero), dbs (k, m), dcs (k, n); any may be None.  k is taken from the inputs unless
+        given.  Returns dict(dx (k, n), dz (k, n+m+1), stats (k, 4)); direction j equals ``forward_differentiate`` of
+        (dAs[j], dbs[j], dcs[j]) up to rounding.  The model's own caches are not touched."""
+        import scipy.sparse as sp
+        from .qp import coo_batch
+        self._gradient_cache()
+        n, m = self.n, self.m
+        if k is None:
+            k = next(len(v) for v in (dAs, dbs, dcs) if v is not None)
+        vec = lambda v, r: None if v is None else np.ascontiguousarray(np.asarray(v, float).reshape(k, r))
+        dbs, dcs = vec(dbs, m), vec(dcs, n)
+        keep = None
+        if dAs is not None:
+            if len(dAs) != k:
+                raise ValueError("dAs needs one entry per direction")
+            arrs = coo_batch([sp.csr_matrix((m, n)) if M is None else M for M in dAs], k)
+            keep = (arrs, _capi.CooBatch(*[a.ctypes.data for a in arrs]))
+        dx = np.empty((k, n))
+        dz = np.empty((k, n + m + 1))
+        stats = np.zeros((k, 4))
+        rc = self.ctx.lib.diffopt_b200_conic_forward_multi(self.ctx.h, k, None if keep is None else _capi.C.addressof(keep[1]),
+                                                           ptr(dbs), ptr(dcs), *self._tol(), ptr(dx), ptr(dz), ptr(stats), HOST)
+        self.ctx.check(rc)
+        return dict(dx=dx, dz=dz, stats=stats)
+
+    def reverse_differentiate_multi(self, dx_seeds):
+        """k reverse seeds in one call (``diffopt_b200_conic_reverse_multi``): dx_seeds (k, n) -> dict(g (k, n+m+1),
+        dc (k, n), db (k, m), stats (k, 4)); row j equals ``reverse_differentiate(dx_seeds[j])`` up to rounding."""
+        self._gradient_cache()
+        n, m = self.n, self.m
+        seeds = np.ascontiguousarray(np.asarray(dx_seeds, dtype=np.float64).reshape(-1, n))
+        k = seeds.shape[0]
+        g = np.empty((k, n + m + 1))
+        dc = np.empty((k, n))
+        db = np.empty((k, m))
+        stats = np.zeros((k, 4))
+        rc = self.ctx.lib.diffopt_b200_conic_reverse_multi(self.ctx.h, k, ptr(seeds), *self._tol(), ptr(g), ptr(dc), ptr(db),
+                                                           ptr(stats), HOST)
+        self.ctx.check(rc)
+        return dict(g=g, dc=dc, db=db, stats=stats)
 
     def reverse_differentiate(self, dx_seed):
         t0 = time.perf_counter()

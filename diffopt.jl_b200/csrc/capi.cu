@@ -70,7 +70,7 @@ int32_t diffopt_b200_destroy(diffopt_b200_ctx* ctx) {
     for (DevBuf* b : {&ctx->qpf.f, &ctx->qpf.fb, &ctx->qpf.gin, &ctx->qpf.gout}) b->release();
     conic_state_release(ctx->conic);
     LsqrWork& l = ctx->lsqr;
-    for (DevBuf* b : {&l.u, &l.v, &l.w, &l.x, &l.tmp, &l.scal}) b->release();
+    for (DevBuf* b : {&l.u, &l.v, &l.w, &l.x, &l.tmp, &l.scal, &l.m_rhs, &l.m_x, &l.m_scal, &l.m_work, &l.m_gather}) b->release();
     release_csr(ctx->lsqr_mat);
     sparse_mf_release(ctx);
     conic_batch_release(ctx);

@@ -115,6 +115,9 @@ void sparse_mf_release(struct diffopt_b200_ctx* ctx);
 
 struct LsqrWork {
     DevBuf u, v, w, x, tmp, scal;  // vectors and a small block of device scalars
+    // conic_forward_multi / conic_reverse_multi: right-hand sides and solutions ([group][N][KB]), their norms and
+    // statistics, the per-group work regions, and the gather lists of the forward right-hand sides
+    DevBuf m_rhs, m_x, m_scal, m_work, m_gather;
 };
 
 struct diffopt_b200_ctx {

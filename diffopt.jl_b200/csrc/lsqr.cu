@@ -1053,6 +1053,516 @@ __global__ void __launch_bounds__(ST_THREADS) st_end_kernel(int N, LsqrVectors v
 
 __global__ void st_stats_kernel(const LsqrState* S, double* stats) { S->sc.write_stats(stats); }
 
+// ================================================================================================================
+// Multi-right-hand-side LSQR (diffopt_b200_conic_forward_multi / _reverse_multi): KB right-hand sides against the SAME
+// conic operator M advance in lock-step in one persistent kernel.  Everything but the vectors is shared: one pass over
+// (val, colind) of A and A' per phase serves all KB directions, and the vectors are stored interleaved ([row][KB]), so
+// one gathered sector carries the values of several directions.  Per direction the arithmetic is that of lsqr_body
+// (the same LsqrScalars methods in the same order, fixed-order reductions), and no value of one direction depends on
+// another's: direction j gives the same bits whatever the other directions of its group hold.  A direction whose stop
+// test fired, or whose right-hand side failed the zero test, is frozen (its x and statistics are final, its vectors are
+// no longer written); the group ends when every direction is frozen.
+// Shape: 256-thread CTAs (the PSD GEMM phases are written for them) on the blk / t_blk row blocks (<= ST_CHUNK nonzeros,
+// <= SP_THREADS rows, or one longer row), KB products per nonzero parked in shared memory.
+constexpr int MR_THREADS = LSQR_THREADS;
+constexpr int MR_NPT = LSQR_NPT;
+constexpr int MR_PLD = ST_CHUNK + 1;  // products of direction j at prod[j * MR_PLD ..] (odd stride: row sums of the
+                                      // directions of one row fall into different banks)
+
+// Work of one group of KB directions against an operator of order N = n + m + 1 (offsets in doubles, all multiples of KB):
+// u, v, w (N KB each) | wc (2 m KB: Dpi t2 / r and Dpi' r) | PSD scratch W1, W2 (sumd2 KB each) | partial sums
+// (LSQR_NSLOTS KB ctas).
+struct MultiArgs {
+    ConicOpView op;            // row blocks blk / t_blk; op.wc and op.psd_w* are unused (per group, in `work`)
+    const double* rhs;         // [group][N][KB]
+    const double* rhs_norm2;   // [group][KB] squared norms of the right-hand sides (zero test)
+    double zero_below;         // a direction whose right-hand side has norm <= zero_below is not iterated
+    double* x;                 // [group][N][KB] solutions
+    double* stats;             // [group][KB][4] istop, itn, rnorm, arnorm
+    double* work;              // one region of `work_stride` doubles per group running concurrently
+    size_t work_stride;
+    long long sumd2;
+    int group0;                // first group of the launch
+    int ctas;                  // CTAs per group (cluster route; the cooperative route uses the whole grid)
+};
+
+template <int KB>
+__device__ __forceinline__ void mr_block_partial(Dev& d, int slot, double v) {
+    // thread t accumulates for direction t % KB: lanes of one direction are KB apart
+#pragma unroll
+    for (int o = 16; o >= KB; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (d.lane < KB) d.red[d.warp * KB + d.lane] = v;
+    __syncthreads();
+    if (d.tid < KB) {
+        double s = 0.0;
+        for (int w = 0; w < d.nwarp; ++w) s += d.red[w * KB + d.tid];
+        d.partials[(size_t)(slot * KB + d.tid) * d.nblk + d.rank()] = s;
+    }
+    __syncthreads();
+}
+
+// after a barrier: fixed-order sum of the CTA partials of (slot, direction j), identical in every CTA
+template <int KB>
+__device__ __forceinline__ double mr_total(const Dev& d, int slot, int j) {
+    const double* p = d.partials + (size_t)(slot * KB + j) * d.nblk;
+    double s = 0.0;
+    for (int i = 0; i < d.nblk; ++i) s += __ldcg(p + i);
+    return s;
+}
+
+// Row-block SpMM: spmv_stream for KB interleaved vectors.  Each (val, colind) is loaded once and KB contiguous values are
+// gathered with 16-byte loads; every row is summed per direction in storage order by one thread (direction j = thread
+// index % KB).  pre(b, row) / epi(b, row, t, operands) see the direction of the calling thread.
+template <int KB, class Sel, class Pre, class Epi>
+__device__ __forceinline__ void spmm_stream(int cta, int ncta, int nblk_total, double* prod, double* red, Sel&& sel, Pre&& pre,
+                                            Epi&& epi) {
+    constexpr int THREADS = MR_THREADS, NPT = MR_NPT, CHUNK = THREADS * NPT, KH = KB / 2;
+    const int tid = threadIdx.x;
+    const int per = (nblk_total + ncta - 1) / ncta;
+    const int b_end = min(nblk_total, (cta + 1) * per);
+    for (int b = cta * per; b < b_end; ++b) {
+        const CsrView* A;
+        const double* x;
+        int lb;
+        sel(b, A, x, lb);
+        const int2 d0 = __ldg(reinterpret_cast<const int2*>(A->blk) + lb);
+        const int2 d1 = __ldg(reinterpret_cast<const int2*>(A->blk) + lb + 1);
+        const int r0 = d0.x, s = d0.y, r1 = d1.x, cnt = d1.y - d0.y;
+        if (cnt > CHUNK) {  // one long row: whole CTA, fixed-order reduction per direction
+            double acc[KB];
+#pragma unroll
+            for (int j = 0; j < KB; ++j) acc[j] = 0.0;
+            for (int k = tid; k < cnt; k += THREADS) {
+                const double a = __ldg(A->val + s + k);
+                const double2* xp = reinterpret_cast<const double2*>(x + (size_t)__ldg(A->colind + s + k) * KB);
+#pragma unroll
+                for (int q = 0; q < KH; ++q) {
+                    const double2 xv = __ldcg(xp + q);
+                    acc[2 * q] = fma(a, xv.x, acc[2 * q]);
+                    acc[2 * q + 1] = fma(a, xv.y, acc[2 * q + 1]);
+                }
+            }
+#pragma unroll
+            for (int j = 0; j < KB; ++j) {
+                const double t = warp_sum_all(acc[j]);
+                if ((tid & 31) == 0) red[(tid >> 5) * KB + j] = t;
+            }
+            __syncthreads();
+            if (tid < KB) {
+                double t = 0.0;
+                for (int w = 0; w < THREADS / 32; ++w) t += red[w * KB + tid];
+                epi(b, r0, t, pre(b, r0));
+            }
+        } else {
+            double av[NPT];
+            int ci[NPT];
+#pragma unroll
+            for (int u = 0; u < NPT; ++u) {
+                const int k = tid + u * THREADS;
+                av[u] = 0.0;
+                ci[u] = 0;
+                if (k < cnt) {
+                    av[u] = __ldg(A->val + s + k);
+                    ci[u] = __ldg(A->colind + s + k);
+                }
+            }
+            double2 xv[NPT][KH];
+#pragma unroll
+            for (int u = 0; u < NPT; ++u) {
+                const double2* xp = reinterpret_cast<const double2*>(x + (size_t)ci[u] * KB);
+#pragma unroll
+                for (int q = 0; q < KH; ++q) xv[u][q] = tid + u * THREADS < cnt ? __ldcg(xp + q) : make_double2(0.0, 0.0);
+            }
+#pragma unroll
+            for (int u = 0; u < NPT; ++u) {
+                const int k = tid + u * THREADS;
+                if (k < cnt) {
+#pragma unroll
+                    for (int q = 0; q < KH; ++q) {
+                        prod[(2 * q) * MR_PLD + k] = av[u] * xv[u][q].x;
+                        prod[(2 * q + 1) * MR_PLD + k] = av[u] * xv[u][q].y;
+                    }
+                }
+            }
+            __syncthreads();
+            const int nrow = r1 - r0;
+            for (int it = tid; it < nrow * KB; it += THREADS) {
+                const int row = r0 + it / KB;
+                const double* pj = prod + (it % KB) * MR_PLD;
+                const int ra = __ldg(A->rowptr + row) - s, rb = __ldg(A->rowptr + row + 1) - s;
+                const double4 o = pre(b, row);
+                double t = 0.0;
+                for (int k = ra; k < rb; ++k) t += pj[k];
+                epi(b, row, t, o);
+            }
+        }
+        __syncthreads();  // prod / red are free again
+    }
+}
+
+// soc_apply for direction j of interleaved vectors
+template <int KB>
+__device__ void soc_apply_multi(const ConicOpView& op, int c, int j, bool valid, const double* __restrict__ y, double* out,
+                                int lig, int T) {
+    int off = 0, dim = 0, cs = 0;
+    double nx = 1.0, t = 0.0;
+    if (valid) {
+        off = op.soc_off[c];
+        dim = op.soc_dim[c];
+        cs = op.soc_case[c];
+        nx = op.soc_nx[c];
+        t = op.v[off];
+    }
+    auto at = [&](int k) { return (size_t)(off + k) * KB + j; };
+    double xy = 0.0;
+    if (valid && cs == 2)
+        for (int k = 1 + lig; k < dim; k += T) xy += op.v[off + k] * __ldcg(y + at(k));
+    for (int o = T >> 1; o > 0; o >>= 1) xy += __shfl_xor_sync(0xffffffffu, xy, o);
+    if (!valid) return;
+    if (cs == 0) {
+        for (int k = lig; k < dim; k += T) out[at(k)] = __ldcg(y + at(k));
+    } else if (cs == 1) {
+        for (int k = lig; k < dim; k += T) out[at(k)] = 0.0;
+    } else {
+        const double y0 = __ldcg(y + at(0));
+        const double inv2 = 1.0 / (2.0 * nx);
+        const double coef = t / (nx * nx) * xy;
+        for (int k = lig; k < dim; k += T) {
+            double r;
+            if (k == 0)
+                r = nx * y0 + xy;
+            else {
+                double xk = op.v[off + k];
+                r = xk * y0 + (nx + t) * __ldcg(y + at(k)) - coef * xk;
+            }
+            out[at(k)] = r * inv2;
+        }
+    }
+}
+
+// psd_apply_all for KB interleaved vectors: one flattened tile list over (direction, cone), so the four GEMM phases of
+// every direction share the three barriers; W1, W2 of direction j at w1 / w2 + j * sumd2
+template <int KB>
+__device__ void psd_apply_multi(Dev& d, const ConicOpView& op, const double* __restrict__ y, double* out, bool transpose,
+                                double* w1, double* w2, long long sumd2) {
+    if (op.npsd == 0) return;
+    __shared__ double As[PT * PLD], Bs[PT * PLD];
+    const double dscale = transpose ? 1.0 : 2.0, oscale = transpose ? 1.0 : 0.5;
+    const int ntot = op.psd_ntiles * KB;
+    for (int phase = 0; phase < 4; ++phase) {
+        for (int tt = blockIdx.x; tt < ntot; tt += gridDim.x) {
+            const int j = tt / op.psd_ntiles, t = tt - j * op.psd_ntiles;
+            int lo = 0, hi = op.npsd - 1;
+            while (lo < hi) {
+                const int mid = (lo + hi + 1) >> 1;
+                if (__ldg(op.psd_toff + mid) <= t) lo = mid; else hi = mid - 1;
+            }
+            const int c = lo, dd = op.psd_d[c], off = op.psd_off[c];
+            const int nt = (dd + PT - 1) / PT, lt = t - __ldg(op.psd_toff + c);
+            const int i0 = (lt % nt) * PT, j0 = (lt / nt) * PT;
+            const long long uo = op.psd_uoff[c];
+            const double* U = op.psd_U + uo;
+            double* W1 = w1 + j * sumd2 + uo;
+            double* W2 = w2 + j * sumd2 + uo;
+            auto tri = [&](int r, int cc) { return (size_t)(off + (long long)cc * (cc + 1) / 2 + r) * KB + j; };
+            if (op.psd_ident[c]) {
+                if (phase == 3)
+                    for (int e = threadIdx.x; e < PT * PT; e += blockDim.x) {
+                        const int i = i0 + e % PT, jj = j0 + e / PT;
+                        if (i <= jj && jj < dd) out[tri(i, jj)] = __ldcg(y + tri(i, jj));
+                    }
+                continue;
+            }
+            if (phase == 0) {
+                psd_tile_gemm(dd, i0, j0, false, true, As, Bs,
+                    [&](int i, int k) { return U[k + (long long)i * dd]; },
+                    [&](int k, int jj) {
+                        const int r = k < jj ? k : jj, cc = k < jj ? jj : k;
+                        const double v = __ldcg(y + tri(r, cc));
+                        return k == jj ? v * dscale : v;
+                    },
+                    [&](int i, int jj, double v) { W1[i + (long long)jj * dd] = v; });
+            } else if (phase == 1) {
+                const double* Bm = op.psd_Bm + uo;
+                psd_tile_gemm(dd, i0, j0, true, true, As, Bs,
+                    [&](int i, int k) { return __ldcg(W1 + i + (long long)k * dd); },
+                    [&](int k, int jj) { return U[k + (long long)jj * dd]; },
+                    [&](int i, int jj, double v) { W2[i + (long long)jj * dd] = v * Bm[i + (long long)jj * dd]; });
+            } else if (phase == 2) {
+                psd_tile_gemm(dd, i0, j0, true, true, As, Bs,
+                    [&](int i, int k) { return U[i + (long long)k * dd]; },
+                    [&](int k, int jj) { return __ldcg(W2 + k + (long long)jj * dd); },
+                    [&](int i, int jj, double v) { W1[i + (long long)jj * dd] = v; });
+            } else if (i0 <= j0 + PT - 1) {
+                psd_tile_gemm(dd, i0, j0, true, false, As, Bs,
+                    [&](int i, int k) { return __ldcg(W1 + i + (long long)k * dd); },
+                    [&](int k, int jj) { return U[jj + (long long)k * dd]; },
+                    [&](int i, int jj, double v) {
+                        if (i <= jj) out[tri(i, jj)] = i == jj ? v * oscale : v;
+                    });
+            }
+        }
+        if (phase < 3) d.sync();
+    }
+}
+
+// dpi_apply for KB interleaved vectors (diagonal and 3 x 3 block rows: one thread per row and direction; SOC: 8 lanes per
+// cone and direction; PSD: psd_apply_multi)
+template <int KB, bool PSD>
+__device__ __forceinline__ void dpi_apply_multi(Dev& d, const ConicOpView& op, const double* __restrict__ y, double* out,
+                                                bool transpose, double* w1, double* w2, long long sumd2) {
+    for (int e = d.gtid; e < op.m * KB; e += d.gthreads) {
+        const int i = e / KB;
+        const int k = op.kind[i];
+        if (k == 0) {
+            out[e] = op.diag[i] * __ldcg(y + e);
+        } else if (k >= 4) {
+            const double* br = op.blk3 + 3 * (long long)i;
+            const double* yc = y + (e - (k - 4) * KB);
+            out[e] = br[0] * __ldcg(yc) + br[1] * __ldcg(yc + KB) + br[2] * __ldcg(yc + 2 * KB);
+        }
+    }
+    {
+        const int T = 8;
+        const int lig = d.lane & (T - 1);
+        const int ngroups = d.gthreads / T;
+        const int g = d.gtid / T;
+        const int npair = op.nsoc * KB;
+        for (int base = 0; base < npair; base += ngroups) {
+            const int p = base + g;
+            soc_apply_multi<KB>(op, p / KB, p % KB, p < npair, y, out, lig, T);
+        }
+    }
+    if constexpr (PSD) psd_apply_multi<KB>(d, op, y, out, transpose, w1, w2, sumd2);
+}
+
+// Per-direction scalars of one operator application, read by every thread for its direction t % KB
+struct MrScal {
+    double s_src, s_dst, src_last;
+    int write;  // 0: the direction's dst is not written (frozen, or beta = 0 before an M' application)
+};
+
+// dst = s_src * OP(src) + s_dst * dst for the KB directions (OP = M, or M' when `transpose`); partial sums of ||dst||^2
+// (without the last row) into `slot`, of the last-row dot product into slot + 1; ends behind a barrier.
+template <int KB, bool PSD>
+__device__ __forceinline__ void conic_apply_multi(Dev& d, const ConicOpView& op, bool transpose, const double* __restrict__ src,
+                                                  double* dst, const MrScal& sc, int slot, double* wc, double* w1, double* w2,
+                                                  long long sumd2) {
+    const int n = op.n, m = op.m;
+    const double ss = sc.s_src, sd = sc.s_dst, t3 = sc.src_last;
+    const bool wr = sc.write != 0;
+    const int j = d.tid % KB;
+    double acc = 0.0, dot = 0.0;
+    auto at = [&](int row) { return (size_t)row * KB + j; };
+    if (!transpose) {
+        dpi_apply_multi<KB, PSD>(d, op, src + (size_t)n * KB, wc, false, w1, w2, sumd2);  // wc = Dpi t2
+        d.sync();
+        const int nbt = op.At.nblk;
+        spmm_stream<KB>(
+            d.rank(), d.nblk, nbt + op.A.nblk, cl_prod, d.red,
+            [&](int b, const CsrView*& A, const double*& x, int& lb) {
+                if (b < nbt) { A = &op.At; x = wc; lb = b; }
+                else { A = &op.A; x = src; lb = b - nbt; }
+            },
+            [&](int b, int row) {
+                return b < nbt ? make_double4(op.c[row], __ldcg(dst + at(row)), __ldcg(src + at(row)), 0.0)
+                               : make_double4(__ldcg(wc + at(row)), __ldcg(src + at(n + row)), op.b[row], __ldcg(dst + at(n + row)));
+            },
+            [&](int b, int row, double t, const double4& o) {
+                if (b < nbt) {
+                    t = (t + o.x * t3) * ss + sd * o.y;
+                    if (wr) dst[at(row)] = t;
+                    acc += t * t;
+                    dot += o.x * o.z;
+                } else {
+                    t = (-t + o.y - o.x + o.z * t3) * ss + sd * o.w;
+                    if (wr) dst[at(n + row)] = t;
+                    acc += t * t;
+                    dot += o.z * o.x;
+                }
+            });
+    } else {
+        spmm_stream<KB>(   // wc = A u1 - u2 - b u3
+            d.rank(), d.nblk, op.A.nblk, cl_prod, d.red,
+            [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.A; x = src; lb = b; },
+            [&](int, int row) { return make_double4(__ldcg(src + at(n + row)), op.b[row], 0.0, 0.0); },
+            [&](int, int row, double t, const double4& o) {
+                wc[at(row)] = t - o.x - o.y * t3;
+                dot += o.y * o.x;
+            });
+        d.sync();
+        double* r2 = wc + (size_t)m * KB;
+        dpi_apply_multi<KB, PSD>(d, op, wc, r2, true, w1, w2, sumd2);
+        d.sync();
+        const double* src2 = src + (size_t)n * KB;
+        spmm_stream<KB>(
+            d.rank(), d.nblk, op.At.nblk, cl_prod, d.red,
+            [&](int b, const CsrView*& A, const double*& x, int& lb) { A = &op.At; x = src2; lb = b; },
+            [&](int, int row) { return make_double4(op.c[row], __ldcg(dst + at(row)), __ldcg(src + at(row)), 0.0); },
+            [&](int, int row, double t, const double4& o) {
+                t = (-t - o.x * t3) * ss + sd * o.y;
+                if (wr) dst[at(row)] = t;
+                acc += t * t;
+                dot += o.x * o.z;
+            });
+        for (int e = d.rank() * MR_THREADS + d.tid; e < m * KB; e += d.nblk * MR_THREADS) {
+            const double t = (__ldcg(r2 + e) + __ldcg(src2 + e)) * ss + sd * __ldcg(dst + (size_t)n * KB + e);
+            if (wr) dst[(size_t)n * KB + e] = t;
+            acc += t * t;
+        }
+    }
+    mr_block_partial<KB>(d, slot, acc);
+    mr_block_partial<KB>(d, slot + 1, dot);
+    d.sync();
+}
+
+// The LSQR iteration of lsqr_body for the KB directions of group g.
+template <int KB, bool CLUSTER>
+__global__ void __launch_bounds__(MR_THREADS, 2) lsqr_multi_kernel(MultiArgs a, LsqrParams prm) {
+    constexpr bool PSD = !CLUSTER;  // problems with PSD cones take the cooperative route
+    __shared__ double red[(MR_THREADS / 32) * KB];
+    __shared__ LsqrScalars sc[KB];
+    __shared__ MrScal fw[KB], bw[KB];   // scalars of the next M v / M' u application
+    __shared__ double ulast[KB], vlast[KB];  // last entries of u and v (never read from memory, see conic_apply)
+    __shared__ int active[KB];
+    const ConicOpView& op = a.op;
+    const int n = op.n, m = op.m, N = n + m + 1;
+    const int slot = CLUSTER ? (int)blockIdx.x / a.ctas : 0;
+    const int g = a.group0 + slot;
+    const int C = CLUSTER ? a.ctas : (int)gridDim.x;
+    const int cta = CLUSTER ? (int)blockIdx.x - slot * a.ctas : (int)blockIdx.x;
+    double* u = a.work + (size_t)slot * a.work_stride;
+    double* v = u + (size_t)N * KB;
+    double* w = v + (size_t)N * KB;
+    double* wc = w + (size_t)N * KB;
+    double* w1 = wc + (size_t)2 * m * KB;
+    double* w2 = w1 + (size_t)a.sumd2 * KB;
+    double* partials = w2 + (size_t)a.sumd2 * KB;
+    const double* rhs = a.rhs + (size_t)g * N * KB;
+    double* x = a.x + (size_t)g * N * KB;
+    double* stats = a.stats + (size_t)g * KB * 4;
+    Dev d{cg::this_grid(), partials, red, (int)threadIdx.x, (int)(threadIdx.x & 31), (int)(threadIdx.x >> 5),
+          (int)(blockDim.x >> 5), C, cta * MR_THREADS + (int)threadIdx.x, C * MR_THREADS, CLUSTER, CLUSTER ? cta : -1, false};
+    const int NK = N * KB;
+    const int jt = d.tid % KB;  // this thread's direction in every element-wise loop and row epilogue
+    auto freeze = [&](int j) {  // by thread j of every CTA
+        active[j] = 0;
+        bw[j].write = 0;
+        if (d.rank() == 0) {
+            stats[j * 4 + 0] = (double)sc[j].istop;
+            stats[j * 4 + 1] = (double)sc[j].itn;
+            stats[j * 4 + 2] = sc[j].rnorm;
+            stats[j * 4 + 3] = sc[j].arnorm;
+        }
+    };
+
+    double acc = 0.0;  // u = b, x = v = w = 0
+    for (int e = d.gtid; e < NK; e += d.gthreads) {
+        const double t = rhs[e];
+        u[e] = t;
+        acc += t * t;
+        x[e] = 0.0;
+        v[e] = 0.0;
+        w[e] = 0.0;
+    }
+    mr_block_partial<KB>(d, 0, acc);
+    d.sync();
+    if (d.tid < KB) {
+        const int j = d.tid;
+        const bool zero = sqrt(a.rhs_norm2[(size_t)g * KB + j]) <= a.zero_below;
+        ulast[j] = rhs[(size_t)(N - 1) * KB + j];
+        vlast[j] = 0.0;
+        const bool op1 = sc[j].start(zero ? 0.0 : mr_total<KB>(d, 0, j), -1.0);
+        bw[j] = MrScal{sc[j].su, 0.0, ulast[j], op1 ? 1 : 0};
+    }
+    __syncthreads();
+    bool any = false;
+    for (int j = 0; j < KB; ++j) any |= bw[j].write != 0;
+    if (any) conic_apply_multi<KB, PSD>(d, op, true, u, v, bw[jt], 2, wc, w1, w2, a.sumd2);  // v_mem = M' u_true
+    if (d.tid < KB) {
+        const int j = d.tid;
+        double a2 = 0.0;
+        if (bw[j].write) {
+            const double last = mr_total<KB>(d, 3, j) * bw[j].s_src;
+            vlast[j] = last;
+            a2 = mr_total<KB>(d, 2, j) + last * last;
+        }
+        sc[j].first_alpha(a2);
+        active[j] = 1;
+        if (sc[j].arnorm == 0.0) freeze(j);
+        fw[j] = MrScal{sc[j].sv, -sc[j].alpha * sc[j].su, vlast[j], active[j]};
+    }
+    bool first = true;
+    long long itn = 0;
+    while (true) {
+        __syncthreads();
+        any = false;
+        for (int j = 0; j < KB; ++j) any |= active[j] != 0;
+        if (!any) break;
+        {   // deferred x / w update of the active directions (w = sv v at start); ||w / rho||^2 into slot 4
+            const bool act = active[jt] != 0;
+            const double svj = sc[jt].sv, t1 = sc[jt].t1, t2 = sc[jt].t2, irho = 1.0 / sc[jt].rho;
+            const double vl = vlast[jt];
+            double dd = 0.0;
+            if (act) {
+                for (int e = d.gtid; e < NK; e += d.gthreads) {
+                    const double ve = e >= NK - KB ? vl : v[e];
+                    if (first) {
+                        w[e] = svj * ve;
+                    } else {
+                        const double wi = w[e];
+                        const double dk = wi * irho;
+                        dd += dk * dk;
+                        x[e] += t1 * wi;
+                        w[e] = svj * ve + t2 * wi;
+                    }
+                }
+            }
+            mr_block_partial<KB>(d, 4, dd);
+        }
+        const bool more = itn < prm.maxiter;
+        if (more) conic_apply_multi<KB, PSD>(d, op, false, v, u, fw[jt], 0, wc, w1, w2, a.sumd2);  // u = M v_true - alpha u_true
+        else d.sync();
+        if (d.tid < KB && active[d.tid]) {
+            const int j = d.tid;
+            double unorm2 = 0.0;
+            if (more) {
+                const double last = -mr_total<KB>(d, 1, j) * fw[j].s_src + fw[j].s_dst * ulast[j];
+                ulast[j] = last;
+                unorm2 = mr_total<KB>(d, 0, j) + last * last;
+            }
+            if (!first) sc[j].stop_tests(mr_total<KB>(d, 4, j), prm);
+            if (sc[j].istop > 0 || !more) {
+                freeze(j);
+            } else {
+                const bool op1 = sc[j].next_beta(unorm2);
+                bw[j] = MrScal{sc[j].su, -sc[j].beta * sc[j].sv, ulast[j], op1 ? 1 : 0};
+            }
+        }
+        first = false;
+        __syncthreads();
+        any = false;
+        bool live = false;
+        for (int j = 0; j < KB; ++j) {
+            any |= bw[j].write != 0 && active[j] != 0;
+            live |= active[j] != 0;
+        }
+        if (!live) break;
+        if (any) conic_apply_multi<KB, PSD>(d, op, true, u, v, bw[jt], 2, wc, w1, w2, a.sumd2);  // v = M' u_true - beta v_true
+        if (d.tid < KB && active[d.tid]) {
+            const int j = d.tid;
+            if (bw[j].write) {
+                const double last = mr_total<KB>(d, 3, j) * bw[j].s_src + bw[j].s_dst * vlast[j];
+                vlast[j] = last;
+                sc[j].next_alpha(mr_total<KB>(d, 2, j) + last * last);
+            }
+            sc[j].rotate();
+            fw[j] = MrScal{sc[j].sv, -sc[j].alpha * sc[j].su, vlast[j], 1};
+        }
+        ++itn;
+    }
+}
+
 CsrView view_of(const DevBuf& rp, const DevBuf& ci, const DevBuf& v, int64_t nrows, int64_t ncols,
                 const DevBuf* blk = nullptr, int64_t nblk = 0, const DevBuf* sval = nullptr, const DevBuf* scol = nullptr,
                 const DevBuf* spos = nullptr) {
@@ -1405,6 +1915,75 @@ int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& sta
     DO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
     DO_CUDA(ctx, cudaLaunchKernelExC(&cfg, kern, args));
     ctx->launches++;
+    DO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    return 0;
+}
+
+// Many right-hand sides against the operator of the current conic_setup (lsqr_multi_kernel), G groups of KB directions.
+// Operators up to CL_CLUSTER_WORK without PSD cones: one thread-block cluster per group, every group in one launch
+// (clusters beyond those the GPU holds at once start as earlier groups retire).  Larger operators and problems with PSD
+// cones: one cooperative grid per group, the groups one after another.
+int32_t lsqr_run_conic_multi(diffopt_b200_ctx* ctx, int KB, int64_t G, const double* rhs, const double* rhs_norm2,
+                             double zero_below, LsqrParams prm, double* x, double* stats) {
+    ConicState& s = ctx->conic;
+    const int64_t n = s.n, m = s.m, N = n + m + 1;
+    MultiArgs a{};
+    a.op = conic_view(ctx, true);  // the blk / t_blk row blocks
+    a.rhs = rhs;
+    a.rhs_norm2 = rhs_norm2;
+    a.zero_below = zero_below;
+    a.x = x;
+    a.stats = stats;
+    a.sumd2 = s.psd_sumd2;
+    const int64_t work = s.A.nnz * 2 + n + 2 * m + s.psd_sumd2 * 8;
+    bool cluster = work <= CL_CLUSTER_WORK && s.npsd == 0;
+    const void* k_cluster = KB == 4 ? (const void*)lsqr_multi_kernel<4, true> : (const void*)lsqr_multi_kernel<8, true>;
+    const void* k_grid = KB == 4 ? (const void*)lsqr_multi_kernel<4, false> : (const void*)lsqr_multi_kernel<8, false>;
+    const size_t dyn = sizeof(double) * (size_t)KB * MR_PLD;
+    int cs = 0;
+    if (cluster) {
+        DO_CUDA(ctx, cudaFuncSetAttribute(k_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+        if (cudaFuncSetAttribute(k_cluster, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess) cudaGetLastError();
+        for (int c : {16, 8}) {
+            cudaLaunchAttribute at;
+            cudaLaunchConfig_t cfg = cluster_config((unsigned)c, (unsigned)c, dyn, nullptr, at);
+            cfg.blockDim = dim3(MR_THREADS);
+            int resident = 0;
+            if (cudaOccupancyMaxActiveClusters(&resident, k_cluster, &cfg) == cudaSuccess && resident >= 1) {
+                cs = c;
+                break;
+            }
+            cudaGetLastError();
+        }
+        cluster = cs > 0;
+    }
+    int grid = cs;
+    if (!cluster) {
+        DO_CUDA(ctx, cudaFuncSetAttribute(k_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
+        grid = coop_grid(ctx, k_grid, dyn, work);
+    }
+    a.ctas = grid;
+    a.work_stride = (size_t)KB * (size_t)(3 * N + 2 * m + 2 * s.psd_sumd2 + (int64_t)LSQR_NSLOTS * grid);
+    const int64_t regions = cluster ? G : 1;
+    DO_CUDA(ctx, ctx->lsqr.m_work.reserve(sizeof(double) * a.work_stride * (size_t)regions));
+    a.work = ctx->lsqr.m_work.as<double>();
+    DO_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+    if (cluster) {
+        a.group0 = 0;
+        void* args[] = {&a, &prm};
+        cudaLaunchAttribute at;
+        cudaLaunchConfig_t cfg = cluster_config((unsigned)(G * cs), (unsigned)cs, dyn, ctx->stream, at);
+        cfg.blockDim = dim3(MR_THREADS);
+        DO_CUDA(ctx, cudaLaunchKernelExC(&cfg, k_cluster, args));
+        ctx->launches++;
+    } else {
+        for (int64_t g = 0; g < G; ++g) {
+            a.group0 = (int)g;
+            void* args[] = {&a, &prm};
+            DO_CUDA(ctx, cudaLaunchCooperativeKernel(k_grid, dim3(grid), dim3(MR_THREADS), args, dyn, ctx->stream));
+            ctx->launches++;
+        }
+    }
     DO_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     return 0;
 }

@@ -86,5 +86,10 @@ int32_t conic_apply_dpi(diffopt_b200_ctx* ctx, const double* t_dev, bool transpo
 int32_t lsqr_run_conic_batch(diffopt_b200_ctx* ctx, std::vector<ConicState>& states, int C, bool stage, double* work,
                              const LsqrBatchLayout& L, LsqrParams prm, double zero_below, DevBuf& ops_buf, DevBuf& vecs_buf,
                              DevBuf& rhs_buf);
+// KB (4 or 8) right-hand sides per group, G groups, against the operator of the current conic_setup (lsqr_multi_kernel):
+// rhs, x [G][N][KB] (interleaved), rhs_norm2 [G][KB] (a right-hand side of norm <= zero_below gives x = 0 and zero
+// statistics), stats [G][KB][4] = istop, itn, rnorm, arnorm.  Enqueued on ctx->stream between ctx->ev0 and ctx->ev1.
+int32_t lsqr_run_conic_multi(diffopt_b200_ctx* ctx, int KB, int64_t G, const double* rhs, const double* rhs_norm2,
+                             double zero_below, LsqrParams prm, double* x, double* stats);
 int32_t csr_from_csc_host(diffopt_b200_ctx* ctx, int64_t nrows, int64_t ncols, const int64_t* colptr,
                           const int64_t* rowval, const double* nzval, CsrDev& out);

@@ -350,6 +350,27 @@ int32_t diffopt_b200_conic_reverse(
     diffopt_b200_ctx* ctx, const double* dx_seed,
     double atol, double btol, double conlim, int64_t maxiter,
     double* g_out, double* dc_out, double* db_out, double* out_stats, int32_t memspace);
+/* Many directions against the current conic_setup (any cone kind), one LSQR launch for all of them; direction j gets
+ * the single-direction semantics of conic_forward / conic_reverse, and its result does not depend on the other
+ * directions of the call (bitwise).  Layout is direction-major: Julia's Matrix{Float64} of size (n, k) passes as is.
+ * k forward directions of forward_differentiate! (ConicProgram.jl:257-334) against the current conic_setup.
+ * dA: triplets with k+1 offsets (direction j = ptr[j] .. ptr[j+1]-1; 1-based rows / cols, duplicates summed,
+ * un-negated as conic_forward takes them); NULL struct or NULL ptr = zero.  db[k][m], dc[k][n] (NULL = zero).
+ * dx_out[k][n] = -(du - x dw), dz_out[k][n+m+1] (may be NULL), out_stats[k][4] = (istop, itn, rnorm, arnorm).
+ * A direction with ||g_j|| = 0 (:320) returns zeros and stats (0, 0, 0, 0); maxiter = 0 means n+m+1.
+ * Returns 0 for k = 0; -1 for k < 0, before conic_setup, or for a triplet outside the m x n matrix (conic_forward
+ * skips such triplets). */
+int32_t diffopt_b200_conic_forward_multi(
+    diffopt_b200_ctx* ctx, int64_t k, const diffopt_b200_coo_batch* dA, const double* db, const double* dc,
+    double atol, double btol, double conlim, int64_t maxiter,
+    double* dx_out, double* dz_out, double* out_stats, int32_t memspace);
+/* k reverse seeds of reverse_differentiate! (ConicProgram.jl:336-394): dx_seeds[k][n] ->
+ * g_out[k][n+m+1], dc_out[k][n], db_out[k][m], out_stats[k][4]; any output may be NULL.  A seed whose right-hand side
+ * has norm <= 1e-4 (:369) returns zeros. */
+int32_t diffopt_b200_conic_reverse_multi(
+    diffopt_b200_ctx* ctx, int64_t k, const double* dx_seeds,
+    double atol, double btol, double conlim, int64_t maxiter,
+    double* g_out, double* dc_out, double* db_out, double* out_stats, int32_t memspace);
 
 /* Lock-step batch of conic problems: B independent problems of equal size (n, m; any sparsity / solution / cone
  * list without PSD cones), each analysed like conic_setup, then ALL reverse solves advanced by ONE persistent kernel

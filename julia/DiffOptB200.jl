@@ -307,6 +307,40 @@ function conic_forward(ctx::Context, n::Int, m::Int, dA_rows::Vector{Int64}, dA_
     return (dx = dx, dz = dz, iterations = Int(stats[2]))
 end
 
+# Many directions per call against the current conic_setup (one LSQR launch): Jacobian columns or many sensitivity
+# directions.  Matrices are (rows, k): column j is direction j.  Like the QP multi helpers, these have not been run yet.
+"k reverse seeds dx (n, k) -> (g (n+m+1, k), dc (n, k), db (n, k), stats (4, k)) of reverse_differentiate! (:336-394)."
+function conic_reverse_multi(ctx::Context, n::Int, m::Int, dx::Matrix{Float64};
+                             atol = sqrt(eps()), btol = sqrt(eps()), conlim = 1 / sqrt(eps()), maxiter = n + m + 1)
+    k = size(dx, 2)
+    g = Matrix{Float64}(undef, n + m + 1, k); dc = Matrix{Float64}(undef, n, k); db = Matrix{Float64}(undef, m, k)
+    stats = zeros(4, k)
+    GC.@preserve dx g dc db stats begin
+        rc = ccall((:diffopt_b200_conic_reverse_multi, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Ptr{Float64}, Float64, Float64, Float64, Int64, Ptr{Float64}, Ptr{Float64},
+                    Ptr{Float64}, Ptr{Float64}, Int32),
+                   ctx.handle, k, dx, atol, btol, conlim, maxiter, g, dc, db, stats, HOST)
+    end
+    check(ctx, rc)
+    return (g = g, dc = dc, db = db, stats = stats)
+end
+
+"k forward directions of forward_differentiate! (:257-334): dA as (ptr, I, J, V) with k+1 offsets (or nothing),
+db (m, k), dc (n, k) (or nothing) -> (dx (n, k), dz (n+m+1, k), stats (4, k))."
+function conic_forward_multi(ctx::Context, n::Int, m::Int, k::Integer; dA = nothing, db = nothing, dc = nothing,
+                             atol = sqrt(eps()), btol = sqrt(eps()), conlim = 1 / sqrt(eps()), maxiter = n + m + 1)
+    dx = Matrix{Float64}(undef, n, k); dz = Matrix{Float64}(undef, n + m + 1, k); stats = zeros(4, k)
+    ca = _coo(dA)
+    GC.@preserve dA db dc ca dx dz stats begin
+        rc = ccall((:diffopt_b200_conic_forward_multi, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Ptr{CooBatch}, Ptr{Float64}, Ptr{Float64}, Float64, Float64, Float64, Int64,
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32),
+                   ctx.handle, k, _cp(ca), _p(db), _p(dc), atol, btol, conlim, maxiter, dx, dz, stats, HOST)
+    end
+    check(ctx, rc)
+    return (dx = dx, dz = dz, stats = stats)
+end
+
 # ------------------------------------------------------------------------------------------------
 # (4) ConicModel <: DiffOpt.AbstractModel -- the conic backend behind `DiffOpt.ModelConstructor`
 #     (no narrow hook exists for ConicProgram, so the backend type itself is provided).  Same stored quantities as
