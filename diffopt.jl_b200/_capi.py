@@ -50,6 +50,8 @@ SIGNATURES = {
     "diffopt_b200_qp_batch_factorize": (C.c_int32, [vp, vp, C.c_int32]),
     "diffopt_b200_qp_batch_reverse_multi": (C.c_int32, [vp, C.c_int64, vp, vp, C.c_int32]),
     "diffopt_b200_qp_batch_forward_multi": (C.c_int32, [vp, C.c_int64] + [vp] * 7 + [C.c_int32]),
+    "diffopt_b200_qp_batch_solve_lsqr": (C.c_int32, [vp, C.c_int64, C.c_int32, C.c_int32, C.c_int32] + [vp] * 13 +
+                                         [C.c_double, C.c_double, C.c_double, C.c_int64, vp, vp, vp, C.c_int32, C.c_int32]),
     "diffopt_b200_qp_batch_param_grads": (C.c_int32, [vp, vp, C.c_int32] + [vp] * 6 + [C.c_int32]),
     "diffopt_b200_kkt_solve_csc": (C.c_int32, [vp, C.c_int64, vp, vp, vp, C.c_int32, C.c_int64, vp, vp, C.c_int32]),
     "diffopt_b200_sparse_setup": (C.c_int32, [vp, C.c_int64, vp, vp, vp, C.c_int32, vp]),

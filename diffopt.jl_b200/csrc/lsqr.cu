@@ -597,104 +597,6 @@ __device__ __forceinline__ double op_apply(Dev& d, const OpArgs& o, bool adjoint
     return norm2;
 }
 
-// Scalars of LSQR (Paige-Saunders, damp = 0): the Golub-Kahan bidiagonalisation with true vectors u = su * u_mem and
-// v = sv * v_mem, the plane rotations, the norm and condition estimates and the stop code.  Every driver advances them
-// with these methods in the same order: start, first_alpha, then per iteration the stop tests of the previous one,
-// next_beta, next_alpha (when beta > 0) and rotate.
-struct LsqrScalars {
-    double alpha, beta, su, sv, rhobar, phibar, rho, t1, t2, tau;
-    double anorm, acond, ddnorm, res2, xnorm, xxnorm, z, sn2, cs2, rnorm, arnorm, bnorm;
-    long long itn;
-    int istop;
-
-    // beta = ||b|| from ||b||^2; right-hand sides of norm <= zero_below count as zero.  True when v = A'u is to be formed.
-    __device__ __forceinline__ bool start(double b2, double zero_below) {
-        *this = LsqrScalars{};
-        beta = sqrt(b2);
-        if (beta <= zero_below) beta = 0.0;
-        su = sv = rho = 1.0;
-        cs2 = -1.0;
-        rnorm = beta;
-        if (beta > 0) su = 1.0 / beta;
-        return beta > 0;
-    }
-    // alpha = ||A'u|| from its square (0 when beta = 0) and the start-up values of the recurrences
-    __device__ __forceinline__ void first_alpha(double a2) {
-        alpha = sqrt(a2);
-        if (alpha > 0) sv = 1.0 / alpha;
-        arnorm = alpha * beta;
-        bnorm = beta;
-        rhobar = alpha;
-        phibar = beta;
-    }
-    // stop tests of the iteration rotated last; dd: its share of ddnorm (sum of ||w / rho||^2)
-    __device__ __forceinline__ void stop_tests(double dd, const LsqrParams& prm) {
-        ddnorm += dd;
-        acond = anorm * sqrt(ddnorm);
-        const double test1 = rnorm / bnorm;
-        const double test2 = arnorm / (anorm * rnorm);
-        const double test3 = 1.0 / acond;
-        const double t1_ = test1 / (1.0 + anorm * xnorm / bnorm);
-        const double rtol = prm.btol + prm.atol * anorm * xnorm / bnorm;
-        const double ctol = prm.conlim > 0 ? 1.0 / prm.conlim : 0.0;
-        if (itn >= prm.maxiter) istop = 7;
-        if (1.0 + test3 <= 1.0) istop = 6;
-        if (1.0 + test2 <= 1.0) istop = 5;
-        if (1.0 + t1_ <= 1.0) istop = 4;
-        if (test3 <= ctol) istop = 3;
-        if (test2 <= prm.atol) istop = 2;
-        if (test1 <= rtol) istop = 1;
-    }
-    // next iteration: beta = ||A v - alpha u|| from its square.  True when the next alpha is to be formed.
-    __device__ __forceinline__ bool next_beta(double u2) {
-        itn += 1;
-        beta = sqrt(u2);
-        if (beta > 0) {
-            su = 1.0 / beta;
-            anorm = sqrt(anorm * anorm + alpha * alpha + beta * beta);
-        } else {
-            su = 1.0;  // u_mem is exactly zero
-        }
-        return beta > 0;
-    }
-    // alpha = ||A'u - beta v|| from its square
-    __device__ __forceinline__ void next_alpha(double v2) {
-        alpha = sqrt(v2);
-        sv = alpha > 0 ? 1.0 / alpha : 1.0;
-    }
-    __device__ __forceinline__ void rotate() {
-        const double rhobar1 = rhobar;
-        rho = hypot(rhobar1, beta);
-        const double cs = rhobar1 / rho, sn = beta / rho;
-        const double theta = sn * alpha;
-        rhobar = -cs * alpha;
-        const double phi = cs * phibar;
-        phibar = sn * phibar;
-        tau = sn * phi;
-        t1 = phi / rho;
-        t2 = -theta / rho;
-        const double delta = sn2 * rho, gambar = -cs2 * rho, rhs_ = phi - delta * z;
-        const double zbar = rhs_ / gambar;
-        xnorm = sqrt(xxnorm + zbar * zbar);
-        const double gamma = hypot(gambar, theta);
-        cs2 = gambar / gamma;
-        sn2 = theta / gamma;
-        z = rhs_ / gamma;
-        xxnorm += z * z;
-        rnorm = sqrt(phibar * phibar + res2);
-        arnorm = alpha * fabs(tau);
-    }
-    __device__ __forceinline__ void write_stats(double* stats) const {
-        stats[0] = (double)istop;
-        stats[1] = (double)itn;
-        stats[2] = rnorm;
-        stats[3] = arnorm;
-        stats[4] = anorm;
-        stats[5] = acond;
-        stats[6] = xnorm;
-    }
-};
-
 // u = b, x = v = w = 0; ||b||^2 into slot 0
 __device__ __forceinline__ void lsqr_init(Dev& d, int nr, int nc, const double* __restrict__ rhs, const LsqrVectors& vec) {
     double acc = 0.0;

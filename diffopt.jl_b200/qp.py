@@ -277,6 +277,44 @@ def solve_batch_ex(ctx, Q, G, A, h, z, lam, nu, fwd_dir=None, seed=None, shared_
     return fwd, rev, info
 
 
+def solve_batch_lsqr(ctx, G, A, h, z, lam, nu, fwd_dir=None, seed=None, shared_matrices=False, atol=None, btol=None,
+                     conlim=None, maxiter=None):
+    """``diffopt_b200_qp_batch_solve_lsqr``: the reference's LSQR branch (Q = 0, every LP) for a batch, one CTA per
+    instance.  Arguments as ``solve_batch_ex`` without Q; ``fwd_dir = (dQ, dq, dG, dh, dA, db)`` (any entry may be None).
+    Tolerances default to ``lsqr.DEFAULTS`` (IterativeSolvers' values), ``maxiter`` to n + m + p.  Returns
+    ``(fwd (B, N) or None, rev (B, N) or None, stats (B, 2, 4))``, stats = (istop, itn, rnorm, arnorm) of the forward,
+    then the reverse solve.  Singular KKT matrices give LSQR's minimum-norm answer, as in the reference."""
+    from .lsqr import DEFAULTS
+    z = np.ascontiguousarray(z, dtype=np.float64)
+    B, n = z.shape
+    m = 0 if lam is None else np.asarray(lam).reshape(B, -1).shape[1]
+    p = 0 if nu is None else np.asarray(nu).reshape(B, -1).shape[1]
+    N = n + m + p
+    def mat(X, r, k):
+        return None if X is None or r == 0 else colmajor(np.asarray(X, float).reshape(k, r, n), r, n, k)
+    vec = lambda v, k: None if v is None or k == 0 else np.ascontiguousarray(np.asarray(v, float).reshape(B, k))
+    km = 1 if shared_matrices else B
+    args = [mat(G, m, km), mat(A, p, km), vec(h, m), z, vec(lam, m), vec(nu, p)]
+    fwd = rev = sd = None
+    if fwd_dir is not None:
+        dQ, dq, dG, dh, dA, db = fwd_dir
+        args += [mat(dQ, n, B), vec(dq, n), mat(dG, m, B), vec(dh, m), mat(dA, p, B), vec(db, p)]
+        fwd = np.empty((B, N))
+    else:
+        args += [None] * 6
+    if seed is not None:
+        sd = vec(seed, n)
+        rev = np.empty((B, N))
+    stats = np.zeros((B, 2, 4))
+    rc = ctx.lib.diffopt_b200_qp_batch_solve_lsqr(
+        ctx.h, B, n, m, p, *[ptr(a) for a in args], ptr(sd),
+        DEFAULTS["atol"] if atol is None else atol, DEFAULTS["btol"] if btol is None else btol,
+        DEFAULTS["conlim"] if conlim is None else conlim, 0 if maxiter is None else int(maxiter),
+        ptr(fwd), ptr(rev), ptr(stats), HOST, _capi.QP_SHARED_MATRICES if shared_matrices else 0)
+    ctx.check(rc)
+    return fwd, rev, stats
+
+
 def shared_param_grads(ctx, z, lam, nu, rev, allreduce=False, flat=False):
     """``diffopt_b200_qp_batch_shared_grads``: batch sums of the reverse-mode parameter gradients (dQ, dq, dG, dh, dA, db)
     for parameters shared by all instances; ``allreduce`` adds the NCCL all-reduce over the ranks of

@@ -242,6 +242,27 @@ int32_t diffopt_b200_qp_batch_forward_multi(
     const diffopt_b200_coo_batch* dQ, const double* dq, const diffopt_b200_coo_batch* dG, const double* dh,
     const diffopt_b200_coo_batch* dA, const double* db, double* fwd_out, int32_t memspace);
 
+/* The LSQR branch of solve_system for a batch of B LPs (Q = 0, QuadraticProgram.jl:333-335, :436-438, :486-488):
+ * per instance, LHS = [0 G'diag(lam) A'; G diag(Gz-h) 0; A 0 0] (create_LHS_matrix with Q = 0);
+ * rev_out = -lsqr(LHS, [dl_dz; 0; 0]), fwd_out = -lsqr(LHS', RHS of :429-433), from x0 = 0 with (atol, btol, conlim,
+ * maxiter) -- maxiter = 0 means N = n+m+p, IterativeSolvers' max(size(LHS)).  Arguments as qp_batch_solve without Q
+ * (dQ still enters the forward right-hand side through dQ z); any direction array may be NULL (zero); fwd_out / rev_out
+ * may be NULL to skip that mode.  stats_out[B][2][4] (may be NULL) = (istop, itn, rnorm, arnorm) of the forward, then
+ * the reverse solve (zeros for a skipped mode).  flags: DIFFOPT_QP_SHARED_MATRICES (G, A one instance for the batch).
+ * An LP's KKT matrix is singular whenever the solution is not a nondegenerate vertex; LSQR then returns the minimum-norm
+ * least-squares answer, as the reference does, where the direct entries above report the instance singular.
+ * Each instance is solved by one CTA, bitwise reproducibly and independently of the rest of the batch.
+ * Never reports singular: returns 0, < 0 for bad arguments / unknown flags / CUDA errors, -3 for an instance whose
+ * LSQR vectors do not fit one CTA (use the single-instance lsqr_csc route).  Blocking; last_kernel_ms is its device time. */
+int32_t diffopt_b200_qp_batch_solve_lsqr(
+    diffopt_b200_ctx* ctx, int64_t B, int32_t n, int32_t m, int32_t p,
+    const double* G, const double* A, const double* h,
+    const double* z, const double* lam, const double* nu,
+    const double* dQ, const double* dq, const double* dG, const double* dh,
+    const double* dA, const double* db, const double* dl_dz,
+    double atol, double btol, double conlim, int64_t maxiter,
+    double* fwd_out, double* rev_out, double* stats_out, int32_t memspace, int32_t flags);
+
 /* Reverse-mode gradients w.r.t. the problem data from rev = (dz, dlam, dnu)
  * (getters QuadraticProgram.jl:307-314, :448-473; signs as the reference's tests read
  * them, test/utils.jl:178-233):

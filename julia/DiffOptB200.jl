@@ -180,6 +180,41 @@ function qp_batch_solve(ctx::Context, Q, G, A, h, z, lam, nu;
     return (forward = split(fwd), reverse = split(rev), info = info)
 end
 
+"""
+    qp_batch_solve_lsqr(ctx, G, A, h, z, lam, nu; dQ, dq, dG, dh, dA, db, dl_dz, shared_matrices, atol, btol, conlim, maxiter)
+
+The LSQR branch of `solve_system` (Q = 0, QuadraticProgram.jl:486-488) for a batch of LPs, one CTA per instance: singular
+KKT matrices give LSQR's minimum-norm answer as in the reference.  Layouts as `qp_batch_solve` without Q (`G` of size
+(m, n, B), or (m, n) with `shared_matrices = true`).  Tolerances default to IterativeSolvers' values; `maxiter = 0` means
+n + m + p.  `stats[:, k, b]` = (istop, itn, rnorm, arnorm) of the forward (k = 1) and reverse (k = 2) solve of instance b.
+"""
+function qp_batch_solve_lsqr(ctx::Context, G, A, h, z, lam, nu;
+                             dQ = nothing, dq = nothing, dG = nothing, dh = nothing, dA = nothing, db = nothing,
+                             dl_dz = nothing, shared_matrices::Bool = false, atol::Float64 = sqrt(eps(Float64)),
+                             btol::Float64 = sqrt(eps(Float64)), conlim::Float64 = 1 / sqrt(eps(Float64)),
+                             maxiter::Integer = 0)
+    n, B = size(z)
+    m = size(lam, 1)
+    p = size(nu, 1)
+    N = n + m + p
+    fwd = any(!isnothing, (dQ, dq, dG, dh, dA, db)) ? Matrix{Float64}(undef, N, B) : nothing
+    rev = dl_dz === nothing ? nothing : Matrix{Float64}(undef, N, B)
+    stats = zeros(Float64, 4, 2, B)
+    GC.@preserve G A h z lam nu dQ dq dG dh dA db dl_dz fwd rev stats begin
+        rc = ccall((:diffopt_b200_qp_batch_solve_lsqr, LIB), Int32,
+                   (Ptr{Cvoid}, Int64, Int32, Int32, Int32,
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                    Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+                    Float64, Float64, Float64, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int32, Int32),
+                   ctx.handle, B, n, m, p, _p(G), _p(A), _p(h), _p(z), _p(lam), _p(nu),
+                   _p(dQ), _p(dq), _p(dG), _p(dh), _p(dA), _p(db), _p(dl_dz), atol, btol, conlim, maxiter,
+                   _p(fwd), _p(rev), stats, HOST, shared_matrices ? QP_SHARED_MATRICES : Int32(0))
+    end
+    check(ctx, rc)
+    split(x) = x === nothing ? nothing : (dz = x[1:n, :], dλ = x[n+1:n+m, :], dν = x[n+m+1:end, :])
+    return (forward = split(fwd), reverse = split(rev), stats = stats)
+end
+
 # Stream-ordered form for device-resident batches (pointers of CUDA.jl arrays, `pointer(x)` converted to Ptr{Float64}):
 # enqueue any number of batches, then `synchronize(ctx)` waits and throws for the status of the last one.
 function qp_batch_solve_async(ctx::Context, B::Integer, n::Integer, m::Integer, p::Integer,
